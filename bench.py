@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                     # B200 path (this repo), default config amos98
     python bench.py --config {amos98|amos2645|btcv_b8_ens3|msd128_ddim25|wide} ...
     python bench.py --impl reference --gpus N --steps K ...           # the reference's CPU path (oracle port), host cores
+    python bench.py ... --dump-outputs DIR                            # also write the last timed step's labels to DIR/labels.npy
 
 One "step" = one pass of the hot path over one synthetic CT volume: window crop, encoder + N DDIM steps per window,
 stitching, division by the coverage counts, binarisation.  Legs of the B200 arm (each bracketed by barrier + synchronize,
@@ -76,6 +77,29 @@ def algorithmic_gflop(features, classes, S, n_steps):
         den3 += conv(V[l - 1], f[l - 1] + up, out) + conv(V[l - 1], out, out)
     other += 2.0 * V[0] * f[5] * classes
     return enc / 1e9, (den3 + other) / 1e9, den3 / 1e9
+
+
+DUMP_MAX_VALUES = 1 << 23  # 32 MB of float32: the largest array --dump-outputs writes whole
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor of ``arrays`` as out_dir/<name>.npy in float32: whole when it has at most DUMP_MAX_VALUES
+    elements, otherwise the elements at DUMP_MAX_VALUES flat indices drawn from numpy default_rng(0) (with repetition,
+    sorted), the same for every run of the same configuration.  Returns what was written, for the JSON line."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    info = {}
+    for name, t in arrays.items():
+        entry = {"shape": list(t.shape), "dtype": str(t.dtype).replace("torch.", "")}
+        if t.numel() > DUMP_MAX_VALUES:
+            idx = np.sort(np.random.default_rng(0).integers(0, t.numel(), DUMP_MAX_VALUES))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+            entry["sample"] = f"{DUMP_MAX_VALUES} flat indices, numpy default_rng(0).integers(0, numel, n), sorted"
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+        info[name] = entry
+    return {"dir": out_dir, "arrays": info}
 
 
 def measured_peaks():
@@ -330,6 +354,7 @@ def run_b200(args, cfg):
         clk = clocks.stop() if clocks else None
         ms = e0.elapsed_time(e1)
         last_labels = labels[0] if rank == 0 else None  # volume 0 of the queue: its windows draw the noise streams (seed, 0 .. n_win - 1)
+        final_labels = labels[-1] if rank == 0 and args.dump_outputs else None  # what the last timed step returned
         del labels
         # ---------------- end-to-end leg: host volume in, host labels out, every step ----------------
         barrier()
@@ -513,6 +538,8 @@ def run_b200(args, cfg):
             te, ts = cpu_window_sample(cfg, threads)
             out["cpu_baseline"] = {"value": 1.0 / (te + cfg["ddim"] * ens * ts), "unit": "patches/s", "cores": threads, "kind": "port",
                                    "sample": cpu_sample_text(cfg)}
+        if final_labels is not None:
+            out["dump_outputs"] = dump_outputs(args.dump_outputs, {"labels": final_labels})
         print_json(out)
     if world > 1:
         dist.destroy_process_group()
@@ -550,7 +577,14 @@ def main():
                     help="N > 1: how the per-rank partial volumes are combined: p2p = one fused kernel over NVLink peer memory (reduce + "
                          "finalize + gather, dist.PeerExchange), nccl = reduce-scatter + finalize + gather collectives; auto = p2p when it applies")
     ap.add_argument("--dual-stream", type=int, default=1, help="DUNET_FLAG_DUAL_STREAM: two half batches on two internal streams (the product default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the label volume the last timed step returned as DIR/labels.npy (float32; "
+                         "volumes over 2^23 voxels as a fixed seeded sample) so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs the B200 path (the reference arm times a sample of one window and returns no volume)")
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
         run_reference(args, cfg)

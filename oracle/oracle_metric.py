@@ -1,8 +1,7 @@
 """CPU restatement of the evaluation metric on the inference path.  TEST INFRASTRUCTURE ONLY (oracle).
 
 Follows the reference's ``dice_coeff`` (metric.py:3-49) and the per-class rule of ``Tester.validation_step``
-(test.py:143-151).  PARITY PIN: tests/test_oracle_metric.py checks this restatement against the reference's own
-``metric.py`` (imported unmodified when /root/reference exists) and against hand-computed known answers.
+(test.py:143-151).  PARITY PIN: tests/test_oracle_metric.py checks this restatement against hand-computed known answers.
 """
 from __future__ import annotations
 

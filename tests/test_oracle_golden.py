@@ -1,5 +1,5 @@
 """Pin the oracle (oracle/) against goldens produced by running the UNMODIFIED reference
-(oracle/make_golden.py) and, when /root/reference is present, against the live reference."""
+(oracle/make_golden.py)."""
 import json
 import os
 
@@ -8,7 +8,6 @@ import pytest
 import torch
 
 from oracle import oracle_ddim, oracle_model
-from oracle.ref_loader import reference_available
 from tests.util import GOLDEN, SMALL, load_golden, rel_l2, seeded_image, seeded_noise
 
 FP32_TOL = 2e-5  # same fp32 algorithm, different summation order across CPU kernels
@@ -72,26 +71,20 @@ def test_window_matches_reference_golden(tag, cout, S, feats):
     assert float(acc.min()) >= -10.0 and float(acc.max()) <= 10.0  # sum of 10 clamped x0 (diffusion.py:94-98)
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present (GPU box)")
-def test_oracle_matches_live_reference():
-    from oracle.ref_loader import build_reference_model
-
+def test_oracle_matches_reference_outputs_tight():
+    """The S32_C2_small case against the reference's own outputs at full resolution (window_S32_C2_small.npz stores every
+    voxel), at the tolerances of a same-machine comparison: the same fp32 graph, only CPU kernel choice may differ.  The
+    weights are pinned bit-exactly by test_weight_init_matches_reference[C2_small]."""
     cout, S = 2, 32
-    m = build_reference_model(1, cout, list(SMALL), seed=0)
-    sd = oracle_model.init_state_dict(1, cout, SMALL, seed=0)
-    for k, v in m.state_dict().items():
-        assert torch.equal(v, sd[k]), k
-    image = seeded_image((1, 1, S, S, S))
-    noise = seeded_noise((1, cout, S, S, S))
-    with torch.no_grad():
-        emb_ref = m.embed_model(image)
-        emb = oracle_model.encoder_forward(sd, image)
-        for a, b in zip(emb, emb_ref):
-            assert rel_l2(a, b) < 1e-6
-        t = torch.tensor([555])
-        assert rel_l2(oracle_model.denoiser_forward(sd, noise, t, image, emb),
-                      m.model(noise, t, image=image, embeddings=emb_ref)) < 1e-6
-        out = m.sample_diffusion.ddim_sample_loop(m.model, tuple(noise.shape), noise=noise,
-                                                  model_kwargs={"image": image, "embeddings": emb_ref})
-        res = oracle_ddim.ddim_sample_window(lambda x, tt: oracle_model.denoiser_forward(sd, x, tt, image, emb), noise)
-    assert rel_l2(res["sample_return"], sum(out["all_samples"])) < 1e-5
+    g = load_golden("window_S32_C2_small.npz")
+    assert int(g["sub"]) == 1
+    emb, res, logits999 = _oracle_window(cout, S, SMALL)
+    assert rel_l2(emb[0][:, ::8, ::4, ::4, ::4], g["emb0"]) < 1e-6
+    assert rel_l2(emb[4], g["emb4"]) < 1e-6
+    for i, e in enumerate(emb):
+        assert abs(float(e.double().sum()) - g["emb_sum"][i]) <= 1e-6 * g["emb_abs"][i]
+    assert rel_l2(logits999, g["logits999"]) < 1e-6
+    for k, o in enumerate(res["model_outputs"]):
+        assert abs(float(o.double().sum()) - g["step_out_sum"][k]) <= 1e-5 * g["step_out_abs"][k]
+    assert rel_l2(res["sample_return"], g["acc"]) < 1e-5
+    assert rel_l2(res["final_x"], g["final_x"]) < 1e-5

@@ -1,15 +1,10 @@
-"""Pins oracle/oracle_metric.py against the reference's own metric.py (when /root/reference is mounted) and against
-hand-computed known answers; checks the product's host-side Dice rule against the oracle."""
-import importlib.util
-import os
-
+"""Pins oracle/oracle_metric.py against hand-computed known answers; checks the product's host-side Dice rule against the
+oracle."""
 import pytest
 import torch
 
 import diff_unet_amos_b200.engine as eng
 from oracle import oracle_metric
-
-REF = "/root/reference/metric.py"
 
 
 def _cases():
@@ -27,18 +22,6 @@ def test_known_answers():
     assert oracle_metric.dice_coeff(z, z) == 0.0  # ZeroDivisionError branch, metric.py:44-47
     assert oracle_metric.per_class_dice(r.view(1, 1, 6), z.view(1, 1, 6)) == [1.0]  # test.py:146-147
     assert oracle_metric.per_class_dice(z.view(1, 1, 6), l.view(1, 1, 6)) == [0.0]
-
-
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference not mounted (GPU box)")
-def test_against_unmodified_reference_metric():
-    spec = importlib.util.spec_from_file_location("_ref_metric", REF)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    a, b = _cases()
-    for c in range(3):
-        assert float(mod.dice_coeff(a[:, c], b[:, c])) == pytest.approx(oracle_metric.dice_coeff(a[:, c], b[:, c]), abs=1e-7)
-    z = torch.zeros(4, 4)
-    assert float(mod.dice_coeff(z, z)) == 0.0 == oracle_metric.dice_coeff(z, z)
 
 
 def test_host_rule_matches_oracle():
