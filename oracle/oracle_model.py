@@ -134,7 +134,7 @@ def sinusoid_embedding(t: torch.Tensor, dim: int = TEMB_DIM) -> torch.Tensor:
 
 def time_embedding(sd, t: torch.Tensor) -> torch.Tensor:
     """TimeStepEmbedder.forward (models/diffusion/utils.py:49-54)."""
-    e = sinusoid_embedding(t)
+    e = sinusoid_embedding(t).to(sd["model.temb.dense.0.weight"].dtype)  # no-op in fp32; lets the oracle run in fp64
     e = F.linear(e, sd["model.temb.dense.0.weight"], sd["model.temb.dense.0.bias"])
     return F.linear(_swish(e), sd["model.temb.dense.1.weight"], sd["model.temb.dense.1.bias"])
 

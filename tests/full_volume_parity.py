@@ -4,7 +4,11 @@ in fp32 on the GPU (TF32 off), window by window with identical weights / image /
 north_star gates on the whole volume: per-patch rel-l2, label agreement of the reference's binarisation (out > 0) and of
 argmax, raw and margin-filtered.  Lives under tests/ because only tests/ may import oracle/.
 
-    python tests/full_volume_parity.py [--windows N]      (N < 98: only the first N windows, for a quick look)
+    python tests/full_volume_parity.py [--windows N] [--image {rand,phantom}]
+        N < 98: only the first N windows, for a quick look
+        phantom: a body-shaped CT phantom through the reference's intensity window (tests/realistic.py: air outside the
+        body, soft tissue with a faint texture, organs, a clipped bone rod) and trained-like parameters (distinct
+        InstanceNorm gamma / beta, large conv biases) instead of torch.rand and the seeded initialisation
 """
 import argparse
 import os
@@ -16,9 +20,11 @@ import torch
 
 import diff_unet_amos_b200 as pkg
 from oracle import oracle_ddim, oracle_model
+from tests import realistic
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--windows", type=int, default=98)
+ap.add_argument("--image", choices=("rand", "phantom"), default="rand")
 a = ap.parse_args()
 torch.backends.cudnn.allow_tf32 = False
 torch.backends.cuda.matmul.allow_tf32 = False
@@ -29,11 +35,13 @@ dev = "cuda"
 torch.manual_seed(0)
 models = {prec: pkg.DiffUNetB200(in_channels=1, out_channels=C, image_size=96, spatial_size=96, batch_max=2, precision=prec).to(dev).eval()
           for prec in PRECS}
+if a.image == "phantom":
+    models[PRECS[0]].load_state_dict(realistic.trained_like_state_dict(models[PRECS[0]].state_dict(), seed=0))
 for prec in PRECS[1:]:
     models[prec].load_state_dict(models[PRECS[0]].state_dict())
 sd = {k: v.detach() for k, v in models[PRECS[0]].state_dict().items()}
 torch.manual_seed(1)
-volume = torch.rand(1, 1, *VOL, device=dev)
+volume = torch.rand(1, 1, *VOL, device=dev) if a.image == "rand" else realistic.ct_phantom(VOL, "body", seed=1).to(dev)
 starts = pkg.window_starts(VOL, ROI, 0.25)[:a.windows]
 sched = oracle_ddim.SpacedSchedule(10)
 gen = torch.Generator(device=dev)
@@ -72,7 +80,8 @@ with torch.no_grad():
             for c in b.counts:
                 c.clamp_(min=1)
     ref_vol = bufs["oracle"].finalize()[0]
-    print(f"\nfull volume {VOL}, {len(starts)} windows, oracle = fp32 torch on the GPU (TF32 off)")
+    print(f"\nfull volume {VOL} ({a.image}), {len(starts)} windows, oracle = fp32 torch on the GPU (TF32 off), "
+          f"{torch.cuda.get_device_name()}")
     failed = []
     for prec in PRECS:
         out = bufs[prec].finalize()[0]
