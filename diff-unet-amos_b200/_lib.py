@@ -11,6 +11,7 @@ from ctypes import POINTER, c_char_p, c_float, c_int32, c_int64, c_size_t, c_uin
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libdunet_b200.so")
+DUNET_VERSION = 200  # include/dunet.h: the ABI the signatures below describe
 
 DUNET_FLAG_REF_CONV = 1
 DUNET_FLAG_KEEP_FP32_WEIGHTS = 2
@@ -60,8 +61,7 @@ SIGNATURES = {
     "dunet_zero": (c_int32, [c_void_p, c_size_t, c_void_p]),
     "dunet_crop_windows": (c_int32, [c_void_p, POINTER(c_int32), c_void_p, POINTER(c_int32), POINTER(c_int32), c_int32, c_void_p]),
     "dunet_infer_windows": (c_int32, [c_void_p, c_void_p, POINTER(c_int32), POINTER(c_int32), c_int32, c_void_p, c_uint64, POINTER(c_int64),
-                                      c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p]),
-    "dunet_infer_flush": (c_int32, [c_void_p, c_void_p]),
+                                      c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "dunet_stitch_add": (c_int32, [c_void_p, POINTER(c_int32), c_int32, c_void_p, POINTER(c_int32), POINTER(c_int32), c_void_p]),
     "dunet_finalize": (c_int32, [c_void_p, POINTER(c_int32), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "dunet_stitch_add_weighted": (c_int32, [c_void_p, c_void_p, POINTER(c_int32), c_int32, c_void_p, c_void_p, POINTER(c_int32), POINTER(c_int32), c_void_p]),
@@ -112,18 +112,13 @@ def load(build_if_missing: bool = True) -> ctypes.CDLL:
         except Exception:
             if not os.path.exists(LIB_PATH):  # no compiler on this box: a prebuilt library (it travels with the tree) is fine
                 raise
-    alt = os.environ.get("DUNET_LIB")  # A/B timing of an alternative build of the same ABI (debugging only)
-    if alt:
-        lib = ctypes.CDLL(alt)
-        for name, (res, args) in SIGNATURES.items():
-            fn = getattr(lib, name)
-            fn.restype = res
-            fn.argtypes = args
-        _lib = lib
-        return lib
     if not os.path.exists(LIB_PATH):
         raise ImportError(f"{LIB_PATH} is missing and there is no non-CUDA fallback; run diff-unet-amos_b200/build.py")
     lib = ctypes.CDLL(LIB_PATH)
+    lib.dunet_version.restype = c_int32
+    if lib.dunet_version() != DUNET_VERSION:  # e.g. a stale prebuilt library whose rebuild failed
+        raise ImportError(f"{LIB_PATH} implements ABI version {lib.dunet_version()}, these bindings need {DUNET_VERSION}; "
+                          "rebuild it with diff-unet-amos_b200/build.py")
     for name, (res, args) in SIGNATURES.items():
         fn = getattr(lib, name)  # AttributeError if the .so does not export a declared symbol
         fn.restype = res

@@ -98,11 +98,6 @@ static int prof_end_(Prof* pr, cudaStream_t st) {
 #define PROF_ON (prof_of(p)->on)
 
 // Launch with programmatic stream serialization (see pdl_sync() in ptx.cuh): only for kernels that call pdl_sync().
-// DUNET_NO_PDL=1 in the environment falls back to plain stream order (debugging / A-B timing).
-static bool pdl_enabled() {
-  static const bool on = [] { const char* e = getenv("DUNET_NO_PDL"); return !(e && e[0] == '1'); }();
-  return on;
-}
 template <typename... KArgs, typename... Args>
 static void launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg;
@@ -111,7 +106,7 @@ static void launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem,
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.attrs = at; cfg.numAttrs = 1;
   (void)cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);  // the error is picked up by LAUNCH_CHECK()
 }
 
@@ -347,7 +342,7 @@ struct Slot {
 };
 
 struct WsLayout {
-  size_t in_pack, raw, mid, partial, ss, splitk, affine, x_t, acc, acc2, image, total;
+  size_t in_pack, raw, mid, partial, ss, splitk, affine, x_t, acc, image, total;
   size_t emb[5], epool[5], x[5], dpool[5], up[5], u[5];
 };
 
@@ -380,19 +375,8 @@ struct dunet_plan {
   std::vector<void*> owned;
   // two internal streams: the two halves of a window batch run out of phase so that the HBM-bound kernels of one half
   // (normalise, final/DDIM, transposed conv) overlap the tensor-core-bound convolutions of the other
-  cudaStream_t half_stream[4] = {nullptr, nullptr, nullptr, nullptr};
-  cudaEvent_t ev_fork = nullptr, ev_join[4] = {nullptr, nullptr, nullptr, nullptr};
-  // deferred (pipelined) dunet_infer_windows: the sub-batches run on the internal streams WITHOUT joining the caller's
-  // stream; the stitch kernels run in window order on a third internal stream; dunet_infer_flush() joins.  Each half
-  // alternates between two accumulator buffers so that its next batch never waits for the stitch of the previous one.
-  cudaStream_t stitch_stream = nullptr;
-  cudaEvent_t ev_done[4] = {nullptr, nullptr, nullptr, nullptr};      // half h finished the DDIM steps of its current batch
-  cudaEvent_t ev_stitched[4][2] = {};                                 // the stitch kernels reading acc buffer f of half h are done
-  bool stitched_valid[4][2] = {};
-  int acc_flip[4] = {0, 0, 0, 0};
-  cudaEvent_t ev_stitch_tail = nullptr;
-  bool async_pending = false;
-  int async_B0 = 0;
+  cudaStream_t half_stream[2] = {nullptr, nullptr};
+  cudaEvent_t ev_fork = nullptr, ev_join[2] = {nullptr, nullptr};
   int num_sms = 0;
   mutable Prof prof;  // per-plan launch profiler (dunet_profile_*)
   // timesteps passed to dunet_denoise_step that are not one shared schedule entry (training-style calls, per-sample t):
@@ -452,28 +436,22 @@ static ConvGeom conv_geom(const dunet_plan* p, const ConvW& c, int lvl, int B) {
   // actually driven: 2-4 windows per launch (dual-stream half batches), so ~24+ work items per sample already fill the GPU.
   // Round 1 split K whenever a sample had < 96 items: at batch 4 that doubled the 24^3 / 12^3 launches into two waves of
   // half-K items, each still streaming its weights from L2, plus the reduce kernels (measured 0.31-0.38 of the tensor peak).
-  // The Cout = 64 z-stacked kernel always uses ZT = 4.
-  static const int zt_items = [] { const char* e = getenv("DUNET_GEOM_ZT_ITEMS"); return e ? atoi(e) : 24; }();
-  static const int split_items = [] { const char* e = getenv("DUNET_GEOM_SPLIT_ITEMS"); return e ? atoi(e) : 20; }();
+  // The Cout = 64 z-stacked kernel always uses ZT = 4.  ZT = 2 below 24 items per sample; split-K below 20.
   {
     const int tz4 = (p->D[lvl] + CONV_ZT - 1) / CONV_ZT;
     const int items4 = g.tiles_x * g.tiles_y * tz4 * c.n_tiles;
-    g.zt = (items4 < zt_items && !(c.coutp == 64 && c.cb_ch == 32)) ? 2 : CONV_ZT;
+    g.zt = (items4 < 24 && !(c.coutp == 64 && c.cb_ch == 32)) ? 2 : CONV_ZT;
   }
   g.tiles_z = (p->D[lvl] + g.zt - 1) / g.zt;
   g.tiles = g.tiles_x * g.tiles_y * g.tiles_z;
   (void)B;
   const int ctas = g.tiles * c.n_tiles, ncb = c.ncb();
   g.ksplit = 1;
-  if (ncb >= 2 && ctas < split_items) g.ksplit = std::max(1, std::min(ncb, 96 / ctas));
+  if (ncb >= 2 && ctas < 20) g.ksplit = std::max(1, std::min(ncb, 96 / ctas));
   // Deep levels (row of at most 30 voxels, Cout a multiple of 128): swapped-operand flattened-plane kernel.  N = positions
   // of a (ty rows x W + 2) halo-plane strip, as many rows as fit N <= 256; ZT slabs (a divisor of D, ZT * N <= 512 TMEM
-  // columns, rule below); split-K until a sample has ~48 items.  Again per-sample shapes only.
-  static const bool flat_on = [] { const char* e = getenv("DUNET_FLAT"); return !(e && e[0] == '0'); }();
-  static const int flat_split_items = [] { const char* e = getenv("DUNET_FLAT_SPLIT_ITEMS"); return e ? atoi(e) : 36; }();
-  static const int flat_target_items = [] { const char* e = getenv("DUNET_FLAT_TARGET_ITEMS"); return e ? atoi(e) : 48; }();
-  if (flat_on && !(p->cfg.flags & (DUNET_FLAG_REF_CONV | DUNET_FLAG_GENERIC_CONV)) && c.cb_ch == 64 && c.n_tile == 128 &&
-      p->W[lvl] + 2 <= 32) {
+  // columns, rule below); split-K when a sample has fewer than 36 items, until it has ~48.  Again per-sample shapes only.
+  if (!(p->cfg.flags & (DUNET_FLAG_REF_CONV | DUNET_FLAG_GENERIC_CONV)) && c.cb_ch == 64 && c.n_tile == 128 && p->W[lvl] + 2 <= 32) {
     const int Dl = p->D[lvl], Hl = p->H[lvl];
     const int hx = p->W[lvl] + 2, ty_max = 258 / hx;
     const int tiles_y = (Hl + ty_max - 1) / ty_max, ty = (Hl + tiles_y - 1) / tiles_y;
@@ -482,11 +460,10 @@ static ConvGeom conv_geom(const dunet_plan* p, const ConvW& c, int lvl, int B) {
     // 16 KB weight tile feeds ZT * npos / 2 MMA clocks; at >= 160 columns (<= ~50 B/clk/SM; measured at 24^3 with 144 CTAs
     // streaming concurrently: no slowdown, L2 serves CTAs that walk the same tiles in step) more items beat more re-use:
     // 24^3 at ZT = 1 has 72 items per sample instead of 36 and the four layers take 132 us instead of 200 (2 windows).
-    static const int min_cols = [] { const char* e = getenv("DUNET_FLAT_MIN_COLS"); return e ? atoi(e) : 160; }();
     int zt = 0;
     for (int cand : {1, 2, 3, 4, 6})
-      if (cand * npos <= 512 && cand <= Dl && Dl % cand == 0 && cand * npos >= min_cols) { zt = cand; break; }
-    if (!zt) {  // min_cols out of reach: the largest feasible slab count
+      if (cand * npos <= 512 && cand <= Dl && Dl % cand == 0 && cand * npos >= 160) { zt = cand; break; }
+    if (!zt) {  // 160 columns out of reach: the largest feasible slab count
       zt = 1;
       for (int cand : {2, 3, 4, 6}) if (cand * npos <= 512 && cand <= Dl && Dl % cand == 0) zt = cand;
     }
@@ -504,12 +481,11 @@ static ConvGeom conv_geom(const dunet_plan* p, const ConvW& c, int lvl, int B) {
       const int items1 = g.tiles * c.n_tiles;
       g.ksplit = 1;
       g.ksub = 1;
-      if (items1 < flat_split_items) {
+      if (items1 < 36) {
         // K is split in units of 64-channel blocks; when a sample still has too few items, in units of one tz slice of a
         // block (9 taps), up to 16 ways
-        const int want = (flat_target_items + items1 - 1) / items1;
-        static const bool tz_split = [] { const char* e = getenv("DUNET_FLAT_TZ_SPLIT"); return !(e && e[0] == '0'); }();
-        if (want > ncb && tz_split) { g.ksub = 3; g.ksplit = std::max(1, std::min(std::min(3 * ncb, 16), want)); }
+        const int want = (48 + items1 - 1) / items1;
+        if (want > ncb) { g.ksub = 3; g.ksplit = std::max(1, std::min(std::min(3 * ncb, 16), want)); }
         else g.ksplit = std::max(1, std::min(ncb, want));
       }
     }
@@ -585,7 +561,6 @@ static WsLayout ws_layout(const dunet_plan* p, int B) {
   const int CP = p->C <= 8 ? 8 : (p->C <= 16 ? 16 : 32);  // voxel-major DDIM state, classes padded to the MMA column tiles
   L.x_t = take((size_t)B * CP * p->V[0] * sizeof(float));
   L.acc = take((size_t)B * CP * p->V[0] * sizeof(float));
-  L.acc2 = take((size_t)B * CP * p->V[0] * sizeof(float));  // second accumulator of the pipelined window loop
   L.image = take((size_t)B * p->cfg.in_channels * p->V[0] * sizeof(float));  // cropped windows (dunet_infer_windows)
   for (int l = 0; l < 5; ++l) {
     L.emb[l] = take(act(p->fp[l], l));
@@ -710,8 +685,7 @@ static bool conv_can_fuse_input(const dunet_plan* p, const ConvW& c, int lvl, in
 // With `pending_split` a K-split conv of a small level may leave its fp32 partial tiles un-reduced (*pending_split = ksplit):
 // the caller's run_norm then sums, normalises and activates them in one launch (splitk_norm_kernel).
 static bool splitk_norm_ok(const dunet_plan* p, bool prec, int lvl) {
-  static const bool on = [] { const char* e = getenv("DUNET_FUSED_SPLITK_NORM"); return !(e && e[0] == '0'); }();
-  return on && !prec && p->V[lvl] <= SKN_MAX_VOX && p->D[lvl] % 2 == 0 && p->H[lvl] % 2 == 0 && p->W[lvl] % 2 == 0;
+  return !prec && p->V[lvl] <= SKN_MAX_VOX && p->D[lvl] % 2 == 0 && p->H[lvl] % 2 == 0 && p->W[lvl] % 2 == 0;
 }
 static int run_conv(const dunet_plan* p, const ConvW& c, Act src0, Act src1, Act out, float* partial, float* splitk,
                     int* nseg_out, int lvl, int B, cudaStream_t st, const FuseIn* fuse = nullptr, int* pending_split = nullptr) {
@@ -896,10 +870,9 @@ static int run_norm(const dunet_plan* p, const ConvW& c, Act raw, const float* p
     TRY(prof_end(st));
     return 0;
   }
-  // ~4 resident blocks per SM in total, each streaming a long contiguous range of one 8-channel plane (the
+  // 8 blocks per SM in total (2 to 32 measured slower), each streaming a long contiguous range of one 8-channel plane (the
   // statistics prologue is paid once per block)
-  static const int norm_grid = [] { const char* e = getenv("DUNET_NORM_GRID"); return e ? atoi(e) : 8; }();  // blocks per SM (A/B timing)
-  const int per_plane = std::max(1, (148 * norm_grid + planes - 1) / planes);
+  const int per_plane = std::max(1, (148 * 8 + planes - 1) / planes);
   // one bf16 read + one bf16 write per element (+ read of the residual, + 1/8 write of the pooled tensor); launches that move
   // less than 64 MB are launch-latency bound and are reported as their own family so that the HBM roofline of the large
   // ones stays readable
@@ -1004,10 +977,9 @@ static int run_deconv(const dunet_plan* p, const DeconvW& d, Act in, Act out, in
     if (!in.lo || !out.lo) return fail(DUNET_E_STATE, "fp32x3 transposed conv needs hi + lo tensors");
     TRY(make_act_tmap(&t[1], in.lo, B * (d.cinp / 8), D, H, W, 8, 0));
   }
-  // A/B: transposed convs with Cin >= this and a row of <= 32 voxels go to the flattened-plane kernel (default: only Cin > 128)
-  static const int flat_min_cin = [] { const char* e = getenv("DUNET_FLAT_DECONV_MIN_CIN"); return e ? atoi(e) : 129; }();
-  const bool flat_first = d.cinp >= flat_min_cin && W <= 32;
-  if (d.cinp <= 128 && !flat_first && !prec && !(p->cfg.flags & DUNET_FLAG_GENERIC_CONV)) {  // persistent, HBM-write-bound variant
+  // Cin <= 128: the persistent, HBM-write-bound kernel (the flattened-plane kernel measured 37 vs 19 us on the 24 -> 48
+  // up-conv, 2 windows)
+  if (d.cinp <= 128 && !prec && !(p->cfg.flags & DUNET_FLAG_GENERIC_CONV)) {
     DeconvTcArgs b;
     memset(&b, 0, sizeof b);
     b.w = d.packed_tc; b.out = out.hi; b.bias = d.bias; b.chunks_in = d.cinp / 8; b.cout = d.coutp; b.D = D; b.H = H; b.W = W;
@@ -1026,8 +998,7 @@ static int run_deconv(const dunet_plan* p, const DeconvW& d, Act in, Act out, in
     TRY(prof_end(st));
     return 0;
   }
-  static const bool flat_on = [] { const char* e = getenv("DUNET_FLAT_DECONV"); return !(e && e[0] == '0'); }();
-  if (flat_on && !prec && !(p->cfg.flags & DUNET_FLAG_GENERIC_CONV) && W <= 32) {
+  if (!prec && !(p->cfg.flags & DUNET_FLAG_GENERIC_CONV) && W <= 32) {
     // deep levels (Cin > 128): the flattened-plane kernel in transposed-conv mode (rows = (tap, cout), positions as N, no halo)
     const int hx = W, ty_max = std::max(1, 256 / hx);
     const int tiles_y = (H + ty_max - 1) / ty_max, ty = (H + tiles_y - 1) / tiles_y;
@@ -1091,10 +1062,42 @@ static int run_deconv(const dunet_plan* p, const DeconvW& d, Act in, Act out, in
   return rc;
 }
 
-// number of sub-batches a batch of B windows is split into in dual-stream mode (experiments: DUNET_NSTREAMS = 2..4)
-static int n_substreams(int B) {
-  static const int ns = [] { const char* e = getenv("DUNET_NSTREAMS"); const int v = e ? atoi(e) : 2; return v < 2 ? 2 : (v > 4 ? 4 : v); }();
-  return std::min(ns, B);
+// Sub-batches of a batch of B windows.  With DUNET_FLAG_DUAL_STREAM a batch of >= 4 windows (2-3 measured within noise)
+// runs as two half batches of B0 = ceil(B / 2) windows on the plan's internal streams.  Half h holds windows
+// [h * B0, h * B0 + nb) and the workspace part at h * ws_stride, which is laid out for nb windows (ws_layout(p, nb) of a
+// shorter last half fits in the B0-window part).  Otherwise there is one part: the whole batch and workspace.
+struct SubBatches {
+  int n, B0;
+  size_t ws_stride;
+};
+static SubBatches sub_batches(const dunet_plan* p, int B, bool dual) {
+  SubBatches s;
+  s.n = dual ? 2 : 1;
+  s.B0 = (B + s.n - 1) / s.n;
+  s.ws_stride = ws_layout(p, s.B0).total;
+  return s;
+}
+static bool dual_batch(const dunet_plan* p, int B) { return B >= 4 && (p->cfg.flags & DUNET_FLAG_DUAL_STREAM); }
+// Does this call run as two sub-batches?  Not while the profiler is on (kernel times would overlap).  A call that skips
+// the encoder must read the embeddings back through the partition they were written with.
+static bool use_dual(dunet_plan* p, int B, int run_encoder) {
+  const bool dual = run_encoder ? (dual_batch(p, B) && !PROF_ON) : (p->emb_dual && p->emb_B == B);
+  if (run_encoder) { p->emb_B = B; p->emb_dual = dual; }
+  return dual;
+}
+// body(b0, nb, ws_h, stream_h) for every sub-batch: one part runs on the caller's stream; two parts are forked from the
+// caller's stream onto half_stream[h] and joined back into it with events (device-side waits, no host synchronisation)
+template <typename Body>
+static int run_sub_batches(dunet_plan* p, const SubBatches& s, int B, uint8_t* ws, cudaStream_t st, Body&& body) {
+  if (s.n == 1) return body(0, B, ws, st);
+  CUDA_TRY(cudaEventRecord(p->ev_fork, st));
+  for (int h = 0; h < s.n; ++h) {
+    CUDA_TRY(cudaStreamWaitEvent(p->half_stream[h], p->ev_fork, 0));
+    TRY(body(h * s.B0, std::min(s.B0, B - h * s.B0), ws + h * s.ws_stride, p->half_stream[h]));
+    CUDA_TRY(cudaEventRecord(p->ev_join[h], p->half_stream[h]));
+  }
+  for (int h = 0; h < s.n; ++h) CUDA_TRY(cudaStreamWaitEvent(st, p->ev_join[h], 0));
+  return 0;
 }
 
 static int check_call(const dunet_plan* p, int B, const void* ws) {
@@ -1102,16 +1105,6 @@ static int check_call(const dunet_plan* p, int B, const void* ws) {
   if (!p->committed) return fail(DUNET_E_STATE, "plan not committed (dunet_plan_commit)");
   if (B < 1 || B > p->cfg.batch_max) return fail(DUNET_E_INVALID, "batch %d outside [1, %d]", B, p->cfg.batch_max);
   if (!ws || (reinterpret_cast<uintptr_t>(ws) & 255u)) return fail(DUNET_E_INVALID, "workspace must be non-NULL and 256-byte aligned");
-  return 0;
-}
-
-// Work of a deferred dunet_infer_windows may still be in flight on the internal streams: every other entry point that
-// touches the workspace first makes the caller's stream wait for it (a device-side wait, no host synchronisation).
-static int drain_async(dunet_plan* p, cudaStream_t st) {
-  if (p && p->async_pending) {
-    CUDA_TRY(cudaStreamWaitEvent(st, p->ev_stitch_tail, 0));  // the stitch stream waited for every half's ev_done
-    p->async_pending = false;
-  }
   return 0;
 }
 
@@ -1182,8 +1175,8 @@ static void final_args_common(dunet_plan* p, FinalDdimArgs& a, uint8_t* ws, cons
 }
 
 static int launch_final(dunet_plan* p, const FinalDdimArgs& a, cudaStream_t st) {
-  static const int final_grid = [] { const char* e = getenv("DUNET_FINAL_GRID"); return e ? atoi(e) : 3; }();  // blocks per SM (A/B timing)
-  const dim3 grid(grid_for((a.vox + 15) / 16 * 32, FINAL_THREADS, std::max(1, 148 * final_grid / a.batch)), a.batch);
+  // 3 blocks per SM in total (2 to 32 measured slower)
+  const dim3 grid(grid_for((a.vox + 15) / 16 * 32, FINAL_THREADS, std::max(1, 148 * 3 / a.batch)), a.batch);
   if (a.F != 64 && a.F != 128) return fail(DUNET_E_UNSUPPORTED, "final conv: padded features[5] must be 64 or 128");
   const bool prec = a.feat_lo != nullptr;
 #define DUNET_FINAL(NT)                                                                            \
@@ -1381,26 +1374,18 @@ int dunet_plan_create(dunet_plan** out, const dunet_cfg* cfg) {
 
 void dunet_plan_destroy(dunet_plan* p) {
   if (!p) return;
-  // deferred window work may still be running on the internal streams: it reads the plan's weights and tables
-  for (int i = 0; i < 4; ++i)
-    if (p->half_stream[i]) cudaStreamSynchronize(p->half_stream[i]);
-  if (p->stitch_stream) cudaStreamSynchronize(p->stitch_stream);
+  // sub-batch work may still be running on the internal streams: it reads the plan's weights and tables
+  for (cudaStream_t s : p->half_stream)
+    if (s) cudaStreamSynchronize(s);
   for (void* q : p->owned) cudaFree(q);
   if (p->h_t) cudaFreeHost(p->h_t);
   for (cudaEvent_t e : p->t_ev) if (e) cudaEventDestroy(e);
   for (ProfRec& r : p->prof.recs) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
-  for (int i = 0; i < 4; ++i) {
+  for (int i = 0; i < 2; ++i) {
     if (p->half_stream[i]) cudaStreamDestroy(p->half_stream[i]);
     if (p->ev_join[i]) cudaEventDestroy(p->ev_join[i]);
   }
   if (p->ev_fork) cudaEventDestroy(p->ev_fork);
-  if (p->stitch_stream) cudaStreamDestroy(p->stitch_stream);
-  if (p->ev_stitch_tail) cudaEventDestroy(p->ev_stitch_tail);
-  for (int i = 0; i < 4; ++i) {
-    if (p->ev_done[i]) cudaEventDestroy(p->ev_done[i]);
-    for (int f = 0; f < 2; ++f)
-      if (p->ev_stitched[i][f]) cudaEventDestroy(p->ev_stitched[i][f]);
-  }
   delete p;
 }
 
@@ -1536,17 +1521,11 @@ int dunet_plan_commit(dunet_plan* p, void* stream) {
     for (int i = 0; i < dunet_plan::T_RING; ++i) CUDA_TRY(cudaEventCreateWithFlags(&p->t_ev[i], cudaEventDisableTiming));
   }
   if (!p->half_stream[0]) {
-    for (int i = 0; i < 4; ++i) {
+    for (int i = 0; i < 2; ++i) {
       CUDA_TRY(cudaStreamCreateWithFlags(&p->half_stream[i], cudaStreamNonBlocking));
       CUDA_TRY(cudaEventCreateWithFlags(&p->ev_join[i], cudaEventDisableTiming));
     }
     CUDA_TRY(cudaEventCreateWithFlags(&p->ev_fork, cudaEventDisableTiming));
-    CUDA_TRY(cudaStreamCreateWithFlags(&p->stitch_stream, cudaStreamNonBlocking));
-    CUDA_TRY(cudaEventCreateWithFlags(&p->ev_stitch_tail, cudaEventDisableTiming));
-    for (int i = 0; i < 4; ++i) {
-      CUDA_TRY(cudaEventCreateWithFlags(&p->ev_done[i], cudaEventDisableTiming));
-      for (int f = 0; f < 2; ++f) CUDA_TRY(cudaEventCreateWithFlags(&p->ev_stitched[i][f], cudaEventDisableTiming));
-    }
   }
   CUDA_TRY(cudaStreamSynchronize(st));  // host vector above must outlive the copy; commit is a setup-time call
   p->committed = true;
@@ -1556,10 +1535,8 @@ int dunet_plan_commit(dunet_plan* p, void* stream) {
 int dunet_workspace_bytes(const dunet_plan* p, int32_t batch, size_t* out) {
   if (!p || !out) return fail(DUNET_E_INVALID, "NULL argument");
   if (batch < 1 || batch > p->cfg.batch_max) return fail(DUNET_E_INVALID, "batch %d outside [1, %d]", batch, p->cfg.batch_max);
-  const size_t single = ws_layout(p, batch).total;
-  const int ns = n_substreams(batch);
-  const size_t halves = batch >= 2 ? ns * ws_layout(p, (batch + ns - 1) / ns).total : 0;
-  *out = std::max(single, halves);
+  const SubBatches s = sub_batches(p, batch, dual_batch(p, batch));
+  *out = std::max(ws_layout(p, batch).total, s.n * s.ws_stride);
   return 0;
 }
 
@@ -1567,14 +1544,12 @@ int dunet_encode(dunet_plan* p, const float* image, int32_t B, void* workspace, 
   TRY(check_call(p, B, workspace));
   if (!image || !aligned16(image)) return fail(DUNET_E_INVALID, "image must be a 16-byte aligned device pointer");
   p->emb_B = B; p->emb_dual = false;
-  TRY(drain_async(p, static_cast<cudaStream_t>(stream)));
   return encode_impl(p, image, B, static_cast<uint8_t*>(workspace), ws_layout(p, B), static_cast<cudaStream_t>(stream));
 }
 
 int dunet_get_embedding(dunet_plan* p, int32_t level, float* out, int32_t B, void* workspace, void* stream) {
   TRY(check_call(p, B, workspace));
   if (level < 0 || level > 4 || !out) return fail(DUNET_E_INVALID, "bad level / NULL out");
-  TRY(drain_async(p, static_cast<cudaStream_t>(stream)));
   const WsLayout L = ws_layout(p, B);
   const Act e = ws_act(p, static_cast<uint8_t*>(workspace), L.emb[level], p->fp[level], level, B);
   DUNET_FMT(fmt_h(p, e.lo != nullptr), unpack_c8_kernel<HF><<<grid_for((long long)B * (p->fp[level] / 8) * p->V[level], 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
@@ -1586,7 +1561,6 @@ int dunet_get_embedding(dunet_plan* p, int32_t level, float* out, int32_t B, voi
 int dunet_set_embedding(dunet_plan* p, int32_t level, const float* in, int32_t B, void* workspace, void* stream) {
   TRY(check_call(p, B, workspace));
   if (level < 0 || level > 4 || !in) return fail(DUNET_E_INVALID, "bad level / NULL in");
-  TRY(drain_async(p, static_cast<cudaStream_t>(stream)));
   p->emb_B = B; p->emb_dual = false;
   const WsLayout L = ws_layout(p, B);
   return launch_pack(p, in, p->fr[level], nullptr, 0, ws_act(p, static_cast<uint8_t*>(workspace), L.emb[level], p->fp[level], level, B),
@@ -1598,7 +1572,6 @@ int dunet_denoise_step(dunet_plan* p, const float* x_t, const float* image, cons
   TRY(check_call(p, B, workspace));
   if (!x_t || !image || !logits_out || !t_original) return fail(DUNET_E_INVALID, "NULL tensor argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  TRY(drain_async(p, st));
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   const WsLayout L = ws_layout(p, B);
   // one timestep shared by the batch and present in the respaced schedule (the inference call): its precomputed row
@@ -1651,11 +1624,11 @@ struct NoiseSrc {
 // initialisation, the N DDIM steps.  Leaves sum_k clamp(x0_k) in ws.acc and the last sample in ws.x_t, both voxel-major.
 // per_step_stride = elements between consecutive steps in per_step_logits (the FULL batch size when halves are used).
 static int ddim_core(dunet_plan* p, const float* image, const NoiseSrc& nz, int id0, float* per_step_logits, size_t per_step_stride,
-                     int B, int run_encoder, int zero_acc, uint8_t* ws, cudaStream_t st, int acc_sel = 0) {
+                     int B, int run_encoder, int zero_acc, uint8_t* ws, cudaStream_t st) {
   const WsLayout L = ws_layout(p, B);
   const int CP = p->C <= 8 ? 8 : (p->C <= 16 ? 16 : 32);
   float* x_t = reinterpret_cast<float*>(ws + L.x_t);   // voxel-major [B][vox][CP]
-  float* acc = reinterpret_cast<float*>(ws + (acc_sel ? L.acc2 : L.acc));
+  float* acc = reinterpret_cast<float*>(ws + L.acc);
   if (run_encoder) TRY(encode_impl(p, image, B, ws, L, st));
   const Act in_pack = ws_act(p, ws, L.in_pack, p->in_pad, 0, B);
   for (int b0 = 0; b0 < B; b0 += INIT_MAX_B) {  // x_t = noise, acc = 0, first conv input = [noise, image] in one pass
@@ -1716,15 +1689,6 @@ static int ddim_sample_impl(dunet_plan* p, const float* image, const float* nois
   return 0;
 }
 
-// does this call run as sub-batches on the plan's internal streams?
-static bool use_dual(dunet_plan* p, int B, int run_encoder) {
-  static const int dual_min = [] { const char* e = getenv("DUNET_DUAL_MIN"); return e ? atoi(e) : 4; }();
-  const bool dual = run_encoder ? (B >= dual_min && B >= 2 && (p->cfg.flags & DUNET_FLAG_DUAL_STREAM) && !PROF_ON)
-                                : (p->emb_dual && p->emb_B == B);
-  if (run_encoder) { p->emb_B = B; p->emb_dual = dual; }
-  return dual;
-}
-
 int dunet_ddim_sample(dunet_plan* p, const float* image, const float* noise, float* acc_out, float* per_step_logits,
                       float* final_x, int32_t B, int32_t run_encoder, float out_scale, int32_t out_accumulate, void* workspace,
                       void* stream) {
@@ -1734,29 +1698,12 @@ int dunet_ddim_sample(dunet_plan* p, const float* image, const float* noise, flo
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   const size_t per_step_stride = (size_t)B * p->C * p->V[0];
-  TRY(drain_async(p, st));
-  if (!use_dual(p, B, run_encoder))
-    return ddim_sample_impl(p, image, noise, acc_out, per_step_logits, per_step_stride, final_x, B, run_encoder, out_scale,
-                            out_accumulate, ws, st);
-  // ---- two half batches on two internal streams (fork from / join into the caller's stream; no host synchronisation)
-  const int ns = n_substreams(B);
-  const int B0 = (B + ns - 1) / ns;
-  const size_t half_ws = ws_layout(p, B0).total;
-  CUDA_TRY(cudaEventRecord(p->ev_fork, st));
-  int used = 0;
-  for (int h = 0; h < ns; ++h) {
-    const int b0 = h * B0, nb = std::min(B0, B - b0);
-    if (nb <= 0) break;
+  const SubBatches s = sub_batches(p, B, use_dual(p, B, run_encoder));
+  return run_sub_batches(p, s, B, ws, st, [&](int b0, int nb, uint8_t* ws_h, cudaStream_t sh) -> int {
     const size_t img_off = (size_t)b0 * p->cfg.in_channels * p->V[0], st_off = (size_t)b0 * p->C * p->V[0];
-    CUDA_TRY(cudaStreamWaitEvent(p->half_stream[h], p->ev_fork, 0));
-    TRY(ddim_sample_impl(p, image + img_off, noise + st_off, acc_out + st_off, per_step_logits ? per_step_logits + st_off : nullptr,
-                         per_step_stride, final_x ? final_x + st_off : nullptr, nb, run_encoder, out_scale, out_accumulate,
-                         ws + h * half_ws, p->half_stream[h]));
-    CUDA_TRY(cudaEventRecord(p->ev_join[h], p->half_stream[h]));
-    ++used;
-  }
-  for (int h = 0; h < used; ++h) CUDA_TRY(cudaStreamWaitEvent(st, p->ev_join[h], 0));
-  return 0;
+    return ddim_sample_impl(p, image + img_off, noise + st_off, acc_out + st_off, per_step_logits ? per_step_logits + st_off : nullptr,
+                            per_step_stride, final_x ? final_x + st_off : nullptr, nb, run_encoder, out_scale, out_accumulate, ws_h, sh);
+  });
 }
 
 static int check_box(const int32_t v[3], const int32_t pd[3], const int32_t s[3]) {
@@ -1807,7 +1754,7 @@ int dunet_crop_windows(const float* volume, const int32_t v[3], float* patches, 
 
 int dunet_infer_windows(dunet_plan* p, const float* volume, const int32_t v[3], const int32_t* starts, int32_t B,
                         const float* noise, uint64_t seed, const int64_t* noise_ids, int32_t ensemble, float* out_volume,
-                        float* count_volume, const float* weights, int32_t deferred, void* workspace, void* stream) {
+                        float* count_volume, const float* weights, void* workspace, void* stream) {
   TRY(check_call(p, B, workspace));
   if (!volume || !v || !starts || !out_volume) return fail(DUNET_E_INVALID, "NULL argument");
   if (!noise && !noise_ids) return fail(DUNET_E_INVALID, "either noise or noise_ids must be given");
@@ -1818,90 +1765,33 @@ int dunet_infer_windows(dunet_plan* p, const float* volume, const int32_t v[3], 
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   const int32_t pd[3] = {p->D[0], p->H[0], p->W[0]};
   const int CP = p->C <= 8 ? 8 : (p->C <= 16 ? 16 : 32);
-  const bool dual = use_dual(p, B, 1);
-  const int ns = dual ? n_substreams(B) : 1;
-  const int B0 = (B + ns - 1) / ns;
-  const WsLayout L0 = ws_layout(p, B0);
-  const size_t sub_ws = dual ? L0.total : 0;
-  const bool pipe = dual && deferred;
-  // Work of an earlier deferred call may still be running on the internal streams.  It only has to be waited for when
-  // this call cannot simply queue behind it on the same streams with the same workspace partition.
-  if (!pipe || B0 != p->async_B0) TRY(drain_async(p, st));
-  const float scale = 1.f / (float)ensemble;
-  auto stitch = [&](int b, const float* acc_base, cudaStream_t ss) -> int {
-    const int32_t* s = starts + 3 * b;
-    if (PROF_ON) prof_of(p)->bytes[PROF_GLUE] += (double)p->V[0] * (4.0 * CP + 8.0 * p->C);
-    TRY(prof_begin(PROF_GLUE, ss));
-    launch_k(stitch_from_vm_kernel, dim3(grid_for(p->V[0], 256, 148 * 8)), dim3(256), 0, ss, out_volume, count_volume, acc_base, weights, p->C, CP,
-             v[0], v[1], v[2], pd[0], pd[1], pd[2], s[0], s[1], s[2], scale);
-    LAUNCH_CHECK();
-    TRY(prof_end(ss));
-    return 0;
-  };
-  auto run_half = [&](int h, cudaStream_t hs, int acc_sel) -> int {
-    const int b0 = h * B0, nb = std::min(B0, B - b0);
-    const WsLayout L = ws_layout(p, nb);
-    float* image = reinterpret_cast<float*>(ws + h * sub_ws + L.image);
-    TRY(crop_batch(p, volume, v, image, pd, starts + 3 * b0, nb, hs));  // window crop: one launch per sub-batch
+  const SubBatches sb = sub_batches(p, B, use_dual(p, B, 1));
+  TRY(run_sub_batches(p, sb, B, ws, st, [&](int b0, int nb, uint8_t* ws_h, cudaStream_t sh) -> int {
+    float* image = reinterpret_cast<float*>(ws_h + ws_layout(p, nb).image);
+    TRY(crop_batch(p, volume, v, image, pd, starts + 3 * b0, nb, sh));  // window crop: one launch per sub-batch
     for (int r = 0; r < ensemble; ++r) {  // BASELINE config 4: R independent noise draws, summed; the encoder runs once
       NoiseSrc nz;
       nz.given = noise ? noise + ((size_t)r * B + b0) * p->C * p->V[0] : nullptr;
       nz.seed = seed; nz.ids = noise_ids; nz.draw = r;
-      TRY(ddim_core(p, image, nz, b0, nullptr, 0, nb, r == 0, r == 0, ws + h * sub_ws, hs, acc_sel));
+      TRY(ddim_core(p, image, nz, b0, nullptr, 0, nb, r == 0, r == 0, ws_h, sh));
     }
     return 0;
-  };
-  auto acc_of = [&](int h, int j, int acc_sel) -> const float* {
-    const int nb = std::min(B0, B - h * B0);
-    const WsLayout L = ws_layout(p, nb);
-    return reinterpret_cast<const float*>(ws + h * sub_ws + (acc_sel ? L.acc2 : L.acc)) + (size_t)j * p->V[0] * CP;
-  };
-  if (!dual) {
-    TRY(run_half(0, st, 0));
-    for (int b = 0; b < B; ++b) TRY(stitch(b, acc_of(0, b, 0), st));  // MONAI's window order: fp32 sums in the oracle's order
-    return 0;
+  }));
+  // MONAI's window order on the caller's stream (fp32 sums in the oracle's order): window b is row b % B0 of the
+  // accumulator of sub-batch b / B0
+  const float scale = 1.f / (float)ensemble;
+  for (int b = 0; b < B; ++b) {
+    const int h = b / sb.B0, nb = std::min(sb.B0, B - h * sb.B0);
+    const float* acc = reinterpret_cast<const float*>(ws + h * sb.ws_stride + ws_layout(p, nb).acc) + (size_t)(b % sb.B0) * p->V[0] * CP;
+    const int32_t* s = starts + 3 * b;
+    if (PROF_ON) prof_of(p)->bytes[PROF_GLUE] += (double)p->V[0] * (4.0 * CP + 8.0 * p->C);
+    TRY(prof_begin(PROF_GLUE, st));
+    launch_k(stitch_from_vm_kernel, dim3(grid_for(p->V[0], 256, 148 * 8)), dim3(256), 0, st, out_volume, count_volume, acc, weights, p->C, CP,
+             v[0], v[1], v[2], pd[0], pd[1], pd[2], s[0], s[1], s[2], scale);
+    LAUNCH_CHECK();
+    TRY(prof_end(st));
   }
-  CUDA_TRY(cudaEventRecord(p->ev_fork, st));
-  if (!pipe) {
-    // sub-batches on the internal streams, joined back into the caller's stream before the stitching
-    for (int h = 0; h < ns && h * B0 < B; ++h) {
-      CUDA_TRY(cudaStreamWaitEvent(p->half_stream[h], p->ev_fork, 0));
-      TRY(run_half(h, p->half_stream[h], 0));
-      CUDA_TRY(cudaEventRecord(p->ev_join[h], p->half_stream[h]));
-    }
-    for (int h = 0; h < ns && h * B0 < B; ++h) CUDA_TRY(cudaStreamWaitEvent(st, p->ev_join[h], 0));
-    for (int b = 0; b < B; ++b) TRY(stitch(b, acc_of(b / B0, b % B0, 0), st));
-    return 0;
-  }
-  // ---- deferred: nothing is joined into the caller's stream (dunet_infer_flush does that).  A half only waits for
-  // (a) the caller's earlier work (ev_fork) and (b) the stitch kernels that last read the accumulator buffer it is
-  // about to overwrite -- two calls back, so consecutive calls keep both internal streams busy without bubbles.
-  CUDA_TRY(cudaStreamWaitEvent(p->stitch_stream, p->ev_fork, 0));
-  for (int h = 0; h < ns && h * B0 < B; ++h) {
-    cudaStream_t hs = p->half_stream[h];
-    const int f = p->acc_flip[h];
-    CUDA_TRY(cudaStreamWaitEvent(hs, p->ev_fork, 0));
-    if (p->stitched_valid[h][f]) CUDA_TRY(cudaStreamWaitEvent(hs, p->ev_stitched[h][f], 0));
-    TRY(run_half(h, hs, f));
-    CUDA_TRY(cudaEventRecord(p->ev_done[h], hs));
-  }
-  for (int h = 0; h < ns && h * B0 < B; ++h) {  // halves hold contiguous window ranges: h = 0 first keeps MONAI's order
-    const int f = p->acc_flip[h], nb = std::min(B0, B - h * B0);
-    CUDA_TRY(cudaStreamWaitEvent(p->stitch_stream, p->ev_done[h], 0));
-    for (int j = 0; j < nb; ++j) TRY(stitch(h * B0 + j, acc_of(h, j, f), p->stitch_stream));
-    CUDA_TRY(cudaEventRecord(p->ev_stitched[h][f], p->stitch_stream));
-    p->stitched_valid[h][f] = true;
-    p->acc_flip[h] = f ^ 1;
-  }
-  CUDA_TRY(cudaEventRecord(p->ev_stitch_tail, p->stitch_stream));
-  p->async_pending = true;
-  p->async_B0 = B0;
   return 0;
-}
-
-int dunet_infer_flush(dunet_plan* p, void* stream) {
-  if (!p) return fail(DUNET_E_INVALID, "plan is NULL");
-  return drain_async(p, static_cast<cudaStream_t>(stream));
 }
 
 int dunet_zero(void* ptr, size_t bytes, void* stream) {

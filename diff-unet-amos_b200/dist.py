@@ -126,11 +126,9 @@ def exchange_and_finalize(buf, dst: int = 0, want_blended: bool = True):
     from .inference import StitchBuffers
 
     world = _world()
-    buf.sync()  # pipelined window work must be complete (on this stream) before the exchange reads the partial volume
     if world > 1 and buf.channels % world == 0 and buf.mode == "constant":
         mine = StitchBuffers.__new__(StitchBuffers)
         mine.vol, mine.roi, mine.mode, mine.counts, mine._finalized = buf.vol, buf.roi, buf.mode, buf.counts, False
-        mine._pending_model, mine._keepalive = None, []
         mine.channels = buf.channels // world
         mine.out = reduce_scatter_channels(buf.out)
         blended_c, binary_c, _ = mine.finalize(binary=True)
@@ -386,8 +384,6 @@ def infer_volumes_distributed(model, images: Sequence[torch.Tensor], sw_batch_si
                     buf.add_windows(model, img[0, 0], starts[a:b], seed=seed, noise_ids=range(base + a, base + b))
         if px is not None:
             # ---- fused peer-memory exchange: every rank finalizes its channels of every volume of the group
-            for buf in bufs.values():
-                buf.sync()
             px.barrier()  # all partial sums of the group are complete on every rank
             for v in range(len(grp)):
                 sources = []

@@ -44,8 +44,6 @@ class StitchBuffers:
             self.out = torch.empty((channels,) + self.vol, dtype=torch.float32, device=device)
             self.zero_()
         self._finalized = False
-        self._pending_model = None
-        self._keepalive = []
         if mode == "constant":
             self.counts = [torch.from_numpy(c).to(device) for c in axis_counts(self.vol, self.roi, overlap)]
         elif mode == "gaussian":
@@ -72,28 +70,17 @@ class StitchBuffers:
                                                      _stream()))
 
     def add_windows(self, model, volume: torch.Tensor, starts, **kw) -> None:
-        """Fused crop + encoder + DDIM + ``out[slices] += pred`` for a batch of windows (model.infer_windows), pipelined:
-        consecutive calls overlap on the library's internal streams; ``sync()`` (called by ``finalize``) joins them.  The
-        volume and any explicit noise tensors are kept alive until then."""
-        self._pending_model = model
-        self._keepalive.append((volume, kw.get("noise")))
+        """Fused crop + encoder + DDIM + ``out[slices] += pred`` for a batch of windows (model.infer_windows), ordered on the
+        current stream."""
         if self.mode == "constant":
-            model.infer_windows(volume, starts, self.out, deferred=True, **kw)
+            model.infer_windows(volume, starts, self.out, **kw)
         else:
-            model.infer_windows(volume, starts, self.out, count_volume=self.count_vol, weights=self.weights, deferred=True, **kw)
-
-    def sync(self) -> None:
-        """Order all pipelined window work of this buffer before whatever is enqueued next on the current stream."""
-        if self._pending_model is not None:
-            self._pending_model.infer_flush()
-            self._pending_model = None
-        self._keepalive.clear()
+            model.infer_windows(volume, starts, self.out, count_volume=self.count_vol, weights=self.weights, **kw)
 
     def finalize(self, binary: bool = False, argmax: bool = False):
         if self._finalized:
             raise RuntimeError("StitchBuffers.finalize() was already called: the volume has been divided by the counts")
         self._finalized = True
-        self.sync()
         b = torch.empty((self.channels,) + self.vol, dtype=torch.uint8, device=self.out.device) if binary else None
         a = torch.empty(self.vol, dtype=torch.uint8, device=self.out.device) if argmax else None
         lib = _lib.load()

@@ -502,14 +502,12 @@ class DiffUNetB200(nn.Module):
 
     def infer_windows(self, volume: torch.Tensor, starts, out_volume: torch.Tensor, *, noise: torch.Tensor = None,
                       seed: int = 0, noise_ids=None, ensemble: int = 1, count_volume: torch.Tensor = None,
-                      weights: torch.Tensor = None, deferred: bool = False) -> None:
+                      weights: torch.Tensor = None) -> None:
         """One iteration of the window loop of the sliding-window driver, fused (``dunet_infer_windows``): crop the windows
         at ``starts`` ([b, 3]) out of ``volume`` ([D, H, W] fp32, padded to >= the patch), run encoder + DDIM on them and do
         ``out_volume[:, window] += pred`` window by window.  Bit-identical to crop + forward(pred_type="ddim_sample") +
         ``out[slices] += pred`` (engine.py:173-177, models/diffusion/diffusion.py:86-102).  ``noise`` ([b, C, *patch] or
-        [R, b, C, *patch]) fixes the initial x_T; otherwise the library draws it from (seed, noise_ids[b], draw).
-        ``deferred=True`` pipelines consecutive calls (see dunet_infer_windows): volume / noise / out_volume must stay alive
-        and untouched until ``infer_flush()``."""
+        [R, b, C, *patch]) fixes the initial x_T; otherwise the library draws it from (seed, noise_ids[b], draw)."""
         if not volume.is_cuda or volume.dtype != torch.float32 or not volume.is_contiguous():
             raise RuntimeError("volume must be a contiguous fp32 CUDA tensor: the B200 path has no CPU fallback")
         b = len(starts)
@@ -534,15 +532,8 @@ class DiffUNetB200(nn.Module):
         with torch.cuda.device(volume.device):
             _lib.check(_lib.load().dunet_infer_windows(plan, _ptr(volume), _lib.i32x3(vol), st, b, _ptr(noise), ctypes.c_uint64(seed & (2 ** 64 - 1)),
                                                        ids, int(ensemble), _ptr(out_volume), _ptr(count_volume), _ptr(weights),
-                                                       1 if deferred else 0, _ptr(ws), _stream()))
+                                                       _ptr(ws), _stream()))
         rt.emb_token = None
-
-    def infer_flush(self) -> None:
-        """Make the current stream wait for all deferred ``infer_windows`` work of this model."""
-        rt = self._rt
-        if rt.plan is not None:
-            with torch.cuda.device(rt.device):
-                _lib.check(_lib.load().dunet_infer_flush(rt.plan, _stream()))
 
     # ---- the reference's Diffusion.forward dispatch (models/diffusion/diffusion.py:49-63) ------------------------
     def forward(self, image: torch.Tensor = None, x: torch.Tensor = None, step: torch.Tensor = None,

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define DUNET_VERSION 100 /* 0.1.0 */
+#define DUNET_VERSION 200 /* 0.2.0; _lib.DUNET_VERSION must match */
 
 enum {
   DUNET_OK = 0,
@@ -79,27 +79,6 @@ enum {
 
 #define DUNET_FLAG_TC64_CB64 64u /* debug / A-B timing: the Cout = 64 kernel walks 64-channel blocks with a 7-slot plane ring
                                    instead of 32-channel blocks with a 13-slot ring */
-
-/* Environment switches read once by the library (debugging / A-B timing only).  The first group changes no result; the
- * DUNET_FLAT* / DUNET_FUSED_SPLITK_NORM switches select a different (equally valid) kernel decomposition of the deep U-Net
- * levels, i.e. another fp32 summation order: results stay within the tested tolerances but are not bit-identical across
- * settings (they ARE bit-identical across batch sizes under any one setting: every rule depends on per-sample shapes only).
- *   DUNET_FLAT=0                 deep levels (row <= 30 voxels, Cout % 128 == 0) on the voxel-as-M generic kernel instead of the
- *                                swapped-operand flattened-plane kernel (csrc/conv3d_flat.cuh)
- *   DUNET_FLAT_DECONV=0          transposed convs with Cin > 128 on the generic kernel instead of the flattened-plane kernel
- *   DUNET_FLAT_DECONV_MIN_CIN=n  smallest Cin the flattened-plane kernel takes in transposed-conv mode (default 129; with 64 the
- *                                24 -> 48 up-conv moves off the persistent deconv2_tc kernel: measured 37 vs 19 us, 2 windows)
- *   DUNET_FLAT_MIN_COLS=n        smallest ZT * N accumulator columns an item may have (default 160; weight re-use vs parallelism)
- *   DUNET_FLAT_SPLIT_ITEMS=n, DUNET_FLAT_TARGET_ITEMS=n, DUNET_FLAT_TZ_SPLIT=0   split-K rule of the flattened-plane kernel
- *                                (split when a sample has < 36 items, until it has ~48; K units of one tz tap slice)
- *   DUNET_FUSED_SPLITK_NORM=0    K-split convs reduce their partial tiles in splitk_reduce_stats_kernel + a separate normalise
- *                                launch instead of the fused splitk_norm_kernel
- *   DUNET_GEOM_ZT_ITEMS=n, DUNET_GEOM_SPLIT_ITEMS=n   ZT / split-K rule of the generic kernel
- *   DUNET_NO_PDL=1      launch without programmatic stream serialization
- *   DUNET_DUAL_MIN=n    smallest batch DUNET_FLAG_DUAL_STREAM splits (default 4; 2-3 measured within noise)
- *   DUNET_NSTREAMS=2..4 number of sub-batches / internal streams used by DUNET_FLAG_DUAL_STREAM (default 2; 3 and 4 measured slower)
- *   DUNET_NORM_GRID=n, DUNET_FINAL_GRID=n   blocks per SM of the normalise / final+DDIM launches (defaults 8 / 3; 2-32 measured slower)
- *   DUNET_DBG_LAUNCH=k, DUNET_DBG_DECONV=1   which launch writes the per-CTA timeline (dunet_debug_set_conv_timeline) */
 
 typedef struct dunet_plan dunet_plan;
 
@@ -197,18 +176,11 @@ int dunet_crop_windows(const float* volume, const int32_t vol_dims[3], float* pa
  *   noise_ids  HOST [batch] stream id per window (e.g. its global index in the volume's window list); needed if noise == NULL
  *   ensemble   R >= 1 independent draws averaged (BASELINE config 4; R = 1 is the reference)
  *   weights / count_volume   both NULL: constant blend.  Otherwise MONAI mode="gaussian": out += w * pred, count += w.
- *   deferred   0: everything is ordered on `stream` when the call returns (like every other entry point).
- *              1: PIPELINED -- with DUNET_FLAG_DUAL_STREAM the sub-batches run on the plan's internal streams and the
- *              stitch kernels on a third one, none of them joined into `stream`: consecutive calls keep both sub-batch
- *              streams busy (each alternates between two accumulator buffers, so it never waits for the other half or
- *              for the stitching of its previous batch).  The caller must keep volume / noise / out_volume alive and
- *              untouched until dunet_infer_flush(plan, stream), which makes `stream` wait for all deferred work.  Other
- *              entry points of the same plan wait for deferred work by themselves.  Results are bit-identical. */
+ * With DUNET_FLAG_DUAL_STREAM the two half batches run on the plan's internal streams, forked from and joined back into
+ * `stream`; the stitching then runs on `stream` in window order.  Everything is ordered on `stream` when the call returns. */
 int dunet_infer_windows(dunet_plan* plan, const float* volume, const int32_t vol_dims[3], const int32_t* starts,
                         int32_t batch, const float* noise, uint64_t seed, const int64_t* noise_ids, int32_t ensemble,
-                        float* out_volume, float* count_volume, const float* weights, int32_t deferred, void* workspace,
-                        void* stream);
-int dunet_infer_flush(dunet_plan* plan, void* stream);
+                        float* out_volume, float* count_volume, const float* weights, void* workspace, void* stream);
 /* counts_d/h/w: device int32 arrays, number of windows covering each coordinate along that axis (the window grid is a
  * Cartesian product so count(z,y,x) = counts_d[z]*counts_h[y]*counts_w[x]).  binary/argmax_labels nullable. */
 int dunet_finalize(float* out_volume, const int32_t vol_dims[3], int32_t channels, const int32_t* counts_d,
@@ -314,7 +286,9 @@ int dunet_debug_conv_geometry(const int32_t dims[3], int32_t cin, int32_t cout, 
 
 /* tools only: when non-NULL every conv CTA writes 8 clock64 stamps to dev_buffer[cta * 8 ..] (kernel start, first MMA
  * batch issued, last MMA committed, accumulators complete, epilogue done).  PROCESS-GLOBAL debugging hook (the one
- * piece of library state that is not per plan): it applies to every plan's generic conv launches until reset. */
+ * piece of library state that is not per plan): it applies to every plan's generic conv launches until reset.
+ * DUNET_DBG_LAUNCH=k in the environment restricts the stamps to the k-th generic / flattened-plane conv launch since the hook
+ * was set; DUNET_DBG_DECONV=1 lets the persistent transposed-conv kernel write them as well.  Neither changes a result. */
 int dunet_debug_set_conv_timeline(int64_t* dev_buffer);
 
 /* Live kernel timing for bench.py's roofline, PER PLAN: when enabled, every launch this plan makes is bracketed by CUDA

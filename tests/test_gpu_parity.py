@@ -593,15 +593,21 @@ def test_uninitialised_workspace_is_never_read(S, B, precision):
 # ---------------------------------------------------------------------------------------------------------------------
 # round 2: fused window loop, library noise generator, per-sample timesteps, use_amp mapping
 # ---------------------------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("mode", ["constant", "gaussian"])
-def test_fused_window_loop_is_bit_identical_to_the_generic_driver(mode):
+@pytest.mark.parametrize("mode,vol,batch", [
+    pytest.param("constant", (48, 56, 24), 4, id="constant"),
+    pytest.param("gaussian", (48, 56, 24), 4, id="gaussian"),
+    pytest.param("constant", (32, 32, 272), 6, id="constant-ragged-halves"),
+    pytest.param("gaussian", (32, 32, 272), 6, id="gaussian-ragged-halves"),
+])
+def test_fused_window_loop_is_bit_identical_to_the_generic_driver(mode, vol, batch):
     """dunet_infer_windows (batched crop + encoder + DDIM + stitch straight from the voxel-major accumulator, sub-batches
     on two internal streams) == crop_window + forward(pred_type='ddim_sample') + `out[slices] += pred`, bit for bit, in
-    both blend modes; a ragged last batch and a volume smaller than the roi on one axis are part of the case."""
-    cout, S, vol = 3, 32, (48, 56, 24)
-    m = _build(cout, S, SMALL, batch_max=4)
+    both blend modes.  48x56x24: one batch of 4 windows (two halves of 2) on a volume smaller than the roi on one axis.
+    32x32x272: 11 windows in a batch of 6 and a ragged batch of 5, i.e. halves of 3 + 3 and then 3 + 2 in one workspace."""
+    cout, S = 3, 32
+    m = _build(cout, S, SMALL, batch_max=batch)
     image = seeded_image((1, 1) + vol).cuda()
-    n_win = len(pkg.window_starts((48, 56, 32), (S, S, S), 0.25))
+    n_win = len(pkg.window_starts(tuple(max(v, S) for v in vol), (S, S, S), 0.25))
     noise = seeded_noise((n_win, cout, S, S, S)).cuda()
     nf = lambda w, b: noise[w:w + b]
     cursor = {"w": 0}
@@ -611,8 +617,8 @@ def test_fused_window_loop_is_bit_identical_to_the_generic_driver(mode):
         cursor["w"] += b.shape[0]
         return m(image=b, pred_type=pred_type, noise=nz)
 
-    generic = pkg.sliding_window_inference(image, (S, S, S), 4, predictor, 0.25, mode=mode, pred_type="ddim_sample")
-    fused = pkg.sliding_window_inference(image, (S, S, S), 4, m, 0.25, mode=mode, noise_fn=nf, pred_type="ddim_sample")
+    generic = pkg.sliding_window_inference(image, (S, S, S), batch, predictor, 0.25, mode=mode, pred_type="ddim_sample")
+    fused = pkg.sliding_window_inference(image, (S, S, S), batch, m, 0.25, mode=mode, noise_fn=nf, pred_type="ddim_sample")
     assert fused.shape == generic.shape == (1, cout) + vol
     assert torch.equal(fused, generic)
 
@@ -835,7 +841,8 @@ def test_fused_window_loop_with_ensemble_draws():
     assert torch.isfinite(a).all() and not torch.equal(a, b)
 
 
-def test_infer_windows_argument_checks():
+def test_infer_windows_checks_arguments_and_orders_on_the_stream():
+    """Bad calls raise before any work is enqueued; a good call is complete on the caller's stream (no flush call exists)."""
     m = _build(2, 32, SMALL, batch_max=2)
     vol = torch.rand(40, 40, 40, device="cuda")
     out = torch.zeros(2, 40, 40, 40, device="cuda")
@@ -848,6 +855,5 @@ def test_infer_windows_argument_checks():
     with pytest.raises(RuntimeError, match="no CPU fallback"):
         m.infer_windows(vol.cpu(), [(0, 0, 0)], out, noise_ids=[0])
     m.infer_windows(vol, [(8, 8, 8)], out, noise_ids=[0])
-    m.infer_flush()
     torch.cuda.synchronize()
     assert float(out[:, :8].abs().sum()) == 0.0 and float(out[:, 8:40, 8:40, 8:40].abs().sum()) > 0.0

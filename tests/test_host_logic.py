@@ -94,14 +94,15 @@ def test_forward_dispatch_errors():
         pkg.model_hub("swin_unetr")
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_at_the_header_version():
     lib = _lib.load()
     header = open(os.path.join(ROOT, "include", "dunet.h")).read()
     declared = set(re.findall(r"\b(dunet_[a-z0-9_]+)\s*\(", header))
     assert declared == set(_lib.SIGNATURES), declared ^ set(_lib.SIGNATURES)
     for name in declared:
         assert hasattr(lib, name), name
-    assert lib.dunet_version() == 100
+    header_version = int(re.search(r"#define DUNET_VERSION (\d+)", header).group(1))
+    assert header_version == _lib.DUNET_VERSION == lib.dunet_version()
     assert ctypes.sizeof(_lib.DunetCfg) == 4 * 14
 
 

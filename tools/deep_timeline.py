@@ -1,7 +1,6 @@
-"""Per-CTA phase timeline (clock64 stamps) of ONE deep-level conv launch (conv3d_flat_kernel, or the generic conv3d_tc_kernel
-under DUNET_FLAT=0) inside a real batch-4 DDIM step.
+"""Per-CTA phase timeline (clock64 stamps) of ONE deep-level conv launch (conv3d_flat_kernel) inside a real batch-4 DDIM step.
 usage: DUNET_DBG_LAUNCH=k python tools/deep_timeline.py   (k-th deep-level conv launch after the warm-up call;
-per DDIM step the generic launches are, in order: down_2.a down_2.b down_3.a down_3.b down_4.a down_4.b upcat_4.a upcat_4.b
+per DDIM step the deep-level launches are, in order: down_2.a down_2.b down_3.a down_3.b down_4.a down_4.b upcat_4.a upcat_4.b
 upcat_3.a upcat_3.b; the encoder contributes 6 first: down.1.a/b, down.2.a/b, down.3.a/b)"""
 import ctypes
 import os
