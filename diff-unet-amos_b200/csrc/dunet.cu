@@ -418,21 +418,71 @@ static void add_twoconv_slots(dunet_plan* p, const std::string& pre, TwoConvW* t
 
 constexpr int CONV_ZT = 4;
 
-struct ConvGeom {
-  int tiles_x, tiles_y, tiles_z, tiles, ksplit, zt;
-  // flattened-plane kernel (conv3d_flat.cuh) selected for this layer: tiles_y x tiles_z items per (sample, cout tile)
-  bool flat = false;
-  int hx = 0, ty = 0, npos = 0, lbo = 0, a_slots = 0, w_slots = 0, flat_smem = 0, ksub = 1;
+// Geometry of the flattened-plane kernel (conv3d_flat.cuh) on a level of D x H x W voxels per sample: strips of ty rows of
+// hx = W + 2 * halo positions (N = npos of them, at most 256), zt z-slabs per work item (a divisor of D, zt * npos <= 512
+// TMEM columns), and the plane and weight rings that fit the shared memory.
+struct FlatGeom {
+  int hx = 0, ty = 0, npos = 0, lbo = 0, a_slots = 0, w_slots = 0, smem = 0, zt = 0, tiles_y = 0, tiles_z = 0;
+};
+// 3x3x3 conv: halo 1, >= 160 accumulator columns, a plane ring of 2 x (zt + 2) slots.  Transposed conv: halo 0, >= 128
+// columns, 3 x zt slots.  False (g untouched) when the row does not fit one TMA box (hx > 32) or the weight ring would get
+// fewer than two slots.
+static bool flat_geom(FlatGeom* g, int D, int H, int W, int halo, int min_cols, int slots_per_plane) {
+  const int hx = W + 2 * halo;
+  if (hx > 32) return false;
+  const int ty_max = std::max(1, (256 + 2 * halo) / hx);  // the last 2 * halo positions of a strip are not outputs
+  const int tiles_y = (H + ty_max - 1) / ty_max, ty = (H + tiles_y - 1) / tiles_y;
+  const int npos = pad_to(std::max(ty * hx - 2 * halo, 1), 16);
+  // ZT: the SMALLEST slab count (dividing D) whose ZT * npos accumulator columns keep the weight stream affordable -- a
+  // 16 KB weight tile feeds ZT * npos / 2 MMA clocks; at >= 160 columns (<= ~50 B/clk/SM; measured at 24^3 with 144 CTAs
+  // streaming concurrently: no slowdown, L2 serves CTAs that walk the same tiles in step) more items beat more re-use:
+  // 24^3 at ZT = 1 has 72 items per sample instead of 36 and the four layers take 132 us instead of 200 (2 windows).
+  int zt = 0;
+  for (int cand : {1, 2, 3, 4, 6})
+    if (cand * npos <= 512 && cand <= D && D % cand == 0 && cand * npos >= min_cols) { zt = cand; break; }
+  if (!zt) {  // min_cols out of reach: the largest feasible slab count
+    zt = 1;
+    for (int cand : {2, 3, 4, 6}) if (cand * npos <= 512 && cand <= D && D % cand == 0) zt = cand;
+  }
+  const int planes = zt + 2 * halo, lbo = (ty + 2 * halo) * hx * 16, plane_bytes = 8 * lbo;
+  const int budget = FLAT_SMEM_MAX - 1024 - 512 - FLAT_EPI_SMEM - FLAT_A_SLACK;
+  const int a_slots = std::max(planes, std::min(std::min(16, slots_per_plane * planes), (budget - 4 * FLAT_W_BYTES) / plane_bytes));
+  const int w_slots = std::min(8, (budget - a_slots * plane_bytes) / FLAT_W_BYTES);
+  if (w_slots < 2) return false;
+  g->hx = hx; g->ty = ty; g->npos = npos; g->lbo = lbo; g->a_slots = a_slots; g->w_slots = w_slots; g->zt = zt;
+  g->smem = 1024 + a_slots * plane_bytes + FLAT_A_SLACK + w_slots * FLAT_W_BYTES + FLAT_EPI_SMEM + 512;
+  g->tiles_y = tiles_y; g->tiles_z = D / zt;
+  return true;
+}
+
+enum ConvKernel {
+  CONV_REF,      // CUDA-core reference kernel (DUNET_FLAG_REF_CONV); it reads none of the tiling below
+  CONV_TC64,     // Cout = 64 z-stacked kernel (conv3d_tc64.cuh), ZT = 4, never split
+  CONV_FLAT,     // flattened-plane kernel of the deep levels (conv3d_flat.cuh)
+  CONV_GENERIC,  // generic voxel-as-M kernel (conv3d_tc.cuh)
+};
+// How one 3x3x3 conv runs: everything run_conv launches with and everything its callers size or decide from it.
+struct ConvPlan {
+  ConvKernel kernel = CONV_GENERIC;
+  int cb = 0;                                       // input-channel block of the kernel and its tensor maps
+  int zt = 0, tiles_x = 0, tiles_y = 0, tiles_z = 0;
+  int tiles = 0;                                    // work items (= statistics rows) per sample and cout tile
+  int ksplit = 1, ksub = 1;                         // K split ksplit ways, in units of 1/ksub of a 64-channel block
+  bool fuse_input = false;                          // the conv may take its input normalised on load (FuseIn)
+  FlatGeom flat;                                    // kernel == CONV_FLAT
 };
 
-// tiling + split-K decision for one conv layer at U-Net level `lvl` with batch B (deterministic: depends on shapes only)
-static ConvGeom conv_geom(const dunet_plan* p, const ConvW& c, int lvl, int B) {
-  ConvGeom g;
+// The one decision of which kernel runs a conv layer at U-Net level `lvl`, with which tiling and K split.  It depends on
+// PER-SAMPLE shapes and the plan flags only, never on the batch: a window's result is bit-identical whatever it is batched
+// with.  may_split = false never splits K (dunet_op_conv3x3x3 has no partial-tile buffers).
+static ConvPlan conv_plan(const dunet_plan* p, const ConvW& c, int lvl, bool may_split) {
+  const uint32_t flags = p->cfg.flags;
+  ConvPlan g;
+  g.cb = c.cb_ch;
   g.tiles_x = (p->W[lvl] + CONV_TX - 1) / CONV_TX;
   g.tiles_y = (p->H[lvl] + CONV_TY - 1) / CONV_TY;
   // ZT (z-slabs per work item) trades weight re-use (each streamed weight tile feeds ZT slabs) against parallelism, and
-  // split-K trades parallelism against an fp32 partial round trip + a reduce launch.  Both are decided from PER-SAMPLE
-  // shapes only (a window's result is bit-identical whatever it is batched with) and are tuned for the way the path is
+  // split-K trades parallelism against an fp32 partial round trip + a reduce launch.  Both are tuned for the way the path is
   // actually driven: 2-4 windows per launch (dual-stream half batches), so ~24+ work items per sample already fill the GPU.
   // Round 1 split K whenever a sample had < 96 items: at batch 4 that doubled the 24^3 / 12^3 launches into two waves of
   // half-K items, each still streaming its weights from L2, plus the reduce kernels (measured 0.31-0.38 of the tensor peak).
@@ -444,52 +494,57 @@ static ConvGeom conv_geom(const dunet_plan* p, const ConvW& c, int lvl, int B) {
   }
   g.tiles_z = (p->D[lvl] + g.zt - 1) / g.zt;
   g.tiles = g.tiles_x * g.tiles_y * g.tiles_z;
-  (void)B;
   const int ctas = g.tiles * c.n_tiles, ncb = c.ncb();
-  g.ksplit = 1;
-  if (ncb >= 2 && ctas < 20) g.ksplit = std::max(1, std::min(ncb, 96 / ctas));
-  // Deep levels (row of at most 30 voxels, Cout a multiple of 128): swapped-operand flattened-plane kernel.  N = positions
-  // of a (ty rows x W + 2) halo-plane strip, as many rows as fit N <= 256; ZT slabs (a divisor of D, ZT * N <= 512 TMEM
-  // columns, rule below); split-K when a sample has fewer than 36 items, until it has ~48.  Again per-sample shapes only.
-  if (!(p->cfg.flags & (DUNET_FLAG_REF_CONV | DUNET_FLAG_GENERIC_CONV)) && c.cb_ch == 64 && c.n_tile == 128 && p->W[lvl] + 2 <= 32) {
-    const int Dl = p->D[lvl], Hl = p->H[lvl];
-    const int hx = p->W[lvl] + 2, ty_max = 258 / hx;
-    const int tiles_y = (Hl + ty_max - 1) / ty_max, ty = (Hl + tiles_y - 1) / tiles_y;
-    const int npos = pad_to(std::max(ty * hx - 2, 1), 16);
-    // ZT: the SMALLEST slab count (dividing D) whose ZT * npos accumulator columns keep the weight stream affordable -- a
-    // 16 KB weight tile feeds ZT * npos / 2 MMA clocks; at >= 160 columns (<= ~50 B/clk/SM; measured at 24^3 with 144 CTAs
-    // streaming concurrently: no slowdown, L2 serves CTAs that walk the same tiles in step) more items beat more re-use:
-    // 24^3 at ZT = 1 has 72 items per sample instead of 36 and the four layers take 132 us instead of 200 (2 windows).
-    int zt = 0;
-    for (int cand : {1, 2, 3, 4, 6})
-      if (cand * npos <= 512 && cand <= Dl && Dl % cand == 0 && cand * npos >= 160) { zt = cand; break; }
-    if (!zt) {  // 160 columns out of reach: the largest feasible slab count
-      zt = 1;
-      for (int cand : {2, 3, 4, 6}) if (cand * npos <= 512 && cand <= Dl && Dl % cand == 0) zt = cand;
-    }
-    const int planes = zt + 2, lbo = (ty + 2) * hx * 16, plane_bytes = 8 * lbo;
-    const int budget = FLAT_SMEM_MAX - 1024 - 512 - FLAT_EPI_SMEM - FLAT_A_SLACK;
-    int a_slots = std::min(std::min(16, 2 * planes), (budget - 4 * FLAT_W_BYTES) / plane_bytes);
-    if (a_slots < planes) a_slots = planes;
-    const int w_slots = std::min(8, (budget - a_slots * plane_bytes) / FLAT_W_BYTES);
-    if (w_slots >= 2) {
-      g.flat = true;
-      g.hx = hx; g.ty = ty; g.npos = npos; g.lbo = lbo; g.a_slots = a_slots; g.w_slots = w_slots; g.zt = zt;
-      g.flat_smem = 1024 + a_slots * plane_bytes + FLAT_A_SLACK + w_slots * FLAT_W_BYTES + FLAT_EPI_SMEM + 512;
-      g.tiles_x = 1; g.tiles_y = tiles_y; g.tiles_z = (Dl + zt - 1) / zt;
-      g.tiles = g.tiles_y * g.tiles_z;
-      const int items1 = g.tiles * c.n_tiles;
-      g.ksplit = 1;
-      g.ksub = 1;
-      if (items1 < 36) {
-        // K is split in units of 64-channel blocks; when a sample still has too few items, in units of one tz slice of a
-        // block (9 taps), up to 16 ways
-        const int want = (48 + items1 - 1) / items1;
-        if (want > ncb) { g.ksub = 3; g.ksplit = std::max(1, std::min(std::min(3 * ncb, 16), want)); }
-        else g.ksplit = std::max(1, std::min(ncb, want));
-      }
+  if (may_split && ncb >= 2 && ctas < 20) g.ksplit = std::max(1, std::min(ncb, 96 / ctas));
+  if (flags & DUNET_FLAG_REF_CONV) {
+    g.kernel = CONV_REF;
+  } else if (flags & DUNET_FLAG_GENERIC_CONV) {
+    g.kernel = CONV_GENERIC;
+  } else if (c.coutp == 64 && g.ksplit == 1 && g.zt == CONV_ZT) {
+    g.kernel = CONV_TC64;
+    g.cb = c.cb64;
+    // normalise-on-load needs a single 16-bit source (a split-precision conv, every conv in fp32x3 mode, reads hi + lo)
+    g.fuse_input = !(flags & DUNET_FLAG_NO_FUSED_NORM) && !c.split && c.nb1 == 0;
+  } else if (c.cb_ch == 64 && c.n_tile == 128 && flat_geom(&g.flat, p->D[lvl], p->H[lvl], p->W[lvl], 1, 160, 2)) {
+    // Deep levels (row of at most 30 voxels, Cout a multiple of 128): swapped-operand flattened-plane kernel, split-K when a
+    // sample has fewer than 36 items, until it has ~48
+    g.kernel = CONV_FLAT;
+    g.zt = g.flat.zt; g.tiles_x = 1; g.tiles_y = g.flat.tiles_y; g.tiles_z = g.flat.tiles_z;
+    g.tiles = g.tiles_y * g.tiles_z;
+    const int items1 = g.tiles * c.n_tiles;
+    g.ksplit = 1;
+    if (may_split && items1 < 36) {
+      // K is split in units of 64-channel blocks; when a sample still has too few items, in units of one tz slice of a
+      // block (9 taps), up to 16 ways
+      const int want = (48 + items1 - 1) / items1;
+      if (want > ncb) { g.ksub = 3; g.ksplit = std::max(1, std::min(std::min(3 * ncb, 16), want)); }
+      else g.ksplit = std::max(1, std::min(ncb, want));
     }
   }
+  return g;
+}
+
+enum DeconvKernel {
+  DECONV_REF,      // CUDA-core reference kernel (DUNET_FLAG_REF_CONV)
+  DECONV_TC,       // persistent deconv2_tc kernel (deconv2_tc.cuh)
+  DECONV_FLAT,     // flattened-plane kernel in transposed-conv mode
+  DECONV_GENERIC,  // generic voxel-as-M kernel in MODE_DECONV2
+};
+struct DeconvPlan {
+  DeconvKernel kernel = DECONV_GENERIC;
+  FlatGeom flat;  // kernel == DECONV_FLAT
+};
+
+// The one decision of which kernel runs the k2 s2 transposed conv d on U-Net level lvl_in (its input level)
+static DeconvPlan deconv_plan(const dunet_plan* p, const DeconvW& d, int lvl_in) {
+  DeconvPlan g;
+  if (p->cfg.flags & DUNET_FLAG_REF_CONV) g.kernel = DECONV_REF;
+  else if (d.parts == 3 || (p->cfg.flags & DUNET_FLAG_GENERIC_CONV)) g.kernel = DECONV_GENERIC;
+  // Cin <= 128: the persistent, HBM-write-bound kernel (the flattened-plane kernel measured 37 vs 19 us on the 24 -> 48
+  // up-conv, 2 windows)
+  else if (d.cinp <= 128) g.kernel = DECONV_TC;
+  // deep levels (Cin > 128): the flattened-plane kernel in transposed-conv mode (rows = (tap, cout), positions as N, no halo)
+  else if (flat_geom(&g.flat, p->D[lvl_in], p->H[lvl_in], p->W[lvl_in], 0, 128, 3)) g.kernel = DECONV_FLAT;
   return g;
 }
 
@@ -544,7 +599,7 @@ static WsLayout ws_layout(const dunet_plan* p, int B) {
   size_t raw_max = 0, part_max = 0, ss_max = 0, split_max = 0;
   auto upd = [&](const ConvW& c, int lvl) {
     raw_max = std::max(raw_max, act_m(c.coutp, lvl, c.split ? 2 : 1));
-    const ConvGeom g = conv_geom(p, c, lvl, B);
+    const ConvPlan g = conv_plan(p, c, lvl, /*may_split=*/true);
     const size_t planes = (size_t)B * (c.coutp / 8);
     part_max = std::max(part_max, planes * std::max(g.tiles, 160) * 16 * sizeof(float));  // rows: tiles, reduction segments (<= 128) or persistent CTAs (<= #SMs)
     ss_max = std::max(ss_max, planes * 16 * sizeof(float));
@@ -653,6 +708,36 @@ static int launch_conv_tc64(const dunet_plan* p, const CUtensorMap (&t)[4], cons
   return 0;
 }
 
+// the flattened-plane kernel (3x3x3 conv, or transposed conv with f.deconv) on geometry g; h: fp16 storage
+static int launch_flat(const dunet_plan* p, const CUtensorMap (&t)[4], ConvFlatArgs f, const FlatGeom& g, bool h, int tag, cudaStream_t st) {
+  f.hx = g.hx; f.ty = g.ty; f.tiles_y = g.tiles_y; f.tiles_z = g.tiles_z;
+  f.npos = g.npos; f.lbo = g.lbo; f.a_slots = g.a_slots; f.w_slots = g.w_slots;
+  const long long items = (long long)f.tiles_y * f.tiles_z * f.n_tiles * f.ksplit * f.batch;
+  const unsigned grid = (unsigned)std::min<long long>(items, p->num_sms);
+  TRY(prof_begin(tag, st));
+  DUNET_FMT(h, {
+    switch (g.zt) {
+      case 1: launch_k(conv3d_flat_kernel<1, HF>, dim3(grid), dim3(FLAT_THREADS), (size_t)g.smem, st, t[0], t[1], t[2], t[3], f); break;
+      case 2: launch_k(conv3d_flat_kernel<2, HF>, dim3(grid), dim3(FLAT_THREADS), (size_t)g.smem, st, t[0], t[1], t[2], t[3], f); break;
+      case 3: launch_k(conv3d_flat_kernel<3, HF>, dim3(grid), dim3(FLAT_THREADS), (size_t)g.smem, st, t[0], t[1], t[2], t[3], f); break;
+      case 4: launch_k(conv3d_flat_kernel<4, HF>, dim3(grid), dim3(FLAT_THREADS), (size_t)g.smem, st, t[0], t[1], t[2], t[3], f); break;
+      default: launch_k(conv3d_flat_kernel<6, HF>, dim3(grid), dim3(FLAT_THREADS), (size_t)g.smem, st, t[0], t[1], t[2], t[3], f); break;
+    }
+  });
+  LAUNCH_CHECK();
+  TRY(prof_end(st));
+  return 0;
+}
+
+// tools: the timeline buffer for this generic / flattened-plane conv launch -- only the DUNET_DBG_LAUNCH-th one since the
+// buffer was set (default: every launch)
+static long long* conv_dbg_stamp() {
+  static const int target = [] { const char* e = getenv("DUNET_DBG_LAUNCH"); return e ? atoi(e) : -1; }();
+  long long* dbg = (g_conv_dbg && (target < 0 || g_conv_dbg_count == target)) ? g_conv_dbg : nullptr;
+  if (g_conv_dbg) ++g_conv_dbg_count;
+  return dbg;
+}
+
 // block list of a conv: bf16 mode [S0, S1]; fp32x3 mode [S0.hi, S1.hi | S0.lo, S1.lo | S0.hi, S1.hi] (tensor maps 0..3 =
 // S0.hi, S1.hi, S0.lo, S1.lo), matching the packed weight blocks [W.hi | W.hi | W.lo]
 static ConvSegs make_segs(int nb0, int chunks0, int nb1, int chunks1, bool prec) {
@@ -673,28 +758,23 @@ struct FuseIn {
   BiasRef bias;
 };
 
-// can conv `c` at level `lvl` take its input through the normalise-on-load path of the Cout = 64 kernel?
-static bool conv_can_fuse_input(const dunet_plan* p, const ConvW& c, int lvl, int B) {
-  if (p->cfg.flags & (DUNET_FLAG_REF_CONV | DUNET_FLAG_GENERIC_CONV | DUNET_FLAG_FP32X3 | DUNET_FLAG_NO_FUSED_NORM)) return false;
-  if (c.split || c.parts != 1 || c.coutp != 64 || c.nb1 != 0 || !c.packed64) return false;
-  const ConvGeom g = conv_geom(p, c, lvl, B);
-  return g.ksplit == 1 && g.zt == CONV_ZT;
-}
-
-// 3x3x3 conv -> raw output (bf16, or hi + lo in fp32x3 mode) + InstanceNorm partial statistics [plane][*nseg_out][16]
-// With `pending_split` a K-split conv of a small level may leave its fp32 partial tiles un-reduced (*pending_split = ksplit):
-// the caller's run_norm then sums, normalises and activates them in one launch (splitk_norm_kernel).
+// 3x3x3 conv as planned by conv_plan -> raw output (bf16, or hi + lo in fp32x3 mode) + InstanceNorm partial statistics
+// [plane][*nseg_out][16].  With `pending_split` a K-split conv of a small level may leave its fp32 partial tiles un-reduced
+// (*pending_split = ksplit): the caller's run_norm then sums, normalises and activates them in one launch (splitk_norm_kernel).
 static bool splitk_norm_ok(const dunet_plan* p, bool prec, int lvl) {
   return !prec && p->V[lvl] <= SKN_MAX_VOX && p->D[lvl] % 2 == 0 && p->H[lvl] % 2 == 0 && p->W[lvl] % 2 == 0;
 }
-static int run_conv(const dunet_plan* p, const ConvW& c, Act src0, Act src1, Act out, float* partial, float* splitk,
-                    int* nseg_out, int lvl, int B, cudaStream_t st, const FuseIn* fuse = nullptr, int* pending_split = nullptr) {
+static int run_conv(const dunet_plan* p, const ConvW& c, const ConvPlan& cp, Act src0, Act src1, Act out, float* partial,
+                    float* splitk, int* nseg_out, int lvl, int B, cudaStream_t st, const FuseIn* fuse = nullptr,
+                    int* pending_split = nullptr) {
   if (pending_split) *pending_split = 0;
   const int D = p->D[lvl], H = p->H[lvl], W = p->W[lvl];
   const int planes = B * (c.coutp / 8);
   const bool prec = c.split, pairs_in = prec && !c.triple;  // triple: one packed source tensor already holds hi, lo, hi
   if (prec && (!out.lo || (pairs_in && (!src0.lo || (c.nb1 > 0 && !src1.lo))))) return fail(DUNET_E_STATE, "split-precision conv needs hi + lo tensors");
-  if (p->cfg.flags & DUNET_FLAG_REF_CONV) {
+  if (fuse && !cp.fuse_input) return fail(DUNET_E_STATE, "normalise-on-load requested for a conv that cannot take it");
+  if (cp.ksplit > 1 && (!partial || !splitk)) return fail(DUNET_E_STATE, "K-split conv without partial-tile buffers");
+  if (cp.kernel == CONV_REF) {
     if (prec) return fail(DUNET_E_UNSUPPORTED, "DUNET_FLAG_REF_CONV and DUNET_FLAG_FP32X3 are mutually exclusive");
     if (!c.w32) return fail(DUNET_E_STATE, "DUNET_FLAG_REF_CONV needs DUNET_FLAG_KEEP_FP32_WEIGHTS");
     // the debug kernel writes only the chunks holding real output channels; padded chunks must still be zero
@@ -716,129 +796,90 @@ static int run_conv(const dunet_plan* p, const ConvW& c, Act src0, Act src1, Act
     prof_of(p)->bytes[conv_tag] += fl;
     if (conv_tag == PROF_CONV) prof_of(p)->flops += fl;
   }
-  const ConvGeom g = conv_geom(p, c, lvl, B);
-  const int want_split = (splitk && partial) ? g.ksplit : 1;
-  const bool use64 = c.packed64 && want_split == 1 && g.zt == CONV_ZT && !(p->cfg.flags & DUNET_FLAG_GENERIC_CONV);
-  const int cb = use64 ? c.cb64 : c.cb_ch;  // input-channel block of the kernel that will run
-  CUtensorMap t[4];
-  TRY(make_act_tmap(&t[0], src0.hi, B * (c.c0p / 8), D, H, W, cb / 8, 1));
+  const ConvSegs segs = make_segs(c.c0p / cp.cb, c.c0p / 8, c.c1p / cp.cb, c.c1p / 8, pairs_in);
+  auto tmap = [&](CUtensorMap* m, const bf16* base, int ch) {
+    return cp.kernel == CONV_FLAT ? make_flat_tmap(m, base, B * (ch / 8), D, H, W, cp.flat.hx, cp.flat.ty)
+                                  : make_act_tmap(m, base, B * (ch / 8), D, H, W, cp.cb / 8, 1);
+  };
+  CUtensorMap t[4];  // S0.hi, S1.hi, S0.lo, S1.lo (see make_segs); the unused ones repeat map 0
+  TRY(tmap(&t[0], src0.hi, c.c0p));
   t[1] = t[2] = t[3] = t[0];
-  if (c.nb1 > 0) TRY(make_act_tmap(&t[1], src1.hi, B * (c.c1p / 8), D, H, W, cb / 8, 1));
+  if (c.nb1 > 0) TRY(tmap(&t[1], src1.hi, c.c1p));
   if (pairs_in) {
-    TRY(make_act_tmap(&t[2], src0.lo, B * (c.c0p / 8), D, H, W, cb / 8, 1));
-    if (c.nb1 > 0) TRY(make_act_tmap(&t[3], src1.lo, B * (c.c1p / 8), D, H, W, cb / 8, 1));
+    TRY(tmap(&t[2], src0.lo, c.c0p));
+    if (c.nb1 > 0) TRY(tmap(&t[3], src1.lo, c.c1p));
   }
-  const ConvSegs segs = make_segs(c.c0p / cb, c.c0p / 8, c.c1p / cb, c.c1p / 8, pairs_in);
-  if (use64) {
-    ConvTc64Args b;
-    memset(&b, 0, sizeof b);
-    b.w = c.packed64; b.out = out.hi; b.out_lo = out.lo; b.stats = partial; b.segs = segs;
-    b.D = D; b.H = H; b.W = W; b.tiles_x = g.tiles_x; b.tiles_y = g.tiles_y; b.tiles_z = g.tiles_z; b.batch = B;
-    unsigned grid = 0;
-    if (fuse) {
-      if (c.nb1 != 0 || prec) return fail(DUNET_E_STATE, "normalise-on-load needs a single bf16 source");
-      b.in_affine = fuse->affine; b.in_bias = fuse->bias.p; b.in_bias_n_stride = fuse->bias.n_stride; b.slope = 0.1f;
-      DUNET_FMT(fmt_h(p, prec), TRY(cb == 32 ? (launch_conv_tc64<32, true, HF>(p, t, b, &grid, st, conv_tag)) : (launch_conv_tc64<64, true, HF>(p, t, b, &grid, st, conv_tag))));
-    } else {
-      DUNET_FMT(fmt_h(p, prec), TRY(cb == 32 ? (launch_conv_tc64<32, false, HF>(p, t, b, &grid, st, conv_tag)) : (launch_conv_tc64<64, false, HF>(p, t, b, &grid, st, conv_tag))));
-    }
-    if (partial) *nseg_out = (int)grid;  // one statistics row per persistent CTA and sample
-    return 0;
-  }
-  if (fuse) return fail(DUNET_E_STATE, "normalise-on-load requested for a conv outside the Cout = 64 kernel");
-  if (g.flat) {
-    // deep levels: swapped-operand flattened-plane kernel (conv3d_flat.cuh)
-    for (int i = 0; i < 4; ++i) {
-      const bf16* base = i == 0 ? src0.hi : i == 1 ? src1.hi : i == 2 ? src0.lo : src1.lo;
-      const bool used = i == 0 || (i == 1 && c.nb1 > 0) || (pairs_in && (i == 2 || c.nb1 > 0));
-      if (used) TRY(make_flat_tmap(&t[i], base, B * ((i & 1 ? c.c1p : c.c0p) / 8), D, H, W, g.hx, g.ty));
-      else t[i] = t[0];
-    }
-    ConvFlatArgs f;
-    memset(&f, 0, sizeof f);
-    f.w = c.packed; f.out = out.hi; f.out_lo = out.lo; f.segs = segs;
-    f.cout = c.coutp; f.D = D; f.H = H; f.W = W;
-    f.hx = g.hx; f.ty = g.ty; f.tiles_y = g.tiles_y; f.tiles_z = g.tiles_z; f.n_tiles = c.n_tiles; f.batch = B;
-    f.npos = g.npos; f.lbo = g.lbo; f.a_slots = g.a_slots; f.w_slots = g.w_slots;
-    f.ksplit = want_split;
-    f.ksub = want_split > 1 ? g.ksub : 1;
-    {
-      static const int target = [] { const char* e = getenv("DUNET_DBG_LAUNCH"); return e ? atoi(e) : -1; }();
-      f.dbg = (g_conv_dbg && (target < 0 || g_conv_dbg_count == target)) ? g_conv_dbg : nullptr;
-      if (g_conv_dbg) ++g_conv_dbg_count;
-    }
-    if (f.ksplit > 1) f.out_partial = splitk;
-    else f.stats = partial;
-    const long long items = (long long)g.tiles * c.n_tiles * f.ksplit * B;
-    const unsigned grid = (unsigned)std::min<long long>(items, p->num_sms);
-    TRY(prof_begin(conv_tag, st));
-    DUNET_FMT(fmt_h(p, prec), {
-      switch (g.zt) {
-        case 1: launch_k(conv3d_flat_kernel<1, HF>, dim3(grid), dim3(FLAT_THREADS), (size_t)g.flat_smem, st, t[0], t[1], t[2], t[3], f); break;
-        case 2: launch_k(conv3d_flat_kernel<2, HF>, dim3(grid), dim3(FLAT_THREADS), (size_t)g.flat_smem, st, t[0], t[1], t[2], t[3], f); break;
-        case 3: launch_k(conv3d_flat_kernel<3, HF>, dim3(grid), dim3(FLAT_THREADS), (size_t)g.flat_smem, st, t[0], t[1], t[2], t[3], f); break;
-        case 4: launch_k(conv3d_flat_kernel<4, HF>, dim3(grid), dim3(FLAT_THREADS), (size_t)g.flat_smem, st, t[0], t[1], t[2], t[3], f); break;
-        default: launch_k(conv3d_flat_kernel<6, HF>, dim3(grid), dim3(FLAT_THREADS), (size_t)g.flat_smem, st, t[0], t[1], t[2], t[3], f); break;
+  switch (cp.kernel) {
+    case CONV_TC64: {
+      if (!c.packed64) return fail(DUNET_E_STATE, "conv weights not packed for the Cout = 64 kernel");
+      ConvTc64Args b;
+      memset(&b, 0, sizeof b);
+      b.w = c.packed64; b.out = out.hi; b.out_lo = out.lo; b.stats = partial; b.segs = segs;
+      b.D = D; b.H = H; b.W = W; b.tiles_x = cp.tiles_x; b.tiles_y = cp.tiles_y; b.tiles_z = cp.tiles_z; b.batch = B;
+      unsigned grid = 0;
+      if (fuse) {
+        b.in_affine = fuse->affine; b.in_bias = fuse->bias.p; b.in_bias_n_stride = fuse->bias.n_stride; b.slope = 0.1f;
+        DUNET_FMT(fmt_h(p, prec), TRY(cp.cb == 32 ? (launch_conv_tc64<32, true, HF>(p, t, b, &grid, st, conv_tag)) : (launch_conv_tc64<64, true, HF>(p, t, b, &grid, st, conv_tag))));
+      } else {
+        DUNET_FMT(fmt_h(p, prec), TRY(cp.cb == 32 ? (launch_conv_tc64<32, false, HF>(p, t, b, &grid, st, conv_tag)) : (launch_conv_tc64<64, false, HF>(p, t, b, &grid, st, conv_tag))));
       }
-    });
-    LAUNCH_CHECK();
-    TRY(prof_end(st));
-    if (f.ksplit > 1 && pending_split && splitk_norm_ok(p, prec, lvl)) {
-      *pending_split = f.ksplit;
-      *nseg_out = 0;
-    } else if (f.ksplit > 1) {
-      const int nseg = (int)std::min<long long>(std::max<long long>((p->V[lvl] + 255) / 256, 1), 128);
-      if (PROF_ON) prof_of(p)->bytes[PROF_SPLITK] += (double)B * c.coutp * (double)p->V[lvl] * (4.0 * f.ksplit + (prec ? 4.0 : 2.0));
-      TRY(prof_begin(PROF_SPLITK, st));
-      DUNET_FMT(fmt_h(p, prec), launch_k(splitk_reduce_stats_kernel<HF>, dim3(nseg, planes), dim3(STATS_THREADS), 0, st, (const float*)splitk, f.ksplit,
-               (long long)B * c.coutp * p->V[lvl], out.hi, out.lo, partial, (long long)p->V[lvl], nseg));
-      LAUNCH_CHECK();
-      TRY(prof_end(st));
-      *nseg_out = nseg;
-    } else if (partial) {
-      *nseg_out = g.tiles;
+      if (partial) *nseg_out = (int)grid;  // one statistics row per persistent CTA and sample
+      return 0;
     }
+    case CONV_FLAT: {
+      ConvFlatArgs f;
+      memset(&f, 0, sizeof f);
+      f.w = c.packed; f.out = out.hi; f.out_lo = out.lo; f.segs = segs;
+      f.cout = c.coutp; f.D = D; f.H = H; f.W = W; f.n_tiles = c.n_tiles; f.batch = B;
+      f.ksplit = cp.ksplit; f.ksub = cp.ksub;
+      f.dbg = conv_dbg_stamp();
+      if (cp.ksplit > 1) f.out_partial = splitk;
+      else f.stats = partial;
+      TRY(launch_flat(p, t, f, cp.flat, fmt_h(p, prec), conv_tag, st));
+      break;
+    }
+    default: {  // CONV_GENERIC
+      ConvTcArgs a;
+      memset(&a, 0, sizeof a);
+      a.w = c.packed; a.out = out.hi; a.out_lo = out.lo; a.segs = segs;
+      a.cout = c.coutp; a.D = D; a.H = H; a.W = W;
+      a.tiles_x = cp.tiles_x; a.tiles_y = cp.tiles_y; a.tiles_z = cp.tiles_z; a.n_tiles = c.n_tiles; a.batch = B;
+      a.ksplit = cp.ksplit;
+      a.dbg = conv_dbg_stamp();
+      if (cp.ksplit > 1) a.out_partial = splitk;
+      else a.stats = partial;
+      int rc = 0;
+      DUNET_FMT(fmt_h(p, prec), {
+        if (c.cb_ch == 32 && c.n_tile == 64) rc = launch_conv_tc<32, 64, CONV_ZT, MODE_CONV3, HF>(p, t, a, st, conv_tag);
+        else if (c.cb_ch == 32 && c.n_tile == 128) rc = launch_conv_tc<32, 128, CONV_ZT, MODE_CONV3, HF>(p, t, a, st, conv_tag);
+        else if (c.cb_ch == 64 && c.n_tile == 64 && cp.zt == 2) rc = launch_conv_tc<64, 64, 2, MODE_CONV3, HF>(p, t, a, st, conv_tag);
+        else if (c.cb_ch == 64 && c.n_tile == 128 && cp.zt == 2) rc = launch_conv_tc<64, 128, 2, MODE_CONV3, HF>(p, t, a, st, conv_tag);
+        else if (c.cb_ch == 64 && c.n_tile == 64) rc = launch_conv_tc<64, 64, CONV_ZT, MODE_CONV3, HF>(p, t, a, st, conv_tag);
+        else if (c.cb_ch == 64 && c.n_tile == 128) rc = launch_conv_tc<64, 128, CONV_ZT, MODE_CONV3, HF>(p, t, a, st, conv_tag);
+        else rc = fail(DUNET_E_UNSUPPORTED, "no conv instantiation for cb_ch=%d n_tile=%d", c.cb_ch, c.n_tile);
+      });
+      TRY(rc);
+      break;
+    }
+  }
+  // flattened-plane and generic kernels: one statistics row per tile, or K-split partial tiles to sum
+  if (cp.ksplit == 1) {
+    if (partial) *nseg_out = cp.tiles;
     return 0;
   }
-  ConvTcArgs a;
-  memset(&a, 0, sizeof a);
-  a.w = c.packed; a.out = out.hi; a.out_lo = out.lo; a.segs = segs;
-  a.cout = c.coutp; a.D = D; a.H = H; a.W = W;
-  a.tiles_x = g.tiles_x; a.tiles_y = g.tiles_y; a.tiles_z = g.tiles_z; a.n_tiles = c.n_tiles; a.batch = B;
-  a.ksplit = want_split;
-  {  // tools: stamp only the DUNET_DBG_LAUNCH-th generic conv launch since the buffer was set (default: every launch)
-    static const int target = [] { const char* e = getenv("DUNET_DBG_LAUNCH"); return e ? atoi(e) : -1; }();
-    a.dbg = (g_conv_dbg && (target < 0 || g_conv_dbg_count == target)) ? g_conv_dbg : nullptr;
-    if (g_conv_dbg) ++g_conv_dbg_count;
-  }
-  if (a.ksplit > 1) a.out_partial = splitk;
-  else a.stats = partial;
-  int rc = 0;
-  DUNET_FMT(fmt_h(p, prec), {
-    if (c.cb_ch == 32 && c.n_tile == 64) rc = launch_conv_tc<32, 64, CONV_ZT, MODE_CONV3, HF>(p, t, a, st, conv_tag);
-    else if (c.cb_ch == 32 && c.n_tile == 128) rc = launch_conv_tc<32, 128, CONV_ZT, MODE_CONV3, HF>(p, t, a, st, conv_tag);
-    else if (c.cb_ch == 64 && c.n_tile == 64 && g.zt == 2) rc = launch_conv_tc<64, 64, 2, MODE_CONV3, HF>(p, t, a, st, conv_tag);
-    else if (c.cb_ch == 64 && c.n_tile == 128 && g.zt == 2) rc = launch_conv_tc<64, 128, 2, MODE_CONV3, HF>(p, t, a, st, conv_tag);
-    else if (c.cb_ch == 64 && c.n_tile == 64) rc = launch_conv_tc<64, 64, CONV_ZT, MODE_CONV3, HF>(p, t, a, st, conv_tag);
-    else if (c.cb_ch == 64 && c.n_tile == 128) rc = launch_conv_tc<64, 128, CONV_ZT, MODE_CONV3, HF>(p, t, a, st, conv_tag);
-    else rc = fail(DUNET_E_UNSUPPORTED, "no conv instantiation for cb_ch=%d n_tile=%d", c.cb_ch, c.n_tile);
-  });
-  TRY(rc);
-  if (a.ksplit > 1 && pending_split && splitk_norm_ok(p, prec, lvl)) {
-    *pending_split = a.ksplit;
+  if (pending_split && splitk_norm_ok(p, prec, lvl)) {
+    *pending_split = cp.ksplit;
     *nseg_out = 0;
-  } else if (a.ksplit > 1) {
-    const int nseg = (int)std::min<long long>(std::max<long long>((p->V[lvl] + 255) / 256, 1), 128);
-    if (PROF_ON) prof_of(p)->bytes[PROF_SPLITK] += (double)B * c.coutp * (double)p->V[lvl] * (4.0 * a.ksplit + (prec ? 4.0 : 2.0));
-    TRY(prof_begin(PROF_SPLITK, st));
-    DUNET_FMT(fmt_h(p, prec), launch_k(splitk_reduce_stats_kernel<HF>, dim3(nseg, planes), dim3(STATS_THREADS), 0, st, (const float*)splitk, a.ksplit,
-             (long long)B * c.coutp * p->V[lvl], out.hi, out.lo, partial, (long long)p->V[lvl], nseg));
-    LAUNCH_CHECK();
-    TRY(prof_end(st));
-    *nseg_out = nseg;
-  } else if (partial) {
-    *nseg_out = g.tiles;
+    return 0;
   }
+  const int nseg = (int)std::min<long long>(std::max<long long>((p->V[lvl] + 255) / 256, 1), 128);
+  if (PROF_ON) prof_of(p)->bytes[PROF_SPLITK] += (double)B * c.coutp * (double)p->V[lvl] * (4.0 * cp.ksplit + (prec ? 4.0 : 2.0));
+  TRY(prof_begin(PROF_SPLITK, st));
+  DUNET_FMT(fmt_h(p, prec), launch_k(splitk_reduce_stats_kernel<HF>, dim3(nseg, planes), dim3(STATS_THREADS), 0, st, (const float*)splitk, cp.ksplit,
+           (long long)B * c.coutp * p->V[lvl], out.hi, out.lo, partial, (long long)p->V[lvl], nseg));
+  LAUNCH_CHECK();
+  TRY(prof_end(st));
+  *nseg_out = nseg;
   return 0;
 }
 
@@ -923,9 +964,9 @@ static int run_twoconv(const dunet_plan* p, const TwoConvW& t, Act src0, Act src
   float* partial = reinterpret_cast<float*>(ws + L.partial);
   float* splitk = reinterpret_cast<float*>(ws + L.splitk);
   int nseg = 0, ps_a = 0;
-  const bool b_fuses = conv_can_fuse_input(p, t.b, lvl, B);
-  TRY(run_conv(p, t.a, src0, src1, raw_a, partial, splitk, &nseg, lvl, B, st, nullptr, b_fuses ? nullptr : &ps_a));
-  if (b_fuses) {
+  const ConvPlan pa = conv_plan(p, t.a, lvl, /*may_split=*/true), pb = conv_plan(p, t.b, lvl, /*may_split=*/true);
+  TRY(run_conv(p, t.a, pa, src0, src1, raw_a, partial, splitk, &nseg, lvl, B, st, nullptr, pb.fuse_input ? nullptr : &ps_a));
+  if (pb.fuse_input) {
     // conv_1 normalises conv_0's raw output on load: only the affine map is materialised.  conv_1 writes its own raw
     // output to ws.mid (ws.raw is still being read) -- callers get the buffer through *raw_out.
     float* affine = reinterpret_cast<float*>(ws + L.affine);
@@ -938,7 +979,7 @@ static int run_twoconv(const dunet_plan* p, const TwoConvW& t, Act src0, Act src
     FuseIn f;
     f.affine = affine; f.bias = temb_bias;
     const Act raw_b2 = ws_act_x(p, ws, L.mid, t.b.coutp, lvl, B, tp);
-    TRY(run_conv(p, t.b, raw_a, Act(), raw_b2, partial, splitk, &nseg, lvl, B, st, &f));
+    TRY(run_conv(p, t.b, pb, raw_a, Act(), raw_b2, partial, splitk, &nseg, lvl, B, st, &f));
     if (raw_out) *raw_out = raw_b2;
     if (defer_last_norm) {
       *nseg_out = nseg;
@@ -950,7 +991,7 @@ static int run_twoconv(const dunet_plan* p, const TwoConvW& t, Act src0, Act src
   if (raw_out) *raw_out = raw_b;
   int ps = 0;  // K-split partial tiles left for the normalise pass (deep levels, see run_conv)
   TRY(run_norm(p, t.a, raw_a, partial, nseg, temb_bias, Act(), mid, Act(), lvl, B, st, ps_a, splitk));
-  TRY(run_conv(p, t.b, mid, Act(), raw_b, partial, splitk, &nseg, lvl, B, st, nullptr, (defer_last_norm || raw_out) ? nullptr : &ps));
+  TRY(run_conv(p, t.b, pb, mid, Act(), raw_b, partial, splitk, &nseg, lvl, B, st, nullptr, (defer_last_norm || raw_out) ? nullptr : &ps));
   if (defer_last_norm) {
     *nseg_out = nseg;
     return 0;
@@ -961,7 +1002,8 @@ static int run_twoconv(const dunet_plan* p, const TwoConvW& t, Act src0, Act src
 
 static int run_deconv(const dunet_plan* p, const DeconvW& d, Act in, Act out, int lvl_in, int B, cudaStream_t st) {
   const bool prec = d.parts == 3;
-  if (p->cfg.flags & DUNET_FLAG_REF_CONV) {  // CUDA-core debug kernel
+  const DeconvPlan dp = deconv_plan(p, d, lvl_in);
+  if (dp.kernel == DECONV_REF) {  // CUDA-core debug kernel
     if (prec) return fail(DUNET_E_UNSUPPORTED, "DUNET_FLAG_REF_CONV and DUNET_FLAG_FP32X3 are mutually exclusive");
     const long long total = (long long)B * (d.coutp / 8) * 8 * p->V[lvl_in];
     DUNET_FMT(fmt_h(p, prec), deconv2_kernel<HF><<<grid_for(total, 256, 148 * 32), 256, 0, st>>>(in.hi, d.cinp, d.packed, d.bias, out.hi, d.coutp,
@@ -969,97 +1011,62 @@ static int run_deconv(const dunet_plan* p, const DeconvW& d, Act in, Act out, in
     LAUNCH_CHECK();
     return 0;
   }
+  if (prec && (!in.lo || !out.lo)) return fail(DUNET_E_STATE, "fp32x3 transposed conv needs hi + lo tensors");
   const int D = p->D[lvl_in], H = p->H[lvl_in], W = p->W[lvl_in];
+  // like the normalise launches: below 64 MB a launch is latency bound and is reported as its own family
+  const double dbytes = (prec ? 2.0 : 1.0) * B * (double)p->V[lvl_in] * 2.0 * (d.cinp + 8.0 * d.coutp);
+  const int dtag = dbytes >= 64e6 ? PROF_DECONV : PROF_DECONV_SMALL;
+  if (PROF_ON) prof_of(p)->bytes[dtag] += dbytes;
   CUtensorMap t[4];
-  TRY(make_act_tmap(&t[0], in.hi, B * (d.cinp / 8), D, H, W, 8, 0));
-  t[1] = t[2] = t[3] = t[0];
-  if (prec) {
-    if (!in.lo || !out.lo) return fail(DUNET_E_STATE, "fp32x3 transposed conv needs hi + lo tensors");
-    TRY(make_act_tmap(&t[1], in.lo, B * (d.cinp / 8), D, H, W, 8, 0));
-  }
-  // Cin <= 128: the persistent, HBM-write-bound kernel (the flattened-plane kernel measured 37 vs 19 us on the 24 -> 48
-  // up-conv, 2 windows)
-  if (d.cinp <= 128 && !prec && !(p->cfg.flags & DUNET_FLAG_GENERIC_CONV)) {
-    DeconvTcArgs b;
-    memset(&b, 0, sizeof b);
-    b.w = d.packed_tc; b.out = out.hi; b.bias = d.bias; b.chunks_in = d.cinp / 8; b.cout = d.coutp; b.D = D; b.H = H; b.W = W;
-    b.tiles_x = (W + CONV_TX - 1) / CONV_TX; b.tiles_y = (H + CONV_TY - 1) / CONV_TY; b.tiles_z = (D + 1) / 2;
-    b.n_tiles = 8 * d.coutp / 128; b.batch = B; b.dbg = getenv("DUNET_DBG_DECONV") ? g_conv_dbg : nullptr;
-    const long long tiles = (long long)b.tiles_x * b.tiles_y * b.tiles_z * B;
-    const unsigned grid = (unsigned)std::min<long long>(tiles, p->num_sms);
-    // like the normalise launches: below 64 MB a launch is latency bound and is reported as its own family
-    const double dbytes = (double)B * (double)p->V[lvl_in] * 2.0 * (d.cinp + 8.0 * d.coutp);
-    const int dtag = dbytes >= 64e6 ? PROF_DECONV : PROF_DECONV_SMALL;
-    if (PROF_ON) prof_of(p)->bytes[dtag] += dbytes;
-    TRY(prof_begin(dtag, st));
-    if (d.cinp == 64) DUNET_FMT(is_fp16(p), launch_k(deconv2_tc_kernel<1, 2, HF>, dim3(grid), dim3(DeconvTc<1, 2>::THREADS), DeconvTc<1, 2>::SMEM_BYTES, st, t[0], b));
-    else DUNET_FMT(is_fp16(p), launch_k(deconv2_tc_kernel<2, 2, HF>, dim3(grid), dim3(DeconvTc<2, 2>::THREADS), DeconvTc<2, 2>::SMEM_BYTES, st, t[0], b));
-    LAUNCH_CHECK();
-    TRY(prof_end(st));
-    return 0;
-  }
-  if (!prec && !(p->cfg.flags & DUNET_FLAG_GENERIC_CONV) && W <= 32) {
-    // deep levels (Cin > 128): the flattened-plane kernel in transposed-conv mode (rows = (tap, cout), positions as N, no halo)
-    const int hx = W, ty_max = std::max(1, 256 / hx);
-    const int tiles_y = (H + ty_max - 1) / ty_max, ty = (H + tiles_y - 1) / tiles_y;
-    const int npos = pad_to(ty * hx, 16);
-    int zt = 0;
-    for (int cand : {1, 2, 3, 4, 6}) if (cand * npos <= 512 && cand <= D && D % cand == 0 && cand * npos >= 128) { zt = cand; break; }
-    if (!zt) { zt = 1; for (int cand : {2, 3, 4, 6}) if (cand * npos <= 512 && cand <= D && D % cand == 0) zt = cand; }
-    const int lbo = ty * hx * 16, plane_bytes = 8 * lbo;
-    const int budget = FLAT_SMEM_MAX - 1024 - 512 - FLAT_EPI_SMEM - FLAT_A_SLACK;
-    const int a_slots = std::max(zt, std::min(std::min(16, 3 * zt), (budget - 4 * FLAT_W_BYTES) / plane_bytes));
-    const int w_slots = std::min(8, (budget - a_slots * plane_bytes) / FLAT_W_BYTES);
-    if (w_slots >= 2) {
-      TRY(make_flat_tmap(&t[0], in.hi, B * (d.cinp / 8), D, H, W, hx, ty, 0));
+  switch (dp.kernel) {
+    case DECONV_TC: {
+      TRY(make_act_tmap(&t[0], in.hi, B * (d.cinp / 8), D, H, W, 8, 0));
+      DeconvTcArgs b;
+      memset(&b, 0, sizeof b);
+      b.w = d.packed_tc; b.out = out.hi; b.bias = d.bias; b.chunks_in = d.cinp / 8; b.cout = d.coutp; b.D = D; b.H = H; b.W = W;
+      b.tiles_x = (W + CONV_TX - 1) / CONV_TX; b.tiles_y = (H + CONV_TY - 1) / CONV_TY; b.tiles_z = (D + 1) / 2;
+      b.n_tiles = 8 * d.coutp / 128; b.batch = B; b.dbg = getenv("DUNET_DBG_DECONV") ? g_conv_dbg : nullptr;
+      const long long tiles = (long long)b.tiles_x * b.tiles_y * b.tiles_z * B;
+      const unsigned grid = (unsigned)std::min<long long>(tiles, p->num_sms);
+      TRY(prof_begin(dtag, st));
+      if (d.cinp == 64) DUNET_FMT(is_fp16(p), launch_k(deconv2_tc_kernel<1, 2, HF>, dim3(grid), dim3(DeconvTc<1, 2>::THREADS), DeconvTc<1, 2>::SMEM_BYTES, st, t[0], b));
+      else DUNET_FMT(is_fp16(p), launch_k(deconv2_tc_kernel<2, 2, HF>, dim3(grid), dim3(DeconvTc<2, 2>::THREADS), DeconvTc<2, 2>::SMEM_BYTES, st, t[0], b));
+      LAUNCH_CHECK();
+      TRY(prof_end(st));
+      return 0;
+    }
+    case DECONV_FLAT: {
+      TRY(make_flat_tmap(&t[0], in.hi, B * (d.cinp / 8), D, H, W, dp.flat.hx, dp.flat.ty, 0));
       t[1] = t[2] = t[3] = t[0];
       ConvFlatArgs f;
       memset(&f, 0, sizeof f);
       f.w = d.packed_tc; f.out = out.hi; f.bias = d.bias; f.deconv = 1;
       f.segs = make_segs(d.cinp / 64, d.cinp / 8, 0, 0, false);
-      f.cout = d.coutp; f.D = D; f.H = H; f.W = W;
-      f.hx = hx; f.ty = ty; f.tiles_y = tiles_y; f.tiles_z = D / zt; f.n_tiles = 8 * d.coutp / 128; f.batch = B;
-      f.npos = npos; f.lbo = lbo; f.a_slots = a_slots; f.w_slots = w_slots; f.ksplit = 1; f.ksub = 1;
-      const size_t smem = 1024 + (size_t)a_slots * plane_bytes + FLAT_A_SLACK + (size_t)w_slots * FLAT_W_BYTES + FLAT_EPI_SMEM + 512;
-      const long long items = (long long)f.tiles_y * f.tiles_z * f.n_tiles * B;
-      const unsigned grid = (unsigned)std::min<long long>(items, p->num_sms);
-      const double dbytes = (double)B * (double)p->V[lvl_in] * 2.0 * (d.cinp + 8.0 * d.coutp);
-      const int dtag = dbytes >= 64e6 ? PROF_DECONV : PROF_DECONV_SMALL;
-      if (PROF_ON) prof_of(p)->bytes[dtag] += dbytes;
-      TRY(prof_begin(dtag, st));
-      DUNET_FMT(is_fp16(p), {
-        switch (zt) {
-          case 1: launch_k(conv3d_flat_kernel<1, HF>, dim3(grid), dim3(FLAT_THREADS), smem, st, t[0], t[1], t[2], t[3], f); break;
-          case 2: launch_k(conv3d_flat_kernel<2, HF>, dim3(grid), dim3(FLAT_THREADS), smem, st, t[0], t[1], t[2], t[3], f); break;
-          case 3: launch_k(conv3d_flat_kernel<3, HF>, dim3(grid), dim3(FLAT_THREADS), smem, st, t[0], t[1], t[2], t[3], f); break;
-          case 4: launch_k(conv3d_flat_kernel<4, HF>, dim3(grid), dim3(FLAT_THREADS), smem, st, t[0], t[1], t[2], t[3], f); break;
-          default: launch_k(conv3d_flat_kernel<6, HF>, dim3(grid), dim3(FLAT_THREADS), smem, st, t[0], t[1], t[2], t[3], f); break;
-        }
-      });
-      LAUNCH_CHECK();
-      TRY(prof_end(st));
-      return 0;
+      f.cout = d.coutp; f.D = D; f.H = H; f.W = W; f.n_tiles = 8 * d.coutp / 128; f.batch = B; f.ksplit = 1; f.ksub = 1;
+      return launch_flat(p, t, f, dp.flat, is_fp16(p), dtag, st);
+    }
+    default: {  // DECONV_GENERIC
+      TRY(make_act_tmap(&t[0], in.hi, B * (d.cinp / 8), D, H, W, 8, 0));
+      t[1] = t[2] = t[3] = t[0];
+      if (prec) TRY(make_act_tmap(&t[1], in.lo, B * (d.cinp / 8), D, H, W, 8, 0));
+      ConvTcArgs a;
+      memset(&a, 0, sizeof a);
+      a.w = d.packed_tc; a.out = out.hi; a.out_lo = out.lo; a.bias = d.bias;
+      // fp32x3: [in.hi | in.lo | in.hi] x [W.hi | W.hi | W.lo]
+      a.segs = make_segs(d.cinp / 64, d.cinp / 8, 0, 0, false);
+      if (prec) {
+        a.segs.n = 3; a.segs.ncb = 3 * (d.cinp / 64);
+        a.segs.s[1] = a.segs.s[0]; a.segs.s[1].tmap = 1;
+        a.segs.s[2] = a.segs.s[0];
+      }
+      a.cout = d.coutp; a.D = D; a.H = H; a.W = W;
+      a.tiles_x = (W + CONV_TX - 1) / CONV_TX; a.tiles_y = (H + CONV_TY - 1) / CONV_TY; a.tiles_z = (D + 1) / 2;
+      a.n_tiles = 8 * d.coutp / 128; a.ksplit = 1; a.batch = B; a.dbg = nullptr;
+      int rc = 0;
+      DUNET_FMT(fmt_h(p, prec), rc = launch_conv_tc<64, 128, 2, MODE_DECONV2, HF>(p, t, a, st, dtag));
+      return rc;
     }
   }
-  ConvTcArgs a;
-  memset(&a, 0, sizeof a);
-  a.w = d.packed_tc; a.out = out.hi; a.out_lo = out.lo; a.bias = d.bias;
-  // fp32x3: [in.hi | in.lo | in.hi] x [W.hi | W.hi | W.lo]
-  a.segs = make_segs(d.cinp / 64, d.cinp / 8, 0, 0, false);
-  if (prec) {
-    a.segs.n = 3; a.segs.ncb = 3 * (d.cinp / 64);
-    a.segs.s[1] = a.segs.s[0]; a.segs.s[1].tmap = 1;
-    a.segs.s[2] = a.segs.s[0];
-  }
-  a.cout = d.coutp; a.D = D; a.H = H; a.W = W;
-  a.tiles_x = (W + CONV_TX - 1) / CONV_TX; a.tiles_y = (H + CONV_TY - 1) / CONV_TY; a.tiles_z = (D + 1) / 2;
-  a.n_tiles = 8 * d.coutp / 128; a.ksplit = 1; a.batch = B; a.dbg = nullptr;
-  const double dbytes = (prec ? 2.0 : 1.0) * B * (double)p->V[lvl_in] * 2.0 * (d.cinp + 8.0 * d.coutp);
-  const int dtag = dbytes >= 64e6 ? PROF_DECONV : PROF_DECONV_SMALL;
-  if (PROF_ON) prof_of(p)->bytes[dtag] += dbytes;
-  int rc = 0;
-  DUNET_FMT(fmt_h(p, prec), rc = launch_conv_tc<64, 128, 2, MODE_DECONV2, HF>(p, t, a, st, dtag));
-  return rc;
 }
 
 // Sub-batches of a batch of B windows.  With DUNET_FLAG_DUAL_STREAM a batch of >= 4 windows (2-3 measured within noise)
@@ -2017,7 +2024,7 @@ int dunet_op_conv3x3x3(const float* src0, int32_t c0, const float* src1, int32_t
     }
   }
   int nseg_unused = 0;
-  rc = run_conv(&tmp, c, a0, a1, raw, nullptr, nullptr, &nseg_unused, 0, B, st);
+  rc = run_conv(&tmp, c, conv_plan(&tmp, c, 0, /*may_split=*/false), a0, a1, raw, nullptr, nullptr, &nseg_unused, 0, B, st);
   if (rc == 0) {
     DUNET_FMT(fp16, unpack_c8_kernel<HF><<<grid_for((long long)B * (c.coutp / 8) * vox, 256), 256, 0, st>>>(raw.hi, raw.lo, c.coutp, out, cout, vox, B));
     g_launches.fetch_add(1);
@@ -2083,11 +2090,10 @@ int dunet_debug_conv_geometry(const int32_t dims[3], int32_t cin, int32_t cout, 
   tmp.V[0] = (long long)dims[0] * dims[1] * dims[2];
   ConvW c;
   c.shape(cin, cin <= 32 ? 32 : pad_to(cin, 64), 0, 0, cout, (flags & DUNET_FLAG_FP32X3) ? 3 : 1);
-  const ConvGeom g = conv_geom(&tmp, c, 0, 1);
-  const bool tc64 = !g.flat && c.coutp == 64 && g.ksplit == 1 && g.zt == CONV_ZT && !(flags & (DUNET_FLAG_GENERIC_CONV | DUNET_FLAG_REF_CONV));
-  out[0] = g.flat ? 2 : (tc64 ? 0 : 1);
-  out[1] = g.zt; out[2] = g.tiles_x; out[3] = g.tiles_y; out[4] = g.tiles_z; out[5] = g.ksplit; out[6] = g.flat ? g.ksub : 1;
-  out[7] = g.hx; out[8] = g.ty; out[9] = g.npos; out[10] = g.a_slots; out[11] = g.w_slots; out[12] = g.flat_smem;
+  const ConvPlan g = conv_plan(&tmp, c, 0, /*may_split=*/true);  // as a layer of a plan runs it
+  out[0] = g.kernel == CONV_TC64 ? 0 : (g.kernel == CONV_FLAT ? 2 : 1);  // the reference kernel reports 1
+  out[1] = g.zt; out[2] = g.tiles_x; out[3] = g.tiles_y; out[4] = g.tiles_z; out[5] = g.ksplit; out[6] = g.ksub;
+  out[7] = g.flat.hx; out[8] = g.flat.ty; out[9] = g.flat.npos; out[10] = g.flat.a_slots; out[11] = g.flat.w_slots; out[12] = g.flat.smem;
   out[13] = g.tiles * c.n_tiles; out[14] = c.n_tiles; out[15] = c.ncb();
   return 0;
 }

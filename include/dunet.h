@@ -266,6 +266,9 @@ int dunet_dice_counts(const uint8_t* pred, const void* label, int32_t label_is_f
  * use_ref_kernel: 0 = production tcgen05 kernels, 1 = CUDA-core debug kernel, 2 = generic tcgen05 kernel only,
  * 3 / 4 = as 0 / 2 in fp32x3 mode (operands split into hi + lo bf16 pairs, see DUNET_FLAG_FP32X3),
  * 5 / 6 = as 0 / 2 with fp16 operands (DUNET_FLAG_FP16).
+ * The kernel is chosen as for a plan's layer at these dims, except that this operator never splits K: a layer that a
+ * plan runs K-split (ksplit > 1 in dunet_debug_conv_geometry) runs here unsplit -- with Cout <= 64 that can mean the
+ * z-stacked kernel where the plan runs the generic one.
  * replaces: nn.Conv3d inside MONAI Convolution (denoiser.py:56-58).  use_ref_kernel != 0 selects the debug CUDA-core
  * kernel.  Allocates its own scratch with cudaMallocAsync on `stream`. */
 int dunet_op_conv3x3x3(const float* src0, int32_t c0, const float* src1, int32_t c1, const float* weight, int32_t cout,
@@ -277,11 +280,13 @@ int dunet_op_deconv2x2x2(const float* src, int32_t cin, const float* weight, con
                          int32_t batch, const int32_t dims[3], int32_t use_ref_kernel, void* stream);
 
 /* Host-only (no CUDA call, works without a GPU): the kernel and tiling a 3x3x3 conv layer cin -> cout gets on a U-Net level of
- * dims = (D, H, W) voxels per sample under plan flags `flags`.  The decision is a function of per-sample shapes only (never of
+ * dims = (D, H, W) voxels per sample under plan flags `flags` -- the plan's own decision, read from the same function that the
+ * layer launches and the workspace size read.  The decision is a function of per-sample shapes only (never of
  * the batch), which is what keeps batching bit-transparent.  out[16] = { kernel (0 = Cout-64 z-stacked conv3d_tc64, 1 = generic
  * voxel-as-M conv3d_tc, 2 = flattened-plane conv3d_flat), zt, tiles_x, tiles_y, tiles_z, ksplit, K units per 64-channel block
  * (1 or 3), hx, ty, npos, plane-ring slots, weight-ring slots, dynamic shared memory bytes (kernel 2), work items per sample and
- * K split, cout tiles, 64-channel input blocks }.  Fields 7-12 are 0 unless kernel == 2. */
+ * K split, cout tiles, 64-channel input blocks }.  Fields 7-12 are 0 unless kernel == 2.  Under DUNET_FLAG_REF_CONV the
+ * CUDA-core kernel runs; it reports kernel 1 and the generic kernel's tiling, from which the workspace is sized. */
 int dunet_debug_conv_geometry(const int32_t dims[3], int32_t cin, int32_t cout, uint32_t flags, int32_t out[16]);
 
 /* tools only: when non-NULL every conv CTA writes 8 clock64 stamps to dev_buffer[cta * 8 ..] (kernel start, first MMA

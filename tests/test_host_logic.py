@@ -228,6 +228,10 @@ def test_deep_level_conv_geometry_known_answers():
     assert _conv_geometry((96, 96, 96), 64, 64)["kernel"] == 0
     assert _conv_geometry((48, 48, 48), 64, 128)["kernel"] == 1
     assert _conv_geometry((24, 24, 24), 128, 128, flags=_lib.DUNET_FLAG_GENERIC_CONV)["kernel"] == 1
+    # Cout = 64 with too few items per sample: a plan splits K over the generic kernel (8 tiles, 3 hi/lo input blocks);
+    # only the stand-alone dunet_op_conv3x3x3, which never splits K, runs such a layer on the z-stacked kernel
+    g = _conv_geometry((16, 16, 16), 17, 64, flags=_lib.DUNET_FLAG_FP32X3)
+    assert (g["kernel"], g["ksplit"], g["items"], g["ncb"]) == (1, 3, 8, 3)
 
 
 @pytest.mark.parametrize("cin,cout", [(64, 128), (128, 128), (256, 128), (256, 256), (512, 256), (512, 512), (1024, 1024), (96, 384)])
