@@ -11,7 +11,7 @@ from ctypes import POINTER, c_char_p, c_float, c_int32, c_int64, c_size_t, c_uin
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libdunet_b200.so")
-DUNET_VERSION = 200  # include/dunet.h: the ABI the signatures below describe
+DUNET_VERSION = 210  # include/dunet.h: the ABI the signatures below describe
 
 DUNET_FLAG_REF_CONV = 1
 DUNET_FLAG_KEEP_FP32_WEIGHTS = 2
@@ -79,6 +79,9 @@ SIGNATURES = {
     "dunet_ipc_free": (c_int32, [c_void_p]),
     "dunet_q_sample": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int64, c_uint64, c_int64, c_void_p]),
     "dunet_dice_counts": (c_int32, [c_void_p, c_void_p, c_int32, c_int32, c_int64, c_void_p, c_void_p]),
+    "dunet_hd95_workspace_bytes": (c_int32, [c_int32, POINTER(c_int32), POINTER(c_size_t)]),
+    "dunet_hd95": (c_int32, [c_void_p, c_void_p, c_int32, c_int32, POINTER(c_int32), POINTER(ctypes.c_double), c_void_p, c_void_p,
+                             c_size_t, c_void_p]),
     "dunet_op_conv3x3x3": (c_int32, [c_void_p, c_int32, c_void_p, c_int32, c_void_p, c_int32, c_void_p, c_int32, POINTER(c_int32), c_int32, c_void_p]),
     "dunet_op_deconv2x2x2": (c_int32, [c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_void_p, c_int32, POINTER(c_int32), c_int32, c_void_p]),
     "dunet_debug_conv_geometry": (c_int32, [POINTER(c_int32), c_int32, c_int32, c_uint32, POINTER(c_int32)]),

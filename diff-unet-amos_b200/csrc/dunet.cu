@@ -2,6 +2,7 @@
 // Host code here only sequences kernels on the caller's stream; all arithmetic is in the sm_100a kernels.
 #include <algorithm>
 #include <atomic>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -23,6 +24,7 @@
 #include "conv3d_flat.cuh"
 #include "deconv2_tc.cuh"
 #include "elementwise.cuh"
+#include "surface.cuh"
 
 using namespace dunet;
 typedef __nv_bfloat16 bf16;
@@ -1211,6 +1213,71 @@ static int launch_final(dunet_plan* p, const FinalDdimArgs& a, cudaStream_t st) 
   return 0;
 }
 
+// ------------------------------------------------------------------------------------------------ HD95
+// HD95 workspace: per-class state, then per voxel an int16 D-offset, an int16 envelope stack, an (int16, int16)
+// (D, H)-offset, and room for d_AB ++ d_BA (at most two fp64 per voxel).  Reused by every class.
+struct Hd95Layout {
+  size_t meta, off1, stack, off2, keys, total;
+};
+static Hd95Layout hd95_layout(const int32_t dims[3]) {
+  const size_t V = (size_t)dims[0] * dims[1] * dims[2];
+  Hd95Layout L;
+  size_t o = 0;
+  auto take = [&](size_t bytes) { const size_t at = o; o += (bytes + 255) / 256 * 256; return at; };
+  L.meta = take(sizeof(Hd95Meta));
+  L.off1 = take(V * sizeof(int16_t));
+  L.stack = take(V * sizeof(int16_t));
+  L.off2 = take(V * sizeof(int32_t));
+  L.keys = take(2 * V * sizeof(unsigned long long));
+  L.total = o;
+  return L;
+}
+static int hd95_check_dims(int32_t channels, const int32_t dims[3]) {
+  if (!dims || channels < 1) return fail(DUNET_E_INVALID, "bad argument");
+  for (int d = 0; d < 3; ++d) {
+    if (dims[d] < 1) return fail(DUNET_E_INVALID, "dims[%d] = %d must be >= 1", d, dims[d]);
+    if (dims[d] > HD_MAX_DIM) return fail(DUNET_E_UNSUPPORTED, "dims[%d] = %d exceeds %d", d, dims[d], HD_MAX_DIM);
+  }
+  return 0;
+}
+
+template <typename LabelT>
+static int hd95_class(const uint8_t* pred, const LabelT* label, const HdGeom& g, char* ws, const Hd95Layout& L, double* out,
+                      cudaStream_t st) {
+  Hd95Meta* m = reinterpret_cast<Hd95Meta*>(ws + L.meta);
+  int16_t* off1 = reinterpret_cast<int16_t*>(ws + L.off1);
+  int16_t* stack = reinterpret_cast<int16_t*>(ws + L.stack);
+  int32_t* off2 = reinterpret_cast<int32_t*>(ws + L.off2);
+  unsigned long long* keys = reinterpret_cast<unsigned long long*>(ws + L.keys);
+  const long long V = (long long)g.D * g.H * g.W;
+  auto lines = [](long long n) { return (unsigned)((n + HD_LINE_THREADS - 1) / HD_LINE_THREADS); };
+  hd95_init_kernel<<<1, 256, 0, st>>>(m);
+  LAUNCH_CHECK();
+  hd95_box_kernel<LabelT><<<grid_for(V, 256, 148 * 8), 256, 0, st>>>(pred, label, g, m);
+  LAUNCH_CHECK();
+  // d_AB: queries border(pred), sites border(label); then d_BA
+  hd95_pass_d_kernel<LabelT><<<lines((long long)g.H * g.W), HD_LINE_THREADS, 0, st>>>(label, g, m, off1);
+  LAUNCH_CHECK();
+  hd95_pass_h_kernel<<<lines((long long)g.D * g.W), HD_LINE_THREADS, 0, st>>>(g, m, off1, stack, off2);
+  LAUNCH_CHECK();
+  hd95_pass_w_kernel<uint8_t><<<lines((long long)g.D * g.H), HD_LINE_THREADS, 0, st>>>(pred, g, m, off2, stack, keys);
+  LAUNCH_CHECK();
+  hd95_pass_d_kernel<uint8_t><<<lines((long long)g.H * g.W), HD_LINE_THREADS, 0, st>>>(pred, g, m, off1);
+  LAUNCH_CHECK();
+  hd95_pass_h_kernel<<<lines((long long)g.D * g.W), HD_LINE_THREADS, 0, st>>>(g, m, off1, stack, off2);
+  LAUNCH_CHECK();
+  hd95_pass_w_kernel<LabelT><<<lines((long long)g.D * g.H), HD_LINE_THREADS, 0, st>>>(label, g, m, off2, stack, keys);
+  LAUNCH_CHECK();
+  const int sel_grid = grid_for(2 * V, 256, 148 * 8);
+  for (int pass = 0; pass < HD_RADIX_PASSES; ++pass) {
+    hd95_select_kernel<<<sel_grid, 256, 0, st>>>(m, keys, 56 - 8 * pass);
+    LAUNCH_CHECK();
+  }
+  hd95_finish_kernel<<<sel_grid, 256, 0, st>>>(m, keys, out);
+  LAUNCH_CHECK();
+  return 0;
+}
+
 // ================================================================================================== C ABI
 extern "C" {
 
@@ -1973,6 +2040,37 @@ int dunet_dice_counts(const uint8_t* pred, const void* label, int32_t label_is_f
     dice_counts_kernel<uint8_t><<<grid, 256, 0, st>>>(pred, static_cast<const uint8_t*>(label), (long long)voxels,
                                                       reinterpret_cast<unsigned long long*>(counts));
   LAUNCH_CHECK();
+  return 0;
+}
+
+int dunet_hd95_workspace_bytes(int32_t channels, const int32_t dims[3], size_t* out_bytes) {
+  TRY(hd95_check_dims(channels, dims));
+  if (!out_bytes) return fail(DUNET_E_INVALID, "out_bytes is NULL");
+  *out_bytes = hd95_layout(dims).total;
+  return 0;
+}
+
+int dunet_hd95(const uint8_t* pred, const void* label, int32_t label_is_float, int32_t channels, const int32_t dims[3],
+               const double spacing[3], double* hd95_out, void* workspace, size_t workspace_bytes, void* stream) {
+  TRY(hd95_check_dims(channels, dims));
+  if (!pred || !label || !spacing || !hd95_out || !workspace) return fail(DUNET_E_INVALID, "NULL argument");
+  if ((label_is_float && (reinterpret_cast<uintptr_t>(label) & 3u)) || (reinterpret_cast<uintptr_t>(hd95_out) & 7u))
+    return fail(DUNET_E_INVALID, "label (fp32) must be 4-byte and hd95_out 8-byte aligned");
+  if (reinterpret_cast<uintptr_t>(workspace) & 255u) return fail(DUNET_E_INVALID, "workspace must be 256-byte aligned");
+  for (int d = 0; d < 3; ++d)
+    if (!std::isfinite(spacing[d]) || !(spacing[d] > 0.0)) return fail(DUNET_E_INVALID, "spacing[%d] must be finite and > 0", d);
+  const Hd95Layout L = hd95_layout(dims);
+  if (workspace_bytes < L.total) return fail(DUNET_E_INVALID, "workspace of %zu bytes, %zu needed", workspace_bytes, L.total);
+  const HdGeom g{dims[0], dims[1], dims[2], spacing[0], spacing[1], spacing[2]};
+  const size_t V = (size_t)dims[0] * dims[1] * dims[2];
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  char* ws = static_cast<char*>(workspace);
+  for (int c = 0; c < channels; ++c) {
+    if (label_is_float)
+      TRY(hd95_class(pred + c * V, static_cast<const float*>(label) + c * V, g, ws, L, hd95_out + c, st));
+    else
+      TRY(hd95_class(pred + c * V, static_cast<const uint8_t*>(label) + c * V, g, ws, L, hd95_out + c, st));
+  }
   return 0;
 }
 

@@ -59,6 +59,38 @@ def dice_counts(pred_u8: torch.Tensor, label: torch.Tensor) -> torch.Tensor:
     return counts
 
 
+def hd95(pred_u8: torch.Tensor, label: torch.Tensor, spacing: Sequence[float] = (1.0, 1.0, 1.0)) -> list:
+    """Per-class HD95 surface distance, computed on the GPU: medpy ``hd95(pred, label, voxelspacing=spacing,
+    connectivity=1)`` for each class (the reference's medpy-based metric).  pred_u8: uint8 [C, D, H, W] in {0, 1}; label:
+    one-hot [C, D, H, W], uint8 / bool / fp32, non-zero = foreground; spacing: per array axis (D, H, W).  A class whose
+    prediction or label is empty gives NaN (medpy raises there); the other classes are unaffected."""
+    if not pred_u8.is_cuda or not label.is_cuda:
+        raise RuntimeError("hd95 runs on the GPU only (no CPU fallback)")
+    if pred_u8.dtype != torch.uint8:
+        raise TypeError("pred must be uint8")
+    if pred_u8.dim() != 4:
+        raise ValueError(f"pred must be [C, D, H, W], got {tuple(pred_u8.shape)}")
+    pred_u8 = pred_u8.contiguous()
+    if label.dtype == torch.bool:
+        label = label.to(torch.uint8)
+    if label.dtype not in (torch.uint8, torch.float32):
+        label = label.float()
+    label = label.contiguous()
+    if label.shape != pred_u8.shape:
+        raise ValueError(f"label shape {tuple(label.shape)} does not match prediction {tuple(pred_u8.shape)}")
+    C, dims = pred_u8.shape[0], _lib.i32x3(pred_u8.shape[1:])
+    lib = _lib.load()
+    nbytes = ctypes.c_size_t()
+    _lib.check(lib.dunet_hd95_workspace_bytes(C, dims, ctypes.byref(nbytes)))
+    ws = torch.empty(nbytes.value, dtype=torch.uint8, device=pred_u8.device)
+    out = torch.empty(C, dtype=torch.float64, device=pred_u8.device)
+    with torch.cuda.device(pred_u8.device):
+        _lib.check(lib.dunet_hd95(_ptr(pred_u8), _ptr(label), 1 if label.dtype == torch.float32 else 0, C, dims,
+                                  (ctypes.c_double * 3)(*[float(s) for s in spacing]), _ptr(out), _ptr(ws), nbytes.value,
+                                  _stream()))
+    return out.cpu().tolist()
+
+
 def dice_from_counts(counts: Sequence[Sequence[int]]) -> list:
     """The reference's per-class rule (test.py:143-151 + metric.py:38-47): prediction non-empty and label empty -> 1;
     otherwise 2|A&B| / (|A| + |B|), with 0/0 -> 0."""
@@ -73,9 +105,24 @@ def dice_from_counts(counts: Sequence[Sequence[int]]) -> list:
     return out
 
 
+METRICS = ("dice", "hd95")
+
+
 class EngineB200:
+    """``metrics``: "dice" (always: ``validation_step`` returns the mean Dice) and optionally "hd95", which appends one
+    ``OrderedDict`` of per-class HD95 per sample to ``self.hd95s`` (NaN for a class with an empty prediction or label);
+    ``spacing`` is the voxel spacing per array axis (D, H, W) that HD95 is measured in."""
+
     def __init__(self, model, class_names: Optional[Dict[int, str]] = None, sw_batch_size: int = 4, overlap: float = 0.25,
-                 include_background: bool = True, use_amp: Optional[bool] = None, device="cuda", epoch: Optional[int] = None):
+                 include_background: bool = True, use_amp: Optional[bool] = None, device="cuda", epoch: Optional[int] = None,
+                 metrics: Sequence[str] = ("dice",), spacing: Sequence[float] = (1.0, 1.0, 1.0)):
+        unknown = set(metrics) - set(METRICS)
+        if unknown or "dice" not in metrics:
+            raise ValueError(f"metrics must include 'dice' and be drawn from {METRICS}, got {tuple(metrics)}")
+        if len(spacing) != 3:
+            raise ValueError(f"spacing needs one value per axis (D, H, W), got {tuple(spacing)}")
+        self.metrics, self.spacing = tuple(metrics), tuple(float(s) for s in spacing)
+        self.hd95s = []
         if use_amp is not None:
             model.set_precision("fp16" if use_amp else "fp32x3")
         self.model = model.to(device).eval()
@@ -142,6 +189,9 @@ class EngineB200:
             if verbose:
                 print(f"{classes[i]} : {d:.4f}")
         self.dices.append(dices)
+        if "hd95" in self.metrics:
+            for n in range(outputs.shape[0]):  # per sample: surfaces must not mix across the batch
+                self.hd95s.append(OrderedDict(zip(classes, hd95(outputs[n], labels[n], self.spacing))))
         self.patient_index += 1
         return float(np.mean(list(dices.values())))
 

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define DUNET_VERSION 200 /* 0.2.0; _lib.DUNET_VERSION must match */
+#define DUNET_VERSION 210 /* 0.2.1; _lib.DUNET_VERSION must match */
 
 enum {
   DUNET_OK = 0,
@@ -260,6 +260,26 @@ int dunet_q_sample(const float* x_start, const float* noise_in, float* noise_out
  * (pred non-empty & label empty -> 1; both empty -> 0) are host arithmetic on these. */
 int dunet_dice_counts(const uint8_t* pred, const void* label, int32_t label_is_float, int32_t channels, int64_t voxels,
                       uint64_t* counts, void* stream);
+
+/* replaces: medpy.metric.binary.hd95(result, reference, voxelspacing, connectivity=1) per class, in the reference's
+ * medpy-based evaluation (metric module, SURVEY row 12; the call is commented out in test.py:153-158).  pred and label
+ * as in dunet_dice_counts, laid out [channels][D][H][W] with dims = (D, H, W); spacing[d] is medpy's voxelspacing of
+ * array axis d (finite, > 0).  hd95_out (device fp64 [channels]) gets per class, with A = pred, B = label:
+ *   border(M) = M ^ binary_erosion(M, 6-connected, border_value 0)   (voxels on the volume edge are border voxels);
+ *   d_AB      = distance_transform_edt(~border(B), sampling=spacing)[border(A)], d_BA likewise;
+ *   HD95      = numpy.percentile(d_AB ++ d_BA, 95), default linear method.
+ * Each distance is formed from the integer offset to the nearest site as sqrt(((s0 d0)^2 + (s1 d1)^2) + (s2 d2)^2) in fp64,
+ * as scipy forms it, and the interpolation is numpy's _lerp without FMA: the result is bit-identical to the scipy / numpy
+ * computation whenever the squared terms are exact in fp64 (e.g. spacings that are multiples of 0.25 mm).
+ * A class whose prediction or label is empty gets NaN (medpy raises); the other classes are unaffected.
+ * Workspace: dunet_hd95_workspace_bytes, 24 bytes per voxel plus 4 KB, independent of the class count (classes run one
+ * after another); 256-byte aligned.  Alignment: an fp32 label 4 bytes, hd95_out 8 bytes, pred and a uint8 label none (per-sample
+ * slices of a batch can be passed as they are).  Per class 17 kernel launches: state init, bounding box of pred ∪ label with the
+ * border counts, three separable passes per direction restricted to that box, eight radix-select passes and the
+ * percentile.  No host synchronisation.  dims must be in [1, 32767] (DUNET_E_UNSUPPORTED above). */
+int dunet_hd95_workspace_bytes(int32_t channels, const int32_t dims[3], size_t* out_bytes);
+int dunet_hd95(const uint8_t* pred, const void* label, int32_t label_is_float, int32_t channels, const int32_t dims[3],
+               const double spacing[3], double* hd95_out, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Stand-alone operator (also the unit-test seam of the tensor-core kernel): y = conv3d(cat([src0, src1]), weight),
  * 3x3x3, stride 1, zero padding 1, no bias.  fp32 NCDHW in/out, bf16 operands + fp32 accumulation inside.
