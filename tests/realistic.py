@@ -212,18 +212,19 @@ def _cast(v, dtype):
         [_cast(e, dtype) for e in v] if isinstance(v, (list, tuple)) else v
 
 
-def amp_oracle(dtype, kind, sd, *args, variant=None):
+def amp_oracle(dtype, kind, sd, *args, variant=None, num_steps=10):
     """The oracle ``kind`` with TF32 off: in fp64 (``dtype=torch.float64``, the ground truth: parameters and inputs are
     widened), in fp32 (``None``), or under ``torch.autocast("cuda", dtype)`` with torch.float16 / torch.bfloat16 like the
     reference's AMP inference (results come back as fp32).  ``variant`` ("storage" | "stats", fp64 only): the fp64 oracle with
     one of the fp32x3 mode's roundings (``_conv_in_act_fp32x3_part``), to tell which one an fp32x3 error comes from.
-    encoder(image) -> 5 maps; denoise(x, t, image, embeddings) -> logits; window(image, noise) -> DDIM-10 sum of clamp(x0)."""
+    encoder(image) -> 5 maps; denoise(x, t, image, embeddings) -> logits; window(image, noise) -> DDIM-``num_steps`` sum of
+    clamp(x0)."""
     assert variant is None or dtype == torch.float64
     if dtype == torch.float64:
         sd, args = {k: v.double() for k, v in sd.items()}, _cast(args, torch.float64)
     fn = {"encoder": lambda im: oracle_model.encoder_forward(sd, im),
           "denoise": lambda x, t, im, e: oracle_model.denoiser_forward(sd, x, t, im, e),
-          "window": lambda im, nz: oracle_window(sd, im, nz)}[kind]
+          "window": lambda im, nz: oracle_window(sd, im, nz, num_steps)}[kind]
     with torch.no_grad(), _precision(dtype, variant):
         r = fn(*args)
     return r if dtype == torch.float64 else _cast(r, torch.float32)

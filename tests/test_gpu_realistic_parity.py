@@ -55,17 +55,16 @@ def _gate(precision, err, amp_err):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-def test_encoder_all_levels_on_ct_windows():
-    """Every level of the embeddings, 96^3, default features, batch [tissue, boundary, air], per sample: fp16 (split-precision
-    encoder, rounded once to fp16) < 1e-3, bf16 within 2x of the bf16-AMP oracle, fp32x3 < 1e-4 or within 2x of the fp64
-    oracle with the fp32x3 number format (bf16 hi + lo operands, three products, raw conv outputs stored as pairs), whichever
-    is larger.  The fp64 oracle with fp32 statistics rows instead is printed next to it: which rounding the error comes from."""
-    S = 96
-    image = _images(("tissue", "boundary", "air"), S)
+def check_encoder_levels(tag, S, feats, kinds):
+    """Every level of the embeddings of the windows ``kinds`` at S^3, per sample: fp16 (split-precision encoder, rounded once
+    to fp16) < 1e-3, bf16 within 2x of the bf16-AMP oracle, fp32x3 < 1e-4 or within 2x of the fp64 oracle with the fp32x3
+    number format (bf16 hi + lo operands, three products, raw conv outputs stored as pairs), whichever is larger.  The fp64
+    oracle with fp32 statistics rows instead is printed next to it: which rounding the error comes from."""
+    image = _images(kinds, S)
     ref = None
     failed = []
     for precision in ("fp16", "bf16", "fp32x3"):
-        m, sd = _model(16, S, DEFAULT, precision)
+        m, sd = _model(16, S, feats, precision)
         if ref is None:
             ref = amp_oracle(torch.float64, "encoder", sd, image)
             amp = amp_oracle(torch.bfloat16, "encoder", sd, image)
@@ -74,9 +73,9 @@ def test_encoder_all_levels_on_ct_windows():
         with torch.no_grad():
             emb = m.embed_model(image)
         for lvl in range(5):
-            for b, kind in enumerate(("tissue", "boundary", "air")):
+            for b, kind in enumerate(kinds):
                 err = rel_l2(emb[lvl][b], ref[lvl][b])
-                line = f"encoder {precision:6s} level {lvl} {kind:8s}: rel-l2 {err:.3e}"
+                line = f"encoder {tag} {precision:6s} level {lvl} {kind:8s}: rel-l2 {err:.3e}"
                 if precision == "fp32x3":
                     fmt_err, stats_err = rel_l2(fmt[lvl][b], ref[lvl][b]), rel_l2(stats[lvl][b], ref[lvl][b])
                     line += f"  (fp32x3 format oracle {fmt_err:.3e}, fp32 statistics rows oracle {stats_err:.3e})"
@@ -97,8 +96,7 @@ def test_encoder_all_levels_on_ct_windows():
     assert not failed, failed
 
 
-@pytest.mark.parametrize("S,cout,feats", [(96, 16, DEFAULT), (32, 13, SMALL)], ids=["96_C16_default", "32_C13_small"])
-def test_denoiser_call_on_ct_windows(S, cout, feats):
+def check_denoiser_call(tag, S, cout, feats):
     """One denoiser call, batch [tissue, boundary, tissue] at t = 999 / 500 / 40 (x_t = q_sample of a block label volume:
     at t = 40 the input is nearly piecewise constant), every mode, vs the fp64 oracle and the AMP oracles."""
     image = _images(("tissue", "boundary", "tissue"), S)
@@ -119,11 +117,23 @@ def test_denoiser_call_on_ct_windows(S, cout, feats):
         for b, tb in enumerate(T3):
             err = rel_l2(got[b], ref[b])
             amp_err = {p: rel_l2(a[b], ref[b]) for p, a in amps.items()}
-            line = (f"denoise {S}^3 C={cout} {precision:6s} t={tb:3d}: rel-l2 {err:.3e}  "
+            line = (f"denoise {tag} {precision:6s} t={tb:3d}: rel-l2 {err:.3e}  "
                     f"(fp16-AMP {amp_err['fp16']:.3e}, bf16-AMP {amp_err['bf16']:.3e})")
             print(line)
             assert _gate(precision, err, amp_err.get(precision, 0.0)), line
         del m
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+def test_encoder_all_levels_on_ct_windows():
+    """check_encoder_levels at 96^3, default features, batch [tissue, boundary, air]."""
+    check_encoder_levels("96^3 default", 96, DEFAULT, ("tissue", "boundary", "air"))
+
+
+@pytest.mark.parametrize("S,cout,feats", [(96, 16, DEFAULT), (32, 13, SMALL)], ids=["96_C16_default", "32_C13_small"])
+def test_denoiser_call_on_ct_windows(S, cout, feats):
+    """check_denoiser_call at the production 96^3 shape and at 32^3 with narrow features."""
+    check_denoiser_call(f"{S}^3 C={cout}", S, cout, feats)
 
 
 def test_ddim_window_on_ct_windows():
