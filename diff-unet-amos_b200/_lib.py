@@ -11,7 +11,8 @@ from ctypes import POINTER, c_char_p, c_float, c_int32, c_int64, c_size_t, c_uin
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libdunet_b200.so")
-DUNET_VERSION = 210  # include/dunet.h: the ABI the signatures below describe
+DUNET_VERSION = 220  # include/dunet.h: the ABI the signatures below describe
+MAX_IN_CHANNELS = 10  # include/dunet.h DUNET_MAX_IN_CHANNELS
 
 DUNET_FLAG_REF_CONV = 1
 DUNET_FLAG_KEEP_FP32_WEIGHTS = 2

@@ -53,7 +53,7 @@ __global__ void __launch_bounds__(128) conv3d_ref_kernel(const __nv_bfloat16* __
                 for (int j = 0; j < 8; ++j) {
                   if (oc * 8 + j >= cout) continue;
                   const float wv =
-                      round_16<HF>(w[((long long)(oc * 8 + j) * cin + (rot ? (ci + k + 1) % c0 : ci + k)) * 27 + tap]);
+                      round_16<HF>(w[((long long)(oc * 8 + j) * cin + (rot ? (ci + k + rot) % c0 : ci + k)) * 27 + tap]);
                   acc[j] = fmaf(xi[k], wv, acc[j]);
                 }
               }

@@ -199,7 +199,7 @@ __global__ void pack_conv_w_kernel(const float* __restrict__ w, bf16* __restrict
     int ci = -1, wpart = part;
     if (triple) {  // one block holds [A.hi | A.lo | A.hi] of the c0r real channels against [W.hi | W.hi | W.lo] (see ConvW::triple)
       if (lc < 3 * c0r) { ci = lc % c0r; wpart = lc / c0r == 2 ? 2 : 0; }
-    } else if (lc < c0p) { if (lc < c0r) ci = rot ? (lc + 1) % c0r : lc; }  // rot: packed order is [x.., image], reference [image, x..]
+    } else if (lc < c0p) { if (lc < c0r) ci = rot ? (lc + rot) % c0r : lc; }  // rot: packed order is [x.., image..], reference [image.., x..]
     else { const int l1 = lc - c0p; if (l1 < c1r) ci = c0r + l1; }
     float v = 0.f;
     if (co < coutr && ci >= 0) v = w[((long long)co * cinr + ci) * 27 + tap];
@@ -228,7 +228,7 @@ __global__ void pack_conv_w64_kernel(const float* __restrict__ w, bf16* __restri
     int ci = -1, wpart = part;
     if (triple) {  // one block holds [A.hi | A.lo | A.hi] of the c0r real channels against [W.hi | W.hi | W.lo] (see ConvW::triple)
       if (lc < 3 * c0r) { ci = lc % c0r; wpart = lc / c0r == 2 ? 2 : 0; }
-    } else if (lc < c0p) { if (lc < c0r) ci = rot ? (lc + 1) % c0r : lc; }  // rot: packed order is [x.., image], reference [image, x..]
+    } else if (lc < c0p) { if (lc < c0r) ci = rot ? (lc + rot) % c0r : lc; }  // rot: packed order is [x.., image..], reference [image.., x..]
     else { const int l1 = lc - c0p; if (l1 < c1r) ci = c0r + l1; }
     float v = 0.f;
     if (co < coutr && ci >= 0) v = w[((long long)co * cinr + ci) * 27 + tap];
@@ -297,7 +297,7 @@ struct ConvW {
   bf16* packed64 = nullptr;  // z-stacked layout for the Cout = 64 kernel (coutp == 64 only)
   float* w32 = nullptr;  // debug copy of the original fp32 weight
   float *gamma = nullptr, *beta = nullptr;
-  int rot = 0;  // 1: packed input channel j holds reference channel (j + 1) % c0r (denoiser input [x.., image])
+  int rot = 0;  // > 0: packed input channel j holds reference channel (j + rot) % c0r (denoiser input [x.., image..], rot = in_channels)
   bool have_w = false, have_cb = false, have_g = false, have_b = false;
   void shape(int c0r_, int c0p_, int c1r_, int c1p_, int coutr_, int parts_ = 1, int cb64_ = 32) {
     c0r = c0r_; c0p = c0p_; c1r = c1r_; c1p = c1p_; coutr = coutr_; parts = parts_;
@@ -1180,7 +1180,7 @@ static void final_args_common(dunet_plan* p, FinalDdimArgs& a, uint8_t* ws, cons
   memset(&a, 0, sizeof a);
   a.feat = feat.hi; a.feat_lo = feat.lo; a.F = p->fp[5]; a.w = p->final_w; a.b = p->final_b; a.C = p->C;
   a.partial = reinterpret_cast<float*>(ws + L.partial); a.nseg = nseg; a.gamma = p->upc[1].b.gamma; a.beta = p->upc[1].b.beta;
-  a.eps = 1e-5f; a.slope = 0.1f; a.in_pad = p->in_pad; a.vox = p->V[0]; a.batch = B;
+  a.eps = 1e-5f; a.slope = 0.1f; a.in_pad = p->in_pad; a.vox = p->V[0]; a.batch = B; a.in_ch = p->cfg.in_channels;
 }
 
 static int launch_final(dunet_plan* p, const FinalDdimArgs& a, cudaStream_t st) {
@@ -1188,18 +1188,23 @@ static int launch_final(dunet_plan* p, const FinalDdimArgs& a, cudaStream_t st) 
   const dim3 grid(grid_for((a.vox + 15) / 16 * 32, FINAL_THREADS, std::max(1, 148 * 3 / a.batch)), a.batch);
   if (a.F != 64 && a.F != 128) return fail(DUNET_E_UNSUPPORTED, "final conv: padded features[5] must be 64 or 128");
   const bool prec = a.feat_lo != nullptr;
-#define DUNET_FINAL(NT)                                                                            \
+#define DUNET_FINAL_MC(NT, MC)                                                                     \
   do {                                                                                             \
     if (prec) {                                                                                    \
-      if (a.F == 64) launch_k(final_ddim_kernel<NT, 4, MODE_FP32X3>, grid, dim3(FINAL_THREADS), 0, st, a);     \
-      else launch_k(final_ddim_kernel<NT, 8, MODE_FP32X3>, grid, dim3(FINAL_THREADS), 0, st, a);               \
+      if (a.F == 64) launch_k(final_ddim_kernel<NT, 4, MODE_FP32X3, MC>, grid, dim3(FINAL_THREADS), 0, st, a); \
+      else launch_k(final_ddim_kernel<NT, 8, MODE_FP32X3, MC>, grid, dim3(FINAL_THREADS), 0, st, a);           \
     } else if (is_fp16(p)) {                                                                       \
-      if (a.F == 64) launch_k(final_ddim_kernel<NT, 4, MODE_FP16>, grid, dim3(FINAL_THREADS), 0, st, a);       \
-      else launch_k(final_ddim_kernel<NT, 8, MODE_FP16>, grid, dim3(FINAL_THREADS), 0, st, a);                 \
+      if (a.F == 64) launch_k(final_ddim_kernel<NT, 4, MODE_FP16, MC>, grid, dim3(FINAL_THREADS), 0, st, a);   \
+      else launch_k(final_ddim_kernel<NT, 8, MODE_FP16, MC>, grid, dim3(FINAL_THREADS), 0, st, a);             \
     } else {                                                                                       \
-      if (a.F == 64) launch_k(final_ddim_kernel<NT, 4, MODE_BF16>, grid, dim3(FINAL_THREADS), 0, st, a);       \
-      else launch_k(final_ddim_kernel<NT, 8, MODE_BF16>, grid, dim3(FINAL_THREADS), 0, st, a);                 \
+      if (a.F == 64) launch_k(final_ddim_kernel<NT, 4, MODE_BF16, MC>, grid, dim3(FINAL_THREADS), 0, st, a);   \
+      else launch_k(final_ddim_kernel<NT, 8, MODE_BF16, MC>, grid, dim3(FINAL_THREADS), 0, st, a);             \
     }                                                                                              \
+  } while (0)
+#define DUNET_FINAL(NT)                         \
+  do {                                          \
+    if (a.in_ch > 1) DUNET_FINAL_MC(NT, true);  \
+    else DUNET_FINAL_MC(NT, false);             \
   } while (0)
   if (PROF_ON)  // feature map read once (bf16) + fp32 state x_t and sum(x0) read+written + bf16 re-pack of the next input
     prof_of(p)->bytes[PROF_FINAL] += (double)a.batch * (double)a.vox * ((prec ? 4.0 : 2.0) * a.F + (a.x_t ? 16.0 * a.C : 0.0) + (a.logits_out ? 4.0 * a.C : 0.0) + (a.next_in ? 2.0 * a.C : 0.0));
@@ -1208,6 +1213,7 @@ static int launch_final(dunet_plan* p, const FinalDdimArgs& a, cudaStream_t st) 
   else if (a.C <= 16) DUNET_FINAL(2);
   else DUNET_FINAL(4);
 #undef DUNET_FINAL
+#undef DUNET_FINAL_MC
   LAUNCH_CHECK();
   TRY(prof_end(st));
   return 0;
@@ -1355,9 +1361,14 @@ int dunet_plan_create(dunet_plan** out, const dunet_cfg* cfg) {
   cudaDeviceProp prop;
   CUDA_TRY(cudaGetDeviceProperties(&prop, dev));
   if (prop.major != 10) return fail(DUNET_E_UNSUPPORTED, "libdunet_b200 needs an sm_100a device (found sm_%d%d); there is no fallback path", prop.major, prop.minor);
-  if (cfg->in_channels != 1) return fail(DUNET_E_UNSUPPORTED, "only in_channels == 1 is implemented");
-  if (cfg->num_classes < 1 || cfg->num_classes + cfg->in_channels > 32 || cfg->num_classes > FINAL_MAX_C)
+  // the encoder's first conv packs [A.hi | A.lo | A.hi] of the image into ONE 32-channel block: 3 * in_channels <= 32
+  if (cfg->in_channels < 1 || cfg->in_channels > DUNET_MAX_IN_CHANNELS)
+    return fail(DUNET_E_UNSUPPORTED, "in_channels = %d outside [1, %d]", cfg->in_channels, DUNET_MAX_IN_CHANNELS);
+  // the denoiser input [x_0 .. x_{C-1}, image ..] is packed into in_pad = 32 channels
+  if (cfg->num_classes < 1 || cfg->num_classes > FINAL_MAX_C)
     return fail(DUNET_E_UNSUPPORTED, "num_classes must be in [1, 31]");
+  if (cfg->num_classes + cfg->in_channels > 32)
+    return fail(DUNET_E_UNSUPPORTED, "num_classes + in_channels = %d exceeds 32", cfg->num_classes + cfg->in_channels);
   for (int d = 0; d < 3; ++d)
     if (cfg->patch[d] < 32 || cfg->patch[d] % 16) return fail(DUNET_E_INVALID, "patch edge %d must be a multiple of 16 and >= 32", cfg->patch[d]);
   for (int i = 0; i < 6; ++i)
@@ -1405,7 +1416,7 @@ int dunet_plan_create(dunet_plan** out, const dunet_cfg* cfg) {
     e.b.shape(p->fr[l], p->fp[l], 0, 0, p->fr[l], parts_enc, cb64);
     TwoConvW& d = p->den[l];
     d.has_temb = true;
-    if (l == 0) { d.a.shape(cfg->in_channels + p->C, p->in_pad, 0, 0, p->fr[0], parts, cb64); d.a.rot = 1; }
+    if (l == 0) { d.a.shape(cfg->in_channels + p->C, p->in_pad, 0, 0, p->fr[0], parts, cb64); d.a.rot = cfg->in_channels; }
     else d.a.shape(p->fr[l - 1], p->fp[l - 1], 0, 0, p->fr[l], parts, cb64);
     d.b.shape(p->fr[l], p->fp[l], 0, 0, p->fr[l], parts, cb64);
   }
@@ -1710,14 +1721,15 @@ static int ddim_core(dunet_plan* p, const float* image, const NoiseSrc& nz, int 
     DdimInitArgs ia;
     memset(&ia, 0, sizeof ia);
     ia.noise = nz.given ? nz.given + (size_t)b0 * p->C * p->V[0] : nullptr;
-    ia.image = image + (size_t)b0 * p->V[0];
+    ia.image = image + (size_t)b0 * p->cfg.in_channels * p->V[0];
     ia.x_t = x_t + (size_t)b0 * p->V[0] * CP; ia.acc = acc + (size_t)b0 * p->V[0] * CP;
     ia.next_in = in_pack.hi + (size_t)b0 * p->in_pad * p->V[0];
     ia.next_in_lo = in_pack.lo ? in_pack.lo + (size_t)b0 * p->in_pad * p->V[0] : nullptr;
     ia.C = p->C; ia.CP = CP; ia.in_pad = p->in_pad; ia.batch = nb; ia.zero_acc = zero_acc; ia.vox = p->V[0]; ia.seed = nz.seed;
+    ia.in_ch = p->cfg.in_channels;
     for (int j = 0; j < nb; ++j) ia.ids[j] = nz.ids ? (long long)(((unsigned long long)nz.ids[id0 + b0 + j] & 0xFFFFFFFFFFull) | ((unsigned long long)nz.draw << 40)) : 0;
     const int nch = std::max(CP, p->in_pad) / 8;
-    if (PROF_ON) prof_of(p)->bytes[PROF_GLUE] += (double)nb * p->V[0] * (CP * 8.0 + p->in_pad * 2.0 + 4.0 + (nz.given ? 4.0 * p->C : 0.0));
+    if (PROF_ON) prof_of(p)->bytes[PROF_GLUE] += (double)nb * p->V[0] * (CP * 8.0 + p->in_pad * 2.0 + 4.0 * p->cfg.in_channels + (nz.given ? 4.0 * p->C : 0.0));
     TRY(prof_begin(PROF_GLUE, st));
     DUNET_FMT(fmt_h(p, in_pack.lo != nullptr), launch_k(ddim_init_kernel<HF>, dim3(grid_for((long long)nb * p->V[0] * nch, 256, 148 * 8)), dim3(256), 0, st, ia));
     LAUNCH_CHECK();
@@ -1796,24 +1808,25 @@ int dunet_crop_window(const float* volume, const int32_t v[3], float* patch, con
   return 0;
 }
 
-static int crop_batch(const dunet_plan* p, const float* volume, const int32_t v[3], float* patches, const int32_t pd[3],
+// volume [nc][v], patches [B][nc][pd]
+static int crop_batch(const dunet_plan* p, const float* volume, const int32_t v[3], int nc, float* patches, const int32_t pd[3],
                       const int32_t* starts, int B, cudaStream_t st) {
-  const long long pv = (long long)pd[0] * pd[1] * pd[2];
+  const long long pe = (long long)pd[0] * pd[1] * pd[2] * nc;  // elements per window
   for (int b0 = 0; b0 < B; b0 += INIT_MAX_B) {
     const int nb = std::min(INIT_MAX_B, B - b0);
     CropArgs c;
     memset(&c, 0, sizeof c);
-    c.vol = volume; c.patches = patches + (size_t)b0 * pv;
-    c.VD = v[0]; c.VH = v[1]; c.VW = v[2]; c.PD = pd[0]; c.PH = pd[1]; c.PW = pd[2]; c.batch = nb;
+    c.vol = volume; c.patches = patches + (size_t)b0 * pe;
+    c.VD = v[0]; c.VH = v[1]; c.VW = v[2]; c.PD = pd[0]; c.PH = pd[1]; c.PW = pd[2]; c.batch = nb; c.nc = nc;
     for (int j = 0; j < nb; ++j) {
       TRY(check_box(v, pd, starts + 3 * (b0 + j)));
       for (int d = 0; d < 3; ++d) c.start[j][d] = starts[3 * (b0 + j) + d];
     }
     if (p) {
-      if (PROF_ON) prof_of(p)->bytes[PROF_GLUE] += 8.0 * nb * pv;
+      if (PROF_ON) prof_of(p)->bytes[PROF_GLUE] += 8.0 * nb * pe;
       TRY(prof_begin(PROF_GLUE, st));
     }
-    launch_k(crop_windows_kernel, dim3(grid_for(pv * nb, 256)), dim3(256), 0, st, c);
+    launch_k(crop_windows_kernel, dim3(grid_for(pe * nb, 256)), dim3(256), 0, st, c);
     LAUNCH_CHECK();
     if (p) TRY(prof_end(st));
   }
@@ -1823,7 +1836,7 @@ static int crop_batch(const dunet_plan* p, const float* volume, const int32_t v[
 int dunet_crop_windows(const float* volume, const int32_t v[3], float* patches, const int32_t pd[3], const int32_t* starts,
                        int32_t B, void* stream) {
   if (!volume || !patches || !v || !pd || !starts || B < 1) return fail(DUNET_E_INVALID, "bad argument");
-  return crop_batch(nullptr, volume, v, patches, pd, starts, B, static_cast<cudaStream_t>(stream));
+  return crop_batch(nullptr, volume, v, 1, patches, pd, starts, B, static_cast<cudaStream_t>(stream));
 }
 
 int dunet_infer_windows(dunet_plan* p, const float* volume, const int32_t v[3], const int32_t* starts, int32_t B,
@@ -1842,7 +1855,7 @@ int dunet_infer_windows(dunet_plan* p, const float* volume, const int32_t v[3], 
   const SubBatches sb = sub_batches(p, B, use_dual(p, B, 1));
   TRY(run_sub_batches(p, sb, B, ws, st, [&](int b0, int nb, uint8_t* ws_h, cudaStream_t sh) -> int {
     float* image = reinterpret_cast<float*>(ws_h + ws_layout(p, nb).image);
-    TRY(crop_batch(p, volume, v, image, pd, starts + 3 * b0, nb, sh));  // window crop: one launch per sub-batch
+    TRY(crop_batch(p, volume, v, p->cfg.in_channels, image, pd, starts + 3 * b0, nb, sh));  // window crop: one launch per sub-batch
     for (int r = 0; r < ensemble; ++r) {  // BASELINE config 4: R independent noise draws, summed; the encoder runs once
       NoiseSrc nz;
       nz.given = noise ? noise + ((size_t)r * B + b0) * p->C * p->V[0] : nullptr;

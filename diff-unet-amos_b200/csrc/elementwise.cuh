@@ -755,9 +755,12 @@ __global__ void __launch_bounds__(256) deconv2_kernel(const __nv_bfloat16* __res
 // hi + lo bf16 parts (two MMAs) so the weights keep ~16 mantissa bits; everything else is plain fp32.
 // The kernel is HBM-bound (reads the 64-channel feature map once, reads/writes the fp32 state once).
 //
-// Packed denoiser-input channel order: [x_0 .. x_{C-1}, image, 0 ...]  (the reference's cat([image, x]) order is
-// restored by permuting the first conv's input channels when its weights are packed), so a thread's two adjacent
-// classes form one aligned 4-byte store.
+// Packed denoiser-input channel order: [x_0 .. x_{C-1}, image_0 .. image_{in_ch-1}, 0 ...]  (the reference's
+// cat([image, x]) order is restored by permuting the first conv's input channels when its weights are packed), so a
+// thread's two adjacent classes form one aligned 4-byte store.  The re-pack rewrites the class tiles (channels < 8 * NT)
+// only: image channels inside them are rewritten every step, those past them keep what ddim_init_kernel wrote.
+// MC (in_ch > 1) reads each image channel where it is stored; MC = false keeps the single-channel path's one
+// hoisted image load per voxel.
 // ---------------------------------------------------------------------------------------------------------------
 struct FinalDdimArgs {
   const __nv_bfloat16* feat;  // RAW output of the last conv (or, with partial == nullptr, the activated u1), C8-planar
@@ -772,15 +775,16 @@ struct FinalDdimArgs {
   const float* w;             // [C][F] fp32
   const float* b;             // [C]
   int C;
-  const float* image;         // [B][1][vox] fp32 (in_channels = 1)
+  const float* image;         // [B][in_ch][vox] fp32
   float* x_t;                 // DDIM state, VOXEL-MAJOR fp32 [B][vox][8*NT], updated in place (nullptr: logits only)
   float* acc;                 // sum of clamped x0, same voxel-major layout, += clamp(logits)
   float* logits_out;          // optional [B][C][vox]
-  __nv_bfloat16* next_in;     // optional packed [x_prev, image, 0..] with in_pad channels
+  __nv_bfloat16* next_in;     // optional packed [x_prev, image.., 0..] with in_pad channels
   int in_pad;
   long long vox;
   int batch;
   float r, m, abp;            // sqrt_recip_alphas_cumprod[i], sqrt_recipm1_alphas_cumprod[i], alphas_cumprod_prev[i]
+  int in_ch;                  // image channels (1 unless MC)
 };
 
 constexpr int FINAL_MAX_C = 32;
@@ -799,8 +803,8 @@ __device__ __forceinline__ void mma_16816(float (&d)[4], const uint32_t (&a)[4],
                  : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
 
-// NT = number of 8-class column tiles (C <= 8 * NT); NKS = F / 16 k-steps
-template <int NT, int NKS, int MODE>
+// NT = number of 8-class column tiles (C <= 8 * NT); NKS = F / 16 k-steps; MC = more than one image channel
+template <int NT, int NKS, int MODE, bool MC>
 __global__ void __launch_bounds__(FINAL_THREADS) final_ddim_kernel(FinalDdimArgs a) {
   constexpr bool PREC = MODE == MODE_FP32X3, H = MODE == MODE_FP16;
   // B fragments of the weights: [k-step][n-tile][hi|lo][b0|b1][lane]
@@ -844,7 +848,7 @@ __global__ void __launch_bounds__(FINAL_THREADS) final_ddim_kernel(FinalDdimArgs
   const unsigned vox = (unsigned)a.vox;
   const uint32_t* __restrict__ fw = reinterpret_cast<const uint32_t*>(a.feat) + (size_t)n * fch * vox * 4 + t;
   const uint32_t* __restrict__ fw_lo = reinterpret_cast<const uint32_t*>(a.feat_lo) + (size_t)n * fch * vox * 4 + t;
-  const float* __restrict__ img_n = a.image ? a.image + (size_t)n * vox : nullptr;
+  const float* __restrict__ img_n = a.image ? a.image + (size_t)n * (MC ? a.in_ch : 1) * vox : nullptr;
   // voxel-major state: a quad of lanes (t = 0..3) covers 8 consecutive classes of one voxel with float2 accesses, so
   // the 8 voxels x NT*8 classes a warp touches per access form one contiguous run
   float2* xt_n = a.x_t ? reinterpret_cast<float2*>(a.x_t) + (size_t)n * vox * (NT * 4) + t : nullptr;
@@ -860,7 +864,7 @@ __global__ void __launch_bounds__(FINAL_THREADS) final_ddim_kernel(FinalDdimArgs
     for (int b = 0; b < 2; ++b) {
       const int cls = nt * 8 + 2 * t + b;
       cls_ok[nt][b] = cls < a.C;
-      cls_img[nt][b] = cls == a.C;
+      cls_img[nt][b] = MC ? (cls >= a.C && cls < a.C + a.in_ch) : cls == a.C;
       cls_off[nt][b] = (unsigned)cls * vox;
     }
   const unsigned warps = gridDim.x * (FINAL_THREADS / 32);
@@ -880,8 +884,8 @@ __global__ void __launch_bounds__(FINAL_THREADS) final_ddim_kernel(FinalDdimArgs
         ac[nt][1] = ok1 ? acc_n[v1 * (NT * 4) + nt * 4] : make_float2(0.f, 0.f);
       }
     }
-    const float img0 = (np_n && ok0) ? img_n[v0] : 0.f;
-    const float img1 = (np_n && ok1) ? img_n[v1] : 0.f;
+    const float img0 = (!MC && np_n && ok0) ? img_n[v0] : 0.f;
+    const float img1 = (!MC && np_n && ok1) ? img_n[v1] : 0.f;
     // A fragments: rows (voxels) v0 / v1, channel pairs (2t, 2t+1) of chunk 2ks and of chunk 2ks+1
     uint32_t af[NKS][4], al[PREC ? NKS : 1][4];
 #pragma unroll
@@ -944,7 +948,11 @@ __global__ void __launch_bounds__(FINAL_THREADS) final_ddim_kernel(FinalDdimArgs
         const bool okv = (j >> 1) ? ok1 : ok0;
         const float xin = (j & 1) ? xt[nt][j >> 1].y : xt[nt][j >> 1].x;
         const float ain = (j & 1) ? ac[nt][j >> 1].y : ac[nt][j >> 1].x;
-        float val = cls_img[nt][j & 1] ? ((j >> 1) ? img1 : img0) : 0.f;
+        float val;
+        if constexpr (MC)  // image channel cls - C of this voxel
+          val = (cls_img[nt][j & 1] && np_n && okv) ? img_n[(unsigned)(nt * 8 + 2 * t + (j & 1) - a.C) * vox + ((j >> 1) ? v1 : v0)] : 0.f;
+        else
+          val = cls_img[nt][j & 1] ? ((j >> 1) ? img1 : img0) : 0.f;
         xp4[j] = 0.f;
         ac4[j] = 0.f;
         if (cls_ok[nt][j & 1] && okv) {
@@ -1010,7 +1018,8 @@ __global__ void state_from_vm_kernel(const float* __restrict__ src, float* __res
 // Start of a DDIM window (gaussian_diffusion.py:690-693 `img = noise or th.randn(shape)`): ONE pass that writes
 //   x_t  = the initial noise, voxel-major fp32 [B][vox][CP]      (state read/written by final_ddim_kernel)
 //   acc  = 0 (same layout; skipped when `zero_acc == 0`: ensemble draws keep accumulating)
-//   next = the packed 16-bit input of the first denoiser conv [x_0 .. x_{C-1}, image, 0 ..] (C8-planar, in_pad channels)
+//   next = the packed 16-bit input of the first denoiser conv [x_0 .. x_{C-1}, image_0 .. image_{in_ch-1}, 0 ..]
+//          (C8-planar, in_pad channels)
 // The noise is either the caller's tensor (planar fp32 [B][C][vox], parity runs) or generated here: Philox4x32-10 keyed by
 // `seed`, counter = (element index / 4, window id), Box-Muller -> N(0,1).  Counter-based: a window's noise depends only
 // on (seed, window id), not on batching, rank or launch order (multi-GPU runs give identical volumes).
@@ -1039,12 +1048,12 @@ __device__ __forceinline__ void box_muller(uint32_t a, uint32_t b, float& z0, fl
 constexpr int INIT_MAX_B = 16;
 struct DdimInitArgs {
   const float* noise;      // [B][C][vox] or nullptr (generate)
-  const float* image;      // [B][1][vox]
+  const float* image;      // [B][in_ch][vox]
   float* x_t;              // [B][vox][CP]
   float* acc;              // [B][vox][CP]
   __nv_bfloat16* next_in;  // [B][in_pad/8][vox][8]
   __nv_bfloat16* next_in_lo;  // fp32x3 mode or nullptr
-  int C, CP, in_pad, batch, zero_acc;
+  int C, CP, in_pad, batch, zero_acc, in_ch;
   long long vox;
   unsigned long long seed;
   long long ids[INIT_MAX_B];  // noise stream id of each window of the batch
@@ -1090,7 +1099,13 @@ __global__ void __launch_bounds__(256) ddim_init_kernel(DdimInitArgs a) {
       }
     }
     if (ck * 8 < a.in_pad) {
-      if (a.C >= ck * 8 && a.C < ck * 8 + 8) f[a.C - ck * 8] = a.image[(long long)n * a.vox + v];  // packed order [x.., image, 0..]
+      if (a.C < ck * 8 + 8 && a.C + a.in_ch > ck * 8) {  // packed order [x.., image.., 0..]
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const int ic = ck * 8 + j - a.C;
+          if (ic >= 0 && ic < a.in_ch) f[j] = a.image[((long long)n * a.in_ch + ic) * a.vox + v];
+        }
+      }
       store_split<H>(a.next_in, a.next_in_lo, ((long long)n * (a.in_pad / 8) + ck) * a.vox + v, f);
     }
   }
@@ -1138,23 +1153,24 @@ __global__ void __launch_bounds__(256) q_sample_kernel(const float* __restrict__
 
 // ---------------------------------------------------------------------------------------------------------------
 // Window crop for a whole batch in one launch (MONAI: `torch.cat([inputs[win_slice] for ...])`, engine.py:173-177 driver):
-// patches[b] = volume[start_b : start_b + roi].
+// patches[b][c] = volume[c][start_b : start_b + roi]   (volume [nc][VD][VH][VW], patches [batch][nc][roi])
 // ---------------------------------------------------------------------------------------------------------------
 struct CropArgs {
   const float* vol;
   float* patches;
-  int VD, VH, VW, PD, PH, PW, batch;
+  int VD, VH, VW, PD, PH, PW, batch, nc;
   int start[INIT_MAX_B][3];
 };
 __global__ void crop_windows_kernel(CropArgs a) {
   pdl_wait();
   const long long pv = (long long)a.PD * a.PH * a.PW;
-  const long long total = pv * a.batch;
+  const long long total = pv * a.nc * a.batch;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const int b = (int)(i / pv);
+    const int bc = (int)(i / pv);  // window * nc + channel
+    const int b = bc / a.nc, c = bc % a.nc;
     const long long r = i % pv;
     const int x = (int)(r % a.PW), y = (int)((r / a.PW) % a.PH), z = (int)(r / ((long long)a.PW * a.PH));
-    a.patches[i] = a.vol[((long long)(a.start[b][0] + z) * a.VH + a.start[b][1] + y) * a.VW + a.start[b][2] + x];
+    a.patches[i] = a.vol[(((long long)c * a.VD + a.start[b][0] + z) * a.VH + a.start[b][1] + y) * a.VW + a.start[b][2] + x];
   }
 }
 

@@ -321,7 +321,7 @@ def infer_volumes_distributed(model, images: Sequence[torch.Tensor], sw_batch_si
                               seed: int = 0, on_result: Optional[Callable[[int, torch.Tensor], None]] = None,
                               noise_fn: Optional[Callable[[int, int], torch.Tensor]] = None, exchange: str = "auto",
                               volume_shape: Optional[Sequence[int]] = None, device=None):
-    """Throughput mode: ``images`` (a sequence of [1, 1, D, H, W] volumes of ONE shape, already >= the roi on every axis,
+    """Throughput mode: ``images`` (a sequence of [1, in_channels, D, H, W] volumes of ONE shape, already >= the roi on every axis,
     available on every rank; an entry may also be a zero-argument callable returning the volume, which is then only called
     on the ranks whose queue share touches that volume -- e.g. a host-to-device copy that the other ranks can skip; pass
     ``volume_shape=`` in that case) are processed as window queues of G volumes (``queue_group_size``) so that every rank does the
@@ -379,9 +379,9 @@ def infer_volumes_distributed(model, images: Sequence[torch.Tensor], sw_batch_si
             for a, b in zip(bounds[:-1], bounds[1:]):
                 base = grp[v] * n_win
                 if noise_fn is not None:
-                    buf.add_windows(model, img[0, 0], starts[a:b], noise=noise_fn(base + a, b - a))
+                    buf.add_windows(model, img[0], starts[a:b], noise=noise_fn(base + a, b - a))
                 else:
-                    buf.add_windows(model, img[0, 0], starts[a:b], seed=seed, noise_ids=range(base + a, base + b))
+                    buf.add_windows(model, img[0], starts[a:b], seed=seed, noise_ids=range(base + a, base + b))
         if px is not None:
             # ---- fused peer-memory exchange: every rank finalizes its channels of every volume of the group
             px.barrier()  # all partial sums of the group are complete on every rank

@@ -118,13 +118,20 @@ def _pad_to_roi(inputs: torch.Tensor, roi) -> Tuple[torch.Tensor, list]:
 
 
 def crop_windows(volume: torch.Tensor, starts, roi) -> torch.Tensor:
-    """volume [1, D, H, W] fp32 -> [len(starts), 1, *roi]: one launch of the batched crop kernel."""
+    """volume [c, D, H, W] fp32 -> [len(starts), c, *roi].  One launch of the batched crop kernel for c == 1; a
+    multi-channel volume is cropped window by window and channel by channel straight into the batch."""
     lib = _lib.load()
     vol = tuple(volume.shape[-3:])
-    b = len(starts)
-    out = torch.empty((b, 1) + tuple(roi), dtype=torch.float32, device=volume.device)
-    st = (ctypes.c_int32 * (3 * b))(*[int(x) for s3 in starts for x in s3])
-    _lib.check(lib.dunet_crop_windows(_ptr(volume), _lib.i32x3(vol), _ptr(out), _lib.i32x3(roi), st, b, _stream()))
+    b, c = len(starts), volume.shape[0]
+    out = torch.empty((b, c) + tuple(roi), dtype=torch.float32, device=volume.device)
+    if c == 1:
+        st = (ctypes.c_int32 * (3 * b))(*[int(x) for s3 in starts for x in s3])
+        _lib.check(lib.dunet_crop_windows(_ptr(volume), _lib.i32x3(vol), _ptr(out), _lib.i32x3(roi), st, b, _stream()))
+        return out
+    for j, s3 in enumerate(starts):
+        for k in range(c):
+            _lib.check(lib.dunet_crop_window(_ptr(volume[k]), _lib.i32x3(vol), _ptr(out[j, k]), _lib.i32x3(roi), _lib.i32x3(s3),
+                                             _stream()))
     return out
 
 
@@ -149,8 +156,6 @@ def sliding_window_inference(inputs: torch.Tensor, roi_size, sw_batch_size: int,
         raise NotImplementedError(f"blend mode {mode!r}: only 'constant' (the reference's) and 'gaussian' exist")
     if not inputs.is_cuda:
         raise RuntimeError("sliding_window_inference runs on the GPU only (no CPU fallback)")
-    if inputs.shape[1] != 1:
-        raise NotImplementedError("single-channel inputs only")
     roi = tuple(int(r) for r in (roi_size if not isinstance(roi_size, int) else (roi_size,) * 3))
     inputs = inputs.float().contiguous()
     orig = tuple(inputs.shape[2:])
@@ -164,6 +169,8 @@ def sliding_window_inference(inputs: torch.Tensor, roi_size, sw_batch_size: int,
     from .model import DiffUNetB200
 
     fused = isinstance(predictor, DiffUNetB200) and kwargs.get("pred_type") == "ddim_sample" and tuple(predictor.patch) == roi
+    if fused and inputs.shape[1] != predictor.in_channels:
+        raise ValueError(f"inputs have {inputs.shape[1]} channels, the model takes in_channels = {predictor.in_channels}")
     if fused and seed is None and noise_fn is None:
         seed = int(torch.randint(0, 2 ** 62, (1,)).item())
     with torch.cuda.device(inputs.device):
@@ -173,7 +180,7 @@ def sliding_window_inference(inputs: torch.Tensor, roi_size, sw_batch_size: int,
                 model = predictor
                 step = min(int(sw_batch_size), model.batch_max)
                 buf = StitchBuffers(model.num_classes, vol, roi, overlap, inputs.device, mode, sigma_scale)
-                vol_n = inputs[n, 0]
+                vol_n = inputs[n]  # [in_channels, D, H, W]
                 if vol_n.data_ptr() % 16:
                     vol_n = vol_n.clone()
                 for g in range(lo, hi, step):

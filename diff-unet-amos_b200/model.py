@@ -504,12 +504,16 @@ class DiffUNetB200(nn.Module):
                       seed: int = 0, noise_ids=None, ensemble: int = 1, count_volume: torch.Tensor = None,
                       weights: torch.Tensor = None) -> None:
         """One iteration of the window loop of the sliding-window driver, fused (``dunet_infer_windows``): crop the windows
-        at ``starts`` ([b, 3]) out of ``volume`` ([D, H, W] fp32, padded to >= the patch), run encoder + DDIM on them and do
+        at ``starts`` ([b, 3]) out of ``volume`` ([in_channels, D, H, W] fp32, padded to >= the patch; [D, H, W] is accepted
+        when in_channels == 1), run encoder + DDIM on them and do
         ``out_volume[:, window] += pred`` window by window.  Bit-identical to crop + forward(pred_type="ddim_sample") +
         ``out[slices] += pred`` (engine.py:173-177, models/diffusion/diffusion.py:86-102).  ``noise`` ([b, C, *patch] or
         [R, b, C, *patch]) fixes the initial x_T; otherwise the library draws it from (seed, noise_ids[b], draw)."""
         if not volume.is_cuda or volume.dtype != torch.float32 or not volume.is_contiguous():
             raise RuntimeError("volume must be a contiguous fp32 CUDA tensor: the B200 path has no CPU fallback")
+        if not ((volume.dim() == 4 and volume.shape[0] == self.in_channels) or (volume.dim() == 3 and self.in_channels == 1)):
+            raise ValueError(f"volume must be [{self.in_channels}, D, H, W]" + (" or [D, H, W]" if self.in_channels == 1 else "")
+                             + f", got {tuple(volume.shape)}")
         b = len(starts)
         if b < 1 or b > self.batch_max:
             raise ValueError(f"{b} windows outside [1, batch_max = {self.batch_max}]")

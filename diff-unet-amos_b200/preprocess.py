@@ -94,7 +94,10 @@ def spacing_resample(t: torch.Tensor, spacing_in: Sequence[float], pixdim: Seque
 def val_transform(image: torch.Tensor, label: Optional[torch.Tensor], spacing_in: Sequence[float],
                   pixdim: Sequence[float] = (1.5, 1.5, 2.0)):
     """The array part of ``transform["val"]`` (utils.py:165-181): intensity scaling, foreground crop, spacing resample.
-    image: [1, D, H, W] raw intensities (HU); label: [L, D, H, W] or None.  Returns (image, label)."""
+    image: [in_channels, D, H, W] raw intensities; label: [L, D, H, W] or None.  Returns (image, label).  Every kernel
+    here is channel-generic: the intensity window applies to every channel (as MONAI's ScaleIntensityRanged does), the
+    foreground box is taken over all channels, and each channel is resampled on the same grid.  The CT window
+    (-175, 250) HU is the reference's; other modalities need their own normalisation before the window driver."""
     image = scale_intensity_range(_chw(image, "image"))
     if label is not None:
         image, label, _ = crop_foreground(image, _chw(label, "label"))

@@ -29,7 +29,12 @@
 extern "C" {
 #endif
 
-#define DUNET_VERSION 210 /* 0.2.1; _lib.DUNET_VERSION must match */
+#define DUNET_VERSION 220 /* 0.2.2; _lib.DUNET_VERSION must match */
+
+/* dunet_cfg.in_channels range.  The encoder's first conv packs the image as [hi | lo | hi] into ONE 32-channel block
+ * (3 * in_channels <= 32), and the denoiser input [x_0 .. x_{C-1}, image ..] is packed into 32 channels
+ * (num_classes + in_channels <= 32).  Outside these bounds dunet_plan_create returns DUNET_E_UNSUPPORTED. */
+#define DUNET_MAX_IN_CHANNELS 10
 
 enum {
   DUNET_OK = 0,
@@ -87,7 +92,7 @@ typedef struct dunet_plan dunet_plan;
  * (models/diffusion/diffusion.py:38-45: 10 respaced DDIM steps). */
 typedef struct dunet_cfg {
   int32_t num_classes;  /* out_channels C; the denoiser input has in_channels + C channels (denoiser.py:298) */
-  int32_t in_channels;  /* image channels; only 1 is implemented (AMOS/BTCV/MSD CT) */
+  int32_t in_channels;  /* image channels (modalities), 1 .. DUNET_MAX_IN_CHANNELS with num_classes + in_channels <= 32 */
   int32_t patch[3];     /* window (D, H, W); each a multiple of 16 and >= 32 (SURVEY 8c) */
   int32_t features[6];  /* models/diff_unet.py:17, default {64,64,128,256,512,64} */
   int32_t batch_max;    /* windows processed together (the reference loops at batch 1, diffusion.py:88-89) */
@@ -122,7 +127,7 @@ int dunet_plan_commit(dunet_plan* plan, void* stream);
 int dunet_workspace_bytes(const dunet_plan* plan, int32_t batch, size_t* out_bytes);
 
 /* replaces: BasicUNetEncoder.forward(image), models/basic_unet/pretrained/basic_unet.py:496-512.
- * image: [batch, 1, D, H, W] fp32.  The five feature maps stay in the workspace (bf16) for the denoiser. */
+ * image: [batch, in_channels, D, H, W] fp32.  The five feature maps stay in the workspace (bf16) for the denoiser. */
 int dunet_encode(dunet_plan* plan, const float* image, int32_t batch, void* workspace, void* stream);
 /* copies feature map `level` (0..4) out as fp32 NCDHW [batch, features[level], D>>level, ...] / back in */
 int dunet_get_embedding(dunet_plan* plan, int32_t level, float* out, int32_t batch, void* workspace, void* stream);
@@ -134,13 +139,14 @@ int dunet_set_embedding(dunet_plan* plan, int32_t level, const float* in, int32_
  * the respace remap), one per sample.  When all are equal and a member of the plan's schedule (the inference call) the
  * precomputed time-embedding row is used; otherwise a per-sample bias table is built for this call (the timesteps are
  * staged through plan-owned pinned memory, nothing is allocated).  Embeddings are those left in the workspace by
- * dunet_encode / dunet_set_embedding.  logits_out: [batch, C, D, H, W] fp32. */
+ * dunet_encode / dunet_set_embedding.  x_t: [batch, C, D, H, W], image: [batch, in_channels, D, H, W], logits_out:
+ * [batch, C, D, H, W], all fp32. */
 int dunet_denoise_step(dunet_plan* plan, const float* x_t, const float* image, const int32_t* t_original,
                        float* logits_out, int32_t batch, void* workspace, void* stream);
 
 /* replaces: Diffusion.ddim_sample(image) for a batch of windows (models/diffusion/diffusion.py:86-102), i.e.
  * embed_model + SpacedDiffusion.ddim_sample_loop (gaussian_diffusion.py:626-716) + the sum of the N clamped x0
- * predictions.  noise: [batch, C, D, H, W] fp32 initial x_T (gaussian_diffusion.py:690-693); acc_out receives
+ * predictions.  image: [batch, in_channels, D, H, W] fp32; noise: [batch, C, D, H, W] fp32 initial x_T (gaussian_diffusion.py:690-693); acc_out receives
  * sum_k clamp(model_output_k, -1, 1); per_step_logits (nullable): [n_steps, batch, C, D, H, W] raw model outputs in
  * loop order (t high -> low); final_x (nullable): the last sample.  run_encoder == 0 skips the encoder and uses the
  * embeddings already in the workspace (the reference's ddim_sample_loop(model, shape, model_kwargs={image, embeddings})
@@ -160,13 +166,14 @@ int dunet_stitch_add(float* out_volume, const int32_t vol_dims[3], int32_t chann
 /* replaces: `output_image = torch.zeros(...)` at the start of sliding_window_inference: clears the caller's accumulator
  * (cudaMemsetAsync on `stream`; no kernel launch). */
 int dunet_zero(void* ptr, size_t bytes, void* stream);
-/* all windows of a batch in one launch: patches[b] = volume[start_b : start_b + patch_dims]; starts: HOST [batch][3] */
+/* all windows of a batch in one launch: patches[b] = volume[start_b : start_b + patch_dims]; starts: HOST [batch][3].
+ * dunet_crop_window(s) take ONE channel ([D, H, W] volume); crop a multi-channel volume channel by channel. */
 int dunet_crop_windows(const float* volume, const int32_t vol_dims[3], float* patches, const int32_t patch_dims[3],
                        const int32_t* starts, int32_t batch, void* stream);
 
 /* replaces: ONE iteration of the window loop of sliding_window_inference with predictor = Diffusion.forward(pred_type=
  * "ddim_sample") (engine.py:173-177 + models/diffusion/diffusion.py:86-102): crop `batch` windows out of `volume`
- * ([1, D, H, W] fp32, already padded to >= the plan's patch), run encoder + N DDIM steps on them, and add the results into
+ * ([in_channels, D, H, W] fp32, already padded to >= the plan's patch), run encoder + N DDIM steps on them, and add the results into
  * `out_volume` ([C, D, H, W] fp32) window by window in the given order -- `out[slices] += pred`, bit-identical to
  * dunet_crop_window + dunet_ddim_sample + dunet_stitch_add, without the planar [batch, C, patch] intermediates.
  *   starts     HOST [batch][3] window corners (MONAI order)

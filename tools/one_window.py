@@ -1,5 +1,5 @@
 """Run ONE 96^3 window (C=16, default features, DDIM-10) through the B200 path: the ncu / timing target.
-usage: python tools/one_window.py [--batch B] [--reps R] [--steps N]"""
+usage: python tools/one_window.py [--batch B] [--reps R] [--ddim N] [--in-channels K]"""
 import argparse
 import os
 import sys
@@ -15,6 +15,7 @@ ap.add_argument("--batch", type=int, default=1)
 ap.add_argument("--reps", type=int, default=1)
 ap.add_argument("--S", type=int, default=96)
 ap.add_argument("--C", type=int, default=16)
+ap.add_argument("--in-channels", type=int, default=1, help="image channels (1 .. 10)")
 ap.add_argument("--ddim", type=int, default=10)
 ap.add_argument("--prof", action="store_true")
 ap.add_argument("--flags", type=int, default=0)
@@ -23,8 +24,8 @@ ap.add_argument("--precision", default="fp16", choices=["fp16", "bf16", "fp32x3"
 ap.add_argument("--features", default="64,64,128,256,512,64")
 a = ap.parse_args()
 torch.manual_seed(0)
-m = pkg.DiffUNetB200(in_channels=1, out_channels=a.C, image_size=a.S, spatial_size=a.S, batch_max=a.batch, num_steps=a.ddim, features=tuple(int(v) for v in a.features.split(",")), debug_flags=a.flags, precision=a.precision).cuda().eval()
-image = torch.rand(a.batch, 1, a.S, a.S, a.S, device="cuda")
+m = pkg.DiffUNetB200(in_channels=a.in_channels, out_channels=a.C, image_size=a.S, spatial_size=a.S, batch_max=a.batch, num_steps=a.ddim, features=tuple(int(v) for v in a.features.split(",")), debug_flags=a.flags, precision=a.precision).cuda().eval()
+image = torch.rand(a.batch, a.in_channels, a.S, a.S, a.S, device="cuda")
 noise = torch.randn(a.batch, a.C, a.S, a.S, a.S, device="cuda")
 with torch.no_grad():
     m(image=image, pred_type="ddim_sample", noise=noise)  # warm-up: packs weights, allocates the workspace
@@ -72,5 +73,5 @@ if a.prof:
         print("one DDIM step, in issue order (us):")
         for tg, us in seq[fin[1] + 1:fin[2] + 1]:
             print(f"   {names[tg]:14s} {us:8.1f}")
-print(f"window batch {a.batch}: {ms:.2f} ms per call ({ms / a.batch:.2f} ms/window, {1e3 * a.batch / ms:.1f} patches/s), "
+print(f"window batch {a.batch}, in_channels {a.in_channels}: {ms:.2f} ms per call ({ms / a.batch:.2f} ms/window, {1e3 * a.batch / ms:.1f} patches/s), "
       f"host wall {1e3 * (t1 - t0) / a.reps:.2f} ms, out range [{out.min().item():.2f}, {out.max().item():.2f}]")
