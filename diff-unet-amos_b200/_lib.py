@@ -11,7 +11,7 @@ from ctypes import POINTER, c_char_p, c_float, c_int32, c_int64, c_size_t, c_uin
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libdunet_b200.so")
-DUNET_VERSION = 220  # include/dunet.h: the ABI the signatures below describe
+DUNET_VERSION = 230  # include/dunet.h: the ABI the signatures below describe
 MAX_IN_CHANNELS = 10  # include/dunet.h DUNET_MAX_IN_CHANNELS
 
 DUNET_FLAG_REF_CONV = 1
@@ -71,6 +71,8 @@ SIGNATURES = {
     "dunet_foreground_bbox": (c_int32, [c_void_p, c_int32, POINTER(c_int32), c_void_p, c_void_p]),
     "dunet_crop_box": (c_int32, [c_void_p, c_int32, POINTER(c_int32), c_void_p, POINTER(c_int32), POINTER(c_int32), c_void_p]),
     "dunet_resample_spacing": (c_int32, [c_void_p, c_int32, POINTER(c_int32), c_void_p, POINTER(c_int32), POINTER(ctypes.c_double), c_int32, c_void_p]),
+    "dunet_invert_labels": (c_int32, [c_void_p, c_int32, POINTER(c_int32), POINTER(c_int32), POINTER(c_int32), POINTER(ctypes.c_double),
+                                      POINTER(c_int32), POINTER(c_int32), POINTER(c_int32), c_int32, c_void_p, c_void_p, c_void_p]),
     "dunet_uncertainty_fuse": (c_int32, [c_void_p, c_int32, c_int32, c_int64, c_void_p, c_void_p]),
     "dunet_finalize_peers": (c_int32, [POINTER(c_void_p), POINTER(c_int32), POINTER(c_int32), c_int32, POINTER(c_int32), c_int32, c_int32,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -1969,6 +1969,37 @@ int dunet_resample_spacing(const float* in, int32_t channels, const int32_t dims
   return 0;
 }
 
+int dunet_invert_labels(const float* blended, int32_t channels, const int32_t vol_dims[3], const int32_t offset[3],
+                        const int32_t res_dims[3], const double ratio[3], const int32_t box_start[3], const int32_t box_dims[3],
+                        const int32_t out_dims[3], int32_t mode, uint8_t* binary, uint8_t* argmax, void* stream) {
+  if (!blended || !vol_dims || !offset || !res_dims || !ratio || !box_start || !box_dims || !out_dims)
+    return fail(DUNET_E_INVALID, "NULL argument");
+  if (!binary && !argmax) return fail(DUNET_E_INVALID, "binary and argmax are both NULL: nothing to write");
+  if (channels < 1) return fail(DUNET_E_INVALID, "channels = %d must be >= 1", channels);
+  if (argmax && channels > 256) return fail(DUNET_E_INVALID, "argmax labels are uint8: channels = %d must be <= 256", channels);
+  if (mode != 0 && mode != 1) return fail(DUNET_E_INVALID, "mode must be 0 (nearest) or 1 (trilinear)");
+  for (int d = 0; d < 3; ++d)
+    if (!(ratio[d] > 0.0) || !std::isfinite(ratio[d])) return fail(DUNET_E_INVALID, "ratio[%d] = %g must be finite and > 0", d, ratio[d]);
+  TRY(check_box(vol_dims, res_dims, offset));     // the resampled volume inside the driver volume
+  TRY(check_box(out_dims, box_dims, box_start));  // the foreground box inside the output grid
+  InvertLabelsArgs a;
+  a.blended = blended;
+  a.C = channels;
+  a.VH = vol_dims[1];
+  a.VW = vol_dims[2];
+  a.vol_vox = (long long)vol_dims[0] * vol_dims[1] * vol_dims[2];
+  for (int d = 0; d < 3; ++d) {
+    a.off[d] = offset[d]; a.res[d] = res_dims[d]; a.box_start[d] = box_start[d]; a.box_dims[d] = box_dims[d];
+    a.out[d] = out_dims[d]; a.ratio[d] = ratio[d];
+  }
+  a.nearest = mode == 0;
+  a.binary = binary;
+  a.argmax = argmax;
+  invert_labels_kernel<<<grid_for((long long)out_dims[0] * out_dims[1] * out_dims[2], 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
+  LAUNCH_CHECK();
+  return 0;
+}
+
 int dunet_uncertainty_fuse(const float* per_step, int32_t runs, int32_t n_steps, int64_t n, float* out, void* stream) {
   if (!per_step || !out || runs < 1 || n_steps < 1 || n < 1) return fail(DUNET_E_INVALID, "bad argument");
   uncertainty_fuse_kernel<<<grid_for(n, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(per_step, out, runs, n_steps, (long long)n);

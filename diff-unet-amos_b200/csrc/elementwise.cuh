@@ -1294,23 +1294,34 @@ __global__ void stitch_add_weighted_kernel(float* __restrict__ vol, float* __res
   }
 }
 
+// The reference's binarisation (sigmoid(o) > 0.5, engine.py:179-180) of every class of voxel v and its argmax label (first
+// maximum, engine.py:187).  logit(c) returns class c's fp32 logit; binary is [C][vv], argmax [vv], either may be NULL.
+template <typename Logit>
+__device__ __forceinline__ void binarise_voxel(Logit logit, int C, long long vv, long long v, uint8_t* __restrict__ binary,
+                                               uint8_t* __restrict__ argmax) {
+  float best = -INFINITY;
+  int bi = 0;
+  for (int c = 0; c < C; ++c) {
+    const float o = logit(c);
+    if (binary) binary[c * vv + v] = (1.f / (1.f + expf(-o)) > 0.5f) ? 1 : 0;
+    if (o > best) {
+      best = o;
+      bi = c;
+    }
+  }
+  if (argmax) argmax[v] = (uint8_t)bi;
+}
+
 // out /= count_map (fp32 volume), then the same binarisation / argmax as finalize_kernel
 __global__ void finalize_weighted_kernel(float* __restrict__ vol, const float* __restrict__ cnt, uint8_t* __restrict__ binary,
                                          uint8_t* __restrict__ argmax, int C, long long vv) {
   for (long long v = blockIdx.x * (long long)blockDim.x + threadIdx.x; v < vv; v += (long long)gridDim.x * blockDim.x) {
     const float cn = cnt[v];
-    float best = -INFINITY;
-    int bi = 0;
-    for (int c = 0; c < C; ++c) {
+    binarise_voxel([&](int c) {
       const float o = vol[c * vv + v] / cn;
       vol[c * vv + v] = o;
-      if (binary) binary[c * vv + v] = (1.f / (1.f + expf(-o)) > 0.5f) ? 1 : 0;
-      if (o > best) {
-        best = o;
-        bi = c;
-      }
-    }
-    if (argmax) argmax[v] = (uint8_t)bi;
+      return o;
+    }, C, vv, v, binary, argmax);
   }
 }
 
@@ -1349,18 +1360,11 @@ __global__ void finalize_kernel(float* __restrict__ vol, const int* __restrict__
        v += (long long)gridDim.x * blockDim.x) {
     const int x = (int)(v % VW), y = (int)((v / VW) % VH), z = (int)(v / ((long long)VW * VH));
     const float cnt = (float)(cd[z] * ch[y] * cw[x]);
-    float best = -INFINITY;
-    int bi = 0;
-    for (int c = 0; c < C; ++c) {
+    binarise_voxel([&](int c) {
       const float o = vol[c * vv + v] / cnt;
       vol[c * vv + v] = o;
-      if (binary) binary[c * vv + v] = (1.f / (1.f + expf(-o)) > 0.5f) ? 1 : 0;
-      if (o > best) {
-        best = o;
-        bi = c;
-      }
-    }
-    if (argmax) argmax[v] = (uint8_t)bi;
+      return o;
+    }, C, vv, v, binary, argmax);
   }
 }
 
@@ -1418,6 +1422,34 @@ __global__ void crop_box_kernel(const float* __restrict__ in, float* __restrict_
 // r = new spacing / old spacing (voxel 0 stays on voxel 0, MONAI compute_shape_offset with scale_extent = False), border
 // clamped.  mode 0: trilinear (image), weights and lerps in fp32 in a fixed order (x, then y, then z); mode 1: nearest
 // (label), index = rint(coordinate) (round half to even, like grid_sample's nearest).  Coordinates are formed in fp64.
+// The sample point of grid voxel (z, y, x) on a D x H x W source; shared by resample_spacing_kernel and invert_labels_kernel.
+struct ResamplePoint {
+  int z0, y0, x0, z1, y1, x1;  // nearest: (z0, y0, x0) only
+  float fz, fy, fx;
+};
+__device__ __forceinline__ ResamplePoint resample_point(int z, int y, int x, double rz, double ry, double rx, int D, int H, int W,
+                                                        bool nearest) {
+  const double cz = fmin(fmax(z * rz, 0.0), (double)(D - 1)), cy = fmin(fmax(y * ry, 0.0), (double)(H - 1)),
+               cx = fmin(fmax(x * rx, 0.0), (double)(W - 1));
+  ResamplePoint p;
+  if (nearest) {
+    p.z0 = (int)rint(cz); p.y0 = (int)rint(cy); p.x0 = (int)rint(cx);
+    return p;
+  }
+  p.z0 = (int)floor(cz); p.y0 = (int)floor(cy); p.x0 = (int)floor(cx);
+  p.z1 = min(p.z0 + 1, D - 1); p.y1 = min(p.y0 + 1, H - 1); p.x1 = min(p.x0 + 1, W - 1);
+  p.fz = (float)(cz - p.z0); p.fy = (float)(cy - p.y0); p.fx = (float)(cx - p.x0);
+  return p;
+}
+// src: one channel, element (z, y, x) at src[(z * SH + y) * SW + x] (SH, SW: row strides of the volume src lies in)
+__device__ __forceinline__ float resample_sample(const float* __restrict__ src, int SH, int SW, const ResamplePoint& p, bool nearest) {
+  auto at = [&](int zz, int yy, int xx) { return src[((long long)zz * SH + yy) * SW + xx]; };
+  if (nearest) return at(p.z0, p.y0, p.x0);
+  auto lerp = [](float a, float b, float t) { return __fadd_rn(a, __fmul_rn(t, __fsub_rn(b, a))); };
+  const float c00 = lerp(at(p.z0, p.y0, p.x0), at(p.z0, p.y0, p.x1), p.fx), c01 = lerp(at(p.z0, p.y1, p.x0), at(p.z0, p.y1, p.x1), p.fx);
+  const float c10 = lerp(at(p.z1, p.y0, p.x0), at(p.z1, p.y0, p.x1), p.fx), c11 = lerp(at(p.z1, p.y1, p.x0), at(p.z1, p.y1, p.x1), p.fx);
+  return lerp(lerp(c00, c01, p.fy), lerp(c10, c11, p.fy), p.fz);
+}
 __global__ void __launch_bounds__(256) resample_spacing_kernel(const float* __restrict__ in, float* __restrict__ out, int C, int D,
                                                                int H, int W, int OD, int OH, int OW, double rz, double ry,
                                                                double rx, int mode) {
@@ -1426,22 +1458,45 @@ __global__ void __launch_bounds__(256) resample_spacing_kernel(const float* __re
     const int c = (int)(i / ov);
     const long long r = i % ov;
     const int x = (int)(r % OW), y = (int)((r / OW) % OH), z = (int)(r / ((long long)OW * OH));
-    const double cz = fmin(fmax(z * rz, 0.0), (double)(D - 1)), cy = fmin(fmax(y * ry, 0.0), (double)(H - 1)),
-                 cx = fmin(fmax(x * rx, 0.0), (double)(W - 1));
-    const float* src = in + (long long)c * D * H * W;
-    if (mode == 1) {
-      const int iz = (int)rint(cz), iy = (int)rint(cy), ix = (int)rint(cx);
-      out[i] = src[((long long)iz * H + iy) * W + ix];
+    const ResamplePoint p = resample_point(z, y, x, rz, ry, rx, D, H, W, mode == 1);
+    out[i] = resample_sample(in + (long long)c * D * H * W, H, W, p, mode == 1);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Labels on the input volume's grid: MONAI Invertd of the val transforms' Spacingd + CropForegroundd, then AsDiscreted
+// (sigmoid > 0.5, engine.py:179-180), fused.  blended: the finalised fp32 [C][VD][VH][VW] volume of the window driver (padded
+// to the roi when the resampled volume was smaller); the resampled volume [RD][RH][RW] sits at `offset` inside it.  For each
+// voxel p of the [D0][H0][W0] output: outside the foreground box [box_start, box_start + box_dims) the logits are the zeros
+// MONAI's inverse BorderPad inserts (binary 0, argmax 0); inside, j = p - box_start samples the resampled volume at
+// clamp(j * ratio, 0, res - 1) with ratio = spacing_in / pixdim -- the exact inverse of resample_spacing_kernel's mapping, with
+// the same sample point and lerp order -- and each class is binarised as in finalize_kernel.  One thread per output voxel
+// (consecutive threads along W: coalesced byte stores per class plane), looping over the classes.
+// ---------------------------------------------------------------------------------------------------------------
+struct InvertLabelsArgs {
+  const float* blended;
+  int C, VH, VW;               // classes, row strides of the driver volume
+  long long vol_vox;           // VD * VH * VW
+  int off[3], res[3], box_start[3], box_dims[3], out[3];
+  double ratio[3];
+  int nearest;
+  uint8_t* binary;             // [C][D0][H0][W0] or NULL
+  uint8_t* argmax;             // [D0][H0][W0] or NULL
+};
+__global__ void __launch_bounds__(256) invert_labels_kernel(InvertLabelsArgs a) {
+  const long long vv = (long long)a.out[0] * a.out[1] * a.out[2];
+  const float* base = a.blended + ((long long)a.off[0] * a.VH + a.off[1]) * a.VW + a.off[2];
+  for (long long v = blockIdx.x * (long long)blockDim.x + threadIdx.x; v < vv; v += (long long)gridDim.x * blockDim.x) {
+    const int jz = (int)(v / ((long long)a.out[2] * a.out[1])) - a.box_start[0];
+    const int jy = (int)((v / a.out[2]) % a.out[1]) - a.box_start[1];
+    const int jx = (int)(v % a.out[2]) - a.box_start[2];
+    if ((unsigned)jz >= (unsigned)a.box_dims[0] || (unsigned)jy >= (unsigned)a.box_dims[1] || (unsigned)jx >= (unsigned)a.box_dims[2]) {
+      binarise_voxel([](int) { return 0.f; }, a.C, vv, v, a.binary, a.argmax);
       continue;
     }
-    const int z0 = (int)floor(cz), y0 = (int)floor(cy), x0 = (int)floor(cx);
-    const int z1 = min(z0 + 1, D - 1), y1 = min(y0 + 1, H - 1), x1 = min(x0 + 1, W - 1);
-    const float fz = (float)(cz - z0), fy = (float)(cy - y0), fx = (float)(cx - x0);
-    auto at = [&](int zz, int yy, int xx) { return src[((long long)zz * H + yy) * W + xx]; };
-    auto lerp = [](float a, float b, float t) { return __fadd_rn(a, __fmul_rn(t, __fsub_rn(b, a))); };
-    const float c00 = lerp(at(z0, y0, x0), at(z0, y0, x1), fx), c01 = lerp(at(z0, y1, x0), at(z0, y1, x1), fx);
-    const float c10 = lerp(at(z1, y0, x0), at(z1, y0, x1), fx), c11 = lerp(at(z1, y1, x0), at(z1, y1, x1), fx);
-    out[i] = lerp(lerp(c00, c01, fy), lerp(c10, c11, fy), fz);
+    const ResamplePoint p = resample_point(jz, jy, jx, a.ratio[0], a.ratio[1], a.ratio[2], a.res[0], a.res[1], a.res[2], a.nearest);
+    binarise_voxel([&](int c) { return resample_sample(base + c * a.vol_vox, a.VH, a.VW, p, a.nearest); }, a.C, vv, v, a.binary,
+                   a.argmax);
   }
 }
 

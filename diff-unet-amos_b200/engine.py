@@ -25,6 +25,7 @@ import torch
 
 from . import _lib
 from .inference import StitchBuffers, crop_to, sliding_window_inference
+from .invert import predict_original
 
 
 def _ptr(t):
@@ -106,22 +107,35 @@ def dice_from_counts(counts: Sequence[Sequence[int]]) -> list:
 
 
 METRICS = ("dice", "hd95")
+SPACES = ("transformed", "original")
 
 
 class EngineB200:
     """``metrics``: "dice" (always: ``validation_step`` returns the mean Dice) and optionally "hd95", which appends one
     ``OrderedDict`` of per-class HD95 per sample to ``self.hd95s`` (NaN for a class with an empty prediction or label);
-    ``spacing`` is the voxel spacing per array axis (D, H, W) that HD95 is measured in."""
+    ``spacing`` is the voxel spacing per array axis (D, H, W) that HD95 is measured in.
+
+    ``space``: "transformed" (the reference's loop: batches hold the val-transformed image and label) or "original": a
+    batch holds the raw-intensity ``"image"`` [N, in_channels, D, H, W], the ``"label"`` on that same grid and its voxel
+    spacing ``"spacing"`` ((3,) or [N, 3]); each sample runs ``predict_original`` (val transform to ``pixdim``, window driver,
+    labels inverted back onto the input grid), Dice is scored against the original label and HD95 in each sample's own
+    ``"spacing"`` (the constructor's ``spacing`` is then unused) -- the way challenge evaluations such as AMOS score."""
 
     def __init__(self, model, class_names: Optional[Dict[int, str]] = None, sw_batch_size: int = 4, overlap: float = 0.25,
                  include_background: bool = True, use_amp: Optional[bool] = None, device="cuda", epoch: Optional[int] = None,
-                 metrics: Sequence[str] = ("dice",), spacing: Sequence[float] = (1.0, 1.0, 1.0)):
+                 metrics: Sequence[str] = ("dice",), spacing: Sequence[float] = (1.0, 1.0, 1.0), space: str = "transformed",
+                 pixdim: Sequence[float] = (1.5, 1.5, 2.0)):
         unknown = set(metrics) - set(METRICS)
         if unknown or "dice" not in metrics:
             raise ValueError(f"metrics must include 'dice' and be drawn from {METRICS}, got {tuple(metrics)}")
         if len(spacing) != 3:
             raise ValueError(f"spacing needs one value per axis (D, H, W), got {tuple(spacing)}")
+        if space not in SPACES:
+            raise ValueError(f"space must be one of {SPACES}, got {space!r}")
+        if len(pixdim) != 3:
+            raise ValueError(f"pixdim needs one value per axis (D, H, W), got {tuple(pixdim)}")
         self.metrics, self.spacing = tuple(metrics), tuple(float(s) for s in spacing)
+        self.space, self.pixdim = space, tuple(float(p) for p in pixdim)
         self.hd95s = []
         if use_amp is not None:
             model.set_precision("fp16" if use_amp else "fp32x3")
@@ -154,15 +168,31 @@ class EngineB200:
         label = self.convert_labels(batch["label"].to(self.device), phase).float()
         return image, label
 
+    def _spacings(self, batch: dict, n: int) -> list:
+        """Per-sample voxel spacing of an original-space batch: ``batch["spacing"]`` as (3,) or [N, 3]."""
+        if "spacing" not in batch:
+            raise ValueError('space="original" needs batch["spacing"], the voxel spacing (D, H, W) of the input grid')
+        s = torch.as_tensor(batch["spacing"], dtype=torch.float64).cpu()
+        if s.shape == (3,):
+            s = s.expand(n, 3)
+        if s.shape != (n, 3):
+            raise ValueError(f'batch["spacing"] must be (3,) or [{n}, 3], got {tuple(s.shape)}')
+        return [tuple(row) for row in s.tolist()]
+
     # ---- engine.py:167-182
     @torch.no_grad()
     def infer(self, batch: dict, noise_fn=None):
         image, labels = self.get_input(batch, phase="val")
-        outputs_u8 = self._infer_binary(image, noise_fn)
+        spacings = self._spacings(batch, image.shape[0]) if self.space == "original" else None
+        outputs_u8 = self._infer_binary(image, noise_fn, spacings)
         return image, outputs_u8.float(), labels
 
-    def _infer_binary(self, image: torch.Tensor, noise_fn=None) -> torch.Tensor:
-        """[N, C, D, H, W] uint8: ``(sigmoid(sliding_window(...)) > 0.5)`` formed by the finalize kernel."""
+    def _infer_binary(self, image: torch.Tensor, noise_fn=None, spacings=None) -> torch.Tensor:
+        """[N, C, D, H, W] uint8: ``(sigmoid(sliding_window(...)) > 0.5)`` formed by the finalize kernel.  With per-sample
+        ``spacings`` the image is raw and each sample runs ``predict_original``: labels on the image's own grid."""
+        if spacings is not None:
+            return torch.stack([predict_original(self.model, image[n], spacings[n], self.pixdim, self.sw_batch_size, self.overlap,
+                                                 noise_fn=noise_fn) for n in range(image.shape[0])])
         roi = tuple(self.model.patch)
         # the reference's call, engine.py:173-177: sliding_window_inference(image, roi, sw_batch_size, self.model, overlap,
         # pred_type="ddim_sample") -- the driver recognises the model and runs the fused window loop
@@ -180,7 +210,8 @@ class EngineB200:
     @torch.no_grad()
     def validation_step(self, batch: dict, noise_fn=None, verbose: bool = False) -> float:
         image, labels = self.get_input(batch, phase="val")
-        outputs = self._infer_binary(image, noise_fn)
+        spacings = self._spacings(batch, image.shape[0]) if self.space == "original" else None
+        outputs = self._infer_binary(image, noise_fn, spacings)
         classes = list(self.class_names.values())
         dices = OrderedDict()
         counts = dice_counts(outputs.transpose(0, 1).contiguous().flatten(1), labels.transpose(0, 1).contiguous().flatten(1))
@@ -191,7 +222,8 @@ class EngineB200:
         self.dices.append(dices)
         if "hd95" in self.metrics:
             for n in range(outputs.shape[0]):  # per sample: surfaces must not mix across the batch
-                self.hd95s.append(OrderedDict(zip(classes, hd95(outputs[n], labels[n], self.spacing))))
+                spacing = self.spacing if spacings is None else spacings[n]
+                self.hd95s.append(OrderedDict(zip(classes, hd95(outputs[n], labels[n], spacing))))
         self.patient_index += 1
         return float(np.mean(list(dices.values())))
 

@@ -12,6 +12,7 @@ Tensors are [C, D, H, W] fp32 on the GPU; there is no CPU fallback.
 from __future__ import annotations
 
 import ctypes
+from dataclasses import dataclass
 from typing import Optional, Sequence, Tuple
 
 import torch
@@ -91,17 +92,58 @@ def spacing_resample(t: torch.Tensor, spacing_in: Sequence[float], pixdim: Seque
     return out
 
 
+@dataclass(frozen=True)
+class ValTransformMeta:
+    """Geometry of one ``val_transform`` call, what its inverse (``invert_labels``) needs: the shape of the array handed
+    to ``val_transform`` (the "original" grid), the foreground box [box_start, box_end) on it, the two spacings and the
+    resampled shape of the box."""
+    orig_shape: Tuple[int, int, int]
+    box_start: Tuple[int, int, int]
+    box_end: Tuple[int, int, int]
+    spacing_in: Tuple[float, float, float]
+    pixdim: Tuple[float, float, float]
+    res_shape: Tuple[int, int, int]
+
+    @property
+    def box_shape(self) -> Tuple[int, ...]:
+        return tuple(e - s for s, e in zip(self.box_start, self.box_end))
+
+    def offset_in(self, vol: Sequence[int]) -> Tuple[int, ...]:
+        """Corner of the resampled volume inside the window driver's volume ``vol``: the driver pads a volume smaller than
+        the roi symmetrically, with the floor on the low side (``crop_to``)."""
+        if len(vol) != 3 or any(int(v) < r for v, r in zip(vol, self.res_shape)):
+            raise ValueError(f"driver volume {tuple(vol)} does not contain the resampled volume {self.res_shape}")
+        return tuple((int(v) - r) // 2 for v, r in zip(vol, self.res_shape))
+
+
+def val_meta(shape: Sequence[int], box, spacing_in: Sequence[float], pixdim: Sequence[float]) -> ValTransformMeta:
+    """Host arithmetic of ``val_transform(return_meta=True)``: ``box`` is ``foreground_bbox``'s (start, end).  An
+    all-background image, which ``crop_foreground`` leaves uncropped, has the whole volume as its box."""
+    shape = tuple(int(n) for n in shape)
+    start, end = (tuple(int(v) for v in b) for b in box)
+    if end == (0, 0, 0):
+        start, end = (0, 0, 0), shape
+    box_shape = tuple(e - s for s, e in zip(start, end))
+    return ValTransformMeta(shape, start, end, tuple(float(s) for s in spacing_in), tuple(float(p) for p in pixdim),
+                            resampled_shape(box_shape, spacing_in, pixdim))
+
+
 def val_transform(image: torch.Tensor, label: Optional[torch.Tensor], spacing_in: Sequence[float],
-                  pixdim: Sequence[float] = (1.5, 1.5, 2.0)):
+                  pixdim: Sequence[float] = (1.5, 1.5, 2.0), return_meta: bool = False):
     """The array part of ``transform["val"]`` (utils.py:165-181): intensity scaling, foreground crop, spacing resample.
-    image: [in_channels, D, H, W] raw intensities; label: [L, D, H, W] or None.  Returns (image, label).  Every kernel
+    image: [in_channels, D, H, W] raw intensities; label: [L, D, H, W] or None.  Returns (image, label), and with
+    ``return_meta=True`` (image, label, ValTransformMeta) for ``invert_labels``.  Every kernel
     here is channel-generic: the intensity window applies to every channel (as MONAI's ScaleIntensityRanged does), the
     foreground box is taken over all channels, and each channel is resampled on the same grid.  The CT window
     (-175, 250) HU is the reference's; other modalities need their own normalisation before the window driver."""
     image = scale_intensity_range(_chw(image, "image"))
+    shape = tuple(image.shape[1:])
     if label is not None:
-        image, label, _ = crop_foreground(image, _chw(label, "label"))
+        image, label, box = crop_foreground(image, _chw(label, "label"))
         label = spacing_resample(label, spacing_in, pixdim, "nearest")
     else:
-        image, _ = crop_foreground(image)
-    return spacing_resample(image, spacing_in, pixdim, "bilinear"), label
+        image, box = crop_foreground(image)
+    image = spacing_resample(image, spacing_in, pixdim, "bilinear")
+    if not return_meta:
+        return image, label
+    return image, label, val_meta(shape, box, spacing_in, pixdim)

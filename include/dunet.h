@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define DUNET_VERSION 220 /* 0.2.2; _lib.DUNET_VERSION must match */
+#define DUNET_VERSION 230 /* 0.2.3; _lib.DUNET_VERSION must match */
 
 /* dunet_cfg.in_channels range.  The encoder's first conv packs the image as [hi | lo | hi] into ONE 32-channel block
  * (3 * in_channels <= 32), and the denoiser input [x_0 .. x_{C-1}, image ..] is packed into 32 channels
@@ -243,6 +243,26 @@ int dunet_crop_box(const float* in, int32_t channels, const int32_t dims[3], flo
  * `out` as round((dim - 1) / ratio) + 1 per axis (MONAI compute_shape_offset).  Interpolation in fp32 in a fixed order. */
 int dunet_resample_spacing(const float* in, int32_t channels, const int32_t dims[3], float* out, const int32_t out_dims[3],
                            const double ratio[3], int32_t mode, void* stream);
+
+/* replaces: MONAI Invertd(keys="pred", transform=val_transforms, orig_keys="image") of the val transforms' Spacingd +
+ * CropForegroundd (utils.py:171-177), followed by AsDiscreted / the binarisation of engine.py:179-180: labels on the grid of
+ * the array the val transforms received, in one pass, without fp32 intermediates on that grid.
+ *   blended   the finalised fp32 [channels][vol_dims] volume (dunet_finalize / dunet_finalize_weighted leave it divided by
+ *             the coverage); the resampled volume [res_dims] lies at `offset` inside it (the window driver pads a volume
+ *             smaller than the roi: offset = (vol - res) / 2 per axis, floor).
+ *   out_dims  the original grid (D0, H0, W0); the foreground box [box_start, box_start + box_dims) lies inside it and has
+ *             the shape the forward crop produced (the forward resample went box_dims -> res_dims).
+ * For every output voxel p: outside the box binary = 0 and argmax = 0 (MONAI's inverse BorderPad inserts zero logits).
+ * Inside, with j = p - box_start, the sample coordinate on axis d is clamp(j_d * ratio[d], 0, res_dims[d] - 1), formed in
+ * fp64, ratio = spacing_in / pixdim (the inverse of dunet_resample_spacing's pixdim / spacing_in); mode 0 nearest (index
+ * rint(coordinate), Invertd's default nearest_interp=True), 1 trilinear (fp32 lerps in dunet_resample_spacing's order).
+ * Then binary[c][p] = sigmoid(logit_c) > 0.5 and argmax[p] = first maximum over classes, as dunet_finalize forms them: the
+ * result is bit-identical to dunet_resample_spacing to box_dims, zero padding to out_dims and dunet_finalize with unit counts.
+ * binary [channels][out_dims] or NULL, argmax [out_dims] or NULL (not both; channels <= 256 with argmax); ratios finite > 0. */
+int dunet_invert_labels(const float* blended, int32_t channels, const int32_t vol_dims[3], const int32_t offset[3],
+                        const int32_t res_dims[3], const double ratio[3], const int32_t box_start[3],
+                        const int32_t box_dims[3], const int32_t out_dims[3], int32_t mode,
+                        uint8_t* binary, uint8_t* argmax, void* stream);
 
 /* Uncertainty-weighted fusion of the DDIM steps of `runs` independent sampling runs (the test-time fusion of upstream
  * Diff-UNet; this reference returns the plain sum instead, models/diffusion/diffusion.py:94-98; SURVEY 8f-4).
